@@ -16,6 +16,10 @@ statistics table is summed with one NCCL allreduce (weak scaling: E per GPU). Pr
   cpu_baseline  the CPU oracle (a port of the reference's Rust loop) on this box's host cores, bounded sample
 
 `--impl reference` times that CPU port alone (rank 0 only) and prints the same line with "impl": "reference".
+
+`--dump-outputs DIR` writes what the last timed step computed on rank 0 as DIR/<name>.npy (float32 / float64, at most 64 MB
+in all; larger outputs are a fixed, seeded sample). The inputs depend on the arguments only, so two builds run with the same
+arguments can be compared array by array.
 """
 import argparse
 import json
@@ -32,6 +36,50 @@ ASSETS = os.path.join(ROOT, "tests", "golden", "ireland_map")
 METRIC = "full 2025-2050 episodes simulated and scored per second"
 UNIT = "episodes/s"
 RESULT_BYTES, TRAJ_BYTES, POLICY_BYTES = 64, 1088, 38784
+DUMP_SEED = 20250101  # the sample --dump-outputs takes of an output too large to write whole
+DUMP_EPISODES, DUMP_RECORDS, DUMP_SITES = 65536, 4096, 4096
+DUMP_LIMIT = 64 << 20
+
+
+def write_outputs(out_dir, arrays):
+    """--dump-outputs: every array as out_dir/<name>.npy."""
+    import numpy as np
+    total = sum(a.nbytes for a in arrays.values())
+    assert total <= DUMP_LIMIT, "outputs of %d bytes exceed the dump limit" % total
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        assert a.dtype in (np.float32, np.float64), name
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
+def dump_sample(n, k):
+    """Indices of a fixed, seeded sample of k out of n items in ascending order (all of them when n <= k)."""
+    import numpy as np
+    if n <= k:
+        return np.arange(n)
+    return np.sort(np.random.default_rng(DUMP_SEED).choice(n, k, replace=False))
+
+
+def rollout_outputs(results, traj, packs):
+    """What a caller of the rollout step receives: every episode's result, the action records, and the exchanged buffer of
+    every rank ([update statistics | score, global id and record of the rank's best episode], trainer.PACK_WORDS int64 each).
+    The statistics words are counts on the initial weight table, so float64 holds them exactly."""
+    import numpy as np
+    from eirgrid_b200 import _abi
+    out = {}
+    pick = dump_sample(len(results), DUMP_EPISODES)
+    out["result_episode"] = pick.astype(np.float64)
+    for f in ("score", "net_emissions", "public_opinion", "total_cost", "power_reliability", "n_generators", "n_offsets",
+              "n_deficit_actions", "n_additional_actions", "flags"):
+        out["result_" + f] = results[f][pick].astype(np.float64)
+    pick = dump_sample(len(traj), DUMP_RECORDS)
+    out["traj_episode"] = pick.astype(np.float64)
+    for f in ("n_deficit", "n_additional", "actions"):
+        out["traj_" + f] = traj[f][pick].astype(np.float32)
+    out["update_stats"] = packs[:, :_abi.STATS_WORDS].sum(axis=0).astype(np.float64)
+    out["rank_best_score"] = packs[:, _abi.STATS_WORDS].copy().view(np.float64)
+    out["rank_best_episode"] = packs[:, _abi.STATS_WORDS + 1].astype(np.float64)
+    return out
 
 
 def load_peaks():
@@ -263,6 +311,10 @@ def run_suitability(args, emit):
             ev[k][2].record(stream)
         barrier()
         launches = ctx.kernel_launches() - launches0
+        if args.dump_outputs and rank == 0:  # this rank's scores of a seeded sample of its sites
+            pick = dump_sample(n_mine, DUMP_SITES)
+            outputs = {"site": (first + pick).astype(np.float64),
+                       "scores": d_mine.view(-1, NY, NT)[torch.from_numpy(pick).to(dev)].cpu().numpy()}
         t = torch.tensor([sum(ev[k][0].elapsed_time(ev[k][2]) for k in range(K)), sum(ev[k][0].elapsed_time(ev[k][1]) for k in range(K))],
                          dtype=torch.float64, device=dev)
         if world > 1:
@@ -348,6 +400,8 @@ def run_suitability(args, emit):
     if world == 1 and not args.no_cpu_baseline:
         rate, sample, threads, _ = cpu_suitability_rate(args.cpu_seconds)
         line["cpu_baseline"] = {"value": rate, "unit": SUIT_UNIT, "cores": threads, "kind": "port", "sample": sample}
+    if args.dump_outputs:
+        write_outputs(args.dump_outputs, outputs)
     emit(line)
     if world > 1:
         dist.destroy_process_group()
@@ -372,7 +426,13 @@ def main():
     ap.add_argument("--sites-per-axis", type=int, default=1001,
                     help="suitability workload: candidate sites per axis over the 50 km map (51 = the placement search's own 1 km grid)")
     ap.add_argument("--suitability-map", choices=["ireland", "scaled10"], default="ireland")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one computed on rank 0 as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs applies to the GPU implementation")
     if args.impl == "reference":
         return run_reference_suitability(args) if args.workload == "suitability" else run_reference(args)
 
@@ -446,6 +506,9 @@ def main():
         barrier()
         launches = tr.ctx.kernel_launches() - launches0
         tr.check_exchange()
+        if args.dump_outputs and rank == 0:  # the later sections reuse the trainer's buffers: copy the last step out now
+            res_last, traj_last = tr.fetch_results()
+            outputs = rollout_outputs(res_last, traj_last, tr.d_all_pack.cpu().numpy().reshape(world, T.PACK_WORDS))
         step_ms = sum(ev[k][0].elapsed_time(ev[k][2]) for k in range(K))
         rollout_ms = sum(ev[k][0].elapsed_time(ev[k][1]) for k in range(K)) / K
         collective_us = sum(ev[k][3].elapsed_time(ev[k][2]) for k in range(K)) / K * 1e3
@@ -637,6 +700,8 @@ def main():
                                 "sample": "%d episodes in %.1f s, oracle in reference-cost mode (literal 100x100 placement scan, per-evaluation opinion sums), %d threads"
                                           % (n_cpu, dt, threads),
                                 "fast_mode": {"value": rate_fast, "sample": "%d episodes in %.1f s with the exact table restructurings" % (n_fast, dt_fast)}}
+    if args.dump_outputs:
+        write_outputs(args.dump_outputs, outputs)
     emit(line)
     if world > 1:
         dist.destroy_process_group()

@@ -1,7 +1,9 @@
-import sys; sys.path.insert(0, "/root/repo")
+import os, sys
+ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+sys.path.insert(0, ROOT)
 import numpy as np
 from eirgrid_b200 import _abi, _lib, trainer as T
-tr = T.BatchTrainer(65536, seed=99, device=0, asset_dir="/root/repo/tests/golden/ireland_map")
+tr = T.BatchTrainer(65536, seed=99, device=0, asset_dir=os.path.join(ROOT, "tests", "golden", "ireland_map"))
 for i in range(6):
     st = tr.step()
     res, traj = tr.fetch_results()

@@ -1,7 +1,8 @@
 import os, sys, time
-sys.path.insert(0, "/root/repo")
+ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+sys.path.insert(0, ROOT)
 from eirgrid_b200 import _lib
-ctx = _lib.Context(0); ctx.map_load_dir("/root/repo/tests/golden/ireland_map")
+ctx = _lib.Context(0); ctx.map_load_dir(os.path.join(ROOT, "tests", "golden", "ireland_map"))
 for half, step in ((25, 2000.0), (50, 1000.0), (100, 500.0)):
     ctx.location_analysis(True, half, step)
     t = time.perf_counter(); s = ctx.location_analysis(True, half, step); dt = time.perf_counter() - t
