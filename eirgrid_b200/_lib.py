@@ -11,7 +11,7 @@ import numpy as np
 from . import _abi
 
 HERE = os.path.dirname(os.path.abspath(__file__))
-LIB_PATH = os.path.join(HERE, os.environ.get("EIRGRID_LIB_NAME", "libeirgrid_b200.so"))  # override: A/B builds only
+LIB_PATH = os.path.join(HERE, os.environ.get("EIRGRID_LIB_NAME", "libeirgrid_b200.so"))  # side-by-side builds: A/B variants, -DEG_DEBUG_BOUNDS
 
 EXPORTS = [
     "eg_init", "eg_destroy", "eg_last_error", "eg_sync", "eg_kernel_launches", "eg_map_load", "eg_map_set",

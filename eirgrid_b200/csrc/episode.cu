@@ -40,34 +40,13 @@ namespace {
 
 constexpr unsigned kFull = 0xFFFFFFFFu;
 
-// Tuning switches of the A/B builds (scripts/build_variants.sh "name:-DEG_...=v"; every setting below is the measured optimum,
-// profiles/r02_eval_loop.md has the table). Outputs do not depend on any of them.
-#ifndef EG_EVAL_UNROLL
-#define EG_EVAL_UNROLL 2             // groups of four plants per trip of the placement evaluation loop
-#endif
-#ifndef EG_EVAL_UNROLL_STAGNATION
-#define EG_EVAL_UNROLL_STAGNATION 1  // the same in the stagnation-sampler instantiation, the larger one (0: as EG_EVAL_UNROLL)
-#endif
-#ifndef EG_YS_UNROLL
-#define EG_YS_UNROLL 1               // year_start's re-sum over the plants
-#endif
-#ifndef EG_FOLD_UNROLL
-#define EG_FOLD_UNROLL 2             // year folds
-#endif
-#ifndef EG_SCAN_UNROLL
-#define EG_SCAN_UNROLL 4             // sequential sampling scans
-#endif
-#ifndef EG_TABLE_COPIES
-#define EG_TABLE_COPIES 1            // compact maps: copies of the block-shared factor table, interleaved entry by entry; with 16, lane l
-#endif                               // reads copy l & 15 — no bank conflicts, but 40 KB less L1 per block and 3-6 % slower
-// further: -DEG_NO_STASH (episode state stays in registers across the placement walk), -DEG_WALK_ALLOCATE (walk loads allocate in
-// L1), -DEG_EPISODE_WARPS / -DEG_EPISODE_MIN_BLOCKS / -DEG_LARGE_WARPS (block shapes), -DEG_SCAN_SEQUENTIAL, -DEG_ROWS_SYNC
-constexpr int kEvalUnroll = EG_EVAL_UNROLL, kYearStartUnroll = EG_YS_UNROLL, kFoldUnroll = EG_FOLD_UNROLL, kScanUnroll = EG_SCAN_UNROLL;
-constexpr int kTableCopies = EG_TABLE_COPIES;
-#ifndef EG_LOOKUP_PREDICATED
-#define EG_LOOKUP_PREDICATED 2       // bit 0: compact maps, bit 1: medium maps — only lanes in range read the factor table, the others
-#endif                               // multiply by a register 1.0. On the 10x grid the shared-memory pipe is the limiter (97 % busy, half
-                                     // of its wavefronts bank conflicts of the random lookups): +3.4 % there, -3.5 % on the shipped map
+// The tuning constants of this file are the measured optimum (profiles/r02_eval_loop.md, r02_ab_candidates.md). An experiment adds
+// its own -D switch on a branch and merges only the winner, without the switch. Outputs do not depend on any of them.
+constexpr int kEvalUnroll = 2;            // groups of four plants per trip of the placement evaluation loop: 1 and 3 are slower, 4 costs 18 % on the trained table
+constexpr int kEvalUnrollStagnation = 1;  // the same in the stagnation-sampler instantiation on compact maps, the larger one: 2 % faster not unrolled
+constexpr int kYearStartUnroll = 1;       // year_start's re-sum over the plants: unrolled by 2 or 4, +1 % on the initial table, -1..-3 % trained
+constexpr int kFoldUnroll = 2;            // year folds: not unrolled is slower
+constexpr int kScanUnroll = 4;            // sequential sampling scans: unrolled by 2 or 1 is slower
 
 // -DEG_DEBUG_BOUNDS: index checks on the shared-memory structures; a violation sets bit 30 of eg_result.flags, which makes
 // every parity test fail (compute-sanitizer is not available on the GPU pool). Compiled out otherwise.
@@ -97,7 +76,7 @@ constexpr int kOffGxy = kOffVars + 8 * 32;                      // uint32[EG_MAX
 constexpr int kOffGat = kOffGxy + 4 * EG_MAX_NEW_GENERATORS;    // uint16[EG_MAX_NEW_GENERATORS] type(4) mult(2) build(5)
 constexpr int kOffOffs = kOffGat + 2 * EG_MAX_NEW_GENERATORS;   // uint16[EG_MAX_OFFSETS]
 constexpr int kOffCounts = kOffOffs + 2 * EG_MAX_OFFSETS;       // uint16[26] deficit + uint16[26] additional recorded per year
-constexpr int kSliceBytes = (kOffCounts + 4 * EG_NY + 15) & ~15;  // 5.6 KB per warp
+constexpr int kSliceBytes = (kOffCounts + 4 * EG_NY + 15) & ~15;  // 6,896 B per warp
 static_assert(kOffScratch % 16 == 0 && kOffVars % 8 == 0 && kOffGxy % 16 == 0 && EG_MAX_NEW_GENERATORS % 4 == 0 && kOffOffs % 4 == 0 && kOffCounts % 4 == 0, "alignment");
 // a plant word no site is in range of (cell (0, 0), squared norm 8191): pads the plant list to a multiple of four on compact maps
 constexpr uint32_t kPlantSentinel = (63u << 16) | (127u << 24);
@@ -169,22 +148,14 @@ __device__ __forceinline__ int dp2a_lo_su(uint32_t a, uint32_t b, int c) {
 // keeps it for the tables that are re-read (type, year and plant terms, site opinions, policy constants): +1 % / +1.8 % (initial /
 // trained table, profiles/r02_eval_loop.md)
 __device__ __forceinline__ double2 ldg_stream(const double2* p) {
-#ifndef EG_WALK_ALLOCATE
   double2 v;
   asm volatile("ld.global.nc.L1::no_allocate.v2.f64 {%0, %1}, [%2];" : "=d"(v.x), "=d"(v.y) : "l"(p));
   return v;
-#else
-  return __ldg(p);
-#endif
 }
 __device__ __forceinline__ int ldg_stream(const uint16_t* p) {
-#ifndef EG_WALK_ALLOCATE
   unsigned short v;
   asm volatile("ld.global.nc.L1::no_allocate.u16 %0, [%1];" : "=h"(v) : "l"(p));
   return (int)v;
-#else
-  return (int)__ldg(p);
-#endif
 }
 
 // keeps a value in a register: the compiler may not re-derive it from its definition inside the hot loops
@@ -263,7 +234,7 @@ __device__ __forceinline__ int deficit_key_action(int k) {
 // no replay-best mode, count weights present — with the plain sampler (iterations_without_improvement <= 500) or the
 // stagnation sampler (> 500) compiled in alone. EG_OPT(x) is x in the general instantiation and false in the lean ones.
 #define EG_OPT(x) (!LEAN && (x))
-// GEOM (EgDeviceMap::near_geom): 0 compact map (at most 64 sites per axis), 1 medium (at most 181; blocks of 8 warps around a
+// GEOM (EgDeviceMap::near_geom): 0 compact map (at most 64 sites per axis), 1 medium (at most 181; blocks of 10 warps around a
 // factor table of up to 5,600 entries), 2 general (at most 256 sites per axis, factor table read from global memory).
 template <bool REPLAY, int GEOM, int MODE>
 struct Warp {
@@ -283,9 +254,6 @@ struct Warp {
   uint32_t n_gens, n_offs, flags;
   uint32_t ep;                // index of the episode in the batch (output slot)
   uint32_t rec_used;          // slots of the action record written so far (all years)
-#ifdef EG_WALK_STATS
-  uint32_t dbg_steps, dbg_evals, dbg_cands, dbg_pairs;
-#endif
   bool rows_dirty, dw_dirty, sorted_valid, total_valid;
   bool folded;                // this year's plant/offset sums (op_sum, gcost, ocost, off_amount) are valid
   // Philox: lane l holds draw number rbase + l of episode `rng_id`
@@ -411,7 +379,6 @@ struct Warp {
     }
   }
 
-#ifndef EG_NO_STASH
   // the episode's running sums and the deficit handler's current state wait in shared memory while the placement walk runs, so the
   // walk has their 26 registers
   __device__ __forceinline__ void stash(const State& cur, double remaining) {
@@ -434,7 +401,6 @@ struct Warp {
     cur.net = lds_v(a + 64); cur.opinion = lds_v(a + 72); cur.balance = lds_v(a + 80); cur.cost = lds_v(a + 88); remaining = lds_v(a + 96);
     __syncwarp();  // every lane has its copy before lane 0 may write the slots again
   }
-#endif
   __device__ __forceinline__ State state(int y) const {  // simulation.rs:122-135
     State s;
     s.net = co2 - off_amount;
@@ -488,12 +454,6 @@ struct Warp {
         sp_next = make_double2(0.0, 0.0);
         if (left > 0) { sp_next = ldg_stream(wp); packed_next = ldg_stream(op); }
       }
-#ifdef EG_WALK_STATS
-      dbg_steps++;
-      dbg_evals++;
-      dbg_cands += __popc(__ballot_sync(kFull, cand));
-      dbg_pairs += n_gens;
-#endif
       // survivors multiply their factors in plant order (== multiplication order of the reference), one site per lane
       double sc = pre;
       if (GEOM == 0) {
@@ -508,30 +468,18 @@ struct Warp {
         // No predicates: a plant out of range reads the 1.0 that ends the class's factors (x * 1.0 == x bit for bit), so the
         // four lookups of a group are in flight together and only the multiplications wait for each other. (Lanes out of the
         // race multiply along; their result is not looked at.) Measured alternatives, all with identical outputs
-        // (profiles/r02_eval_loop.md): predicated lookups, a two-stage software pipeline, unrolling by 1, 3 and 4.
+        // (profiles/r02_eval_loop.md): predicated lookups as on medium maps (-3.5 % on the shipped map), a two-stage software
+        // pipeline, unrolling by 1, 3 and 4, 16 lane-private copies of the table (no bank conflicts, but 3-6 % slower: less L1).
         const int lim = nf_off + r2lim;
-        constexpr int kUnroll = EG_EVAL_UNROLL_STAGNATION > 0 && MODE == 2 ? EG_EVAL_UNROLL_STAGNATION : kEvalUnroll;
-        constexpr uint32_t kStride = 8u * kTableCopies;
-        const uint32_t nf_lane = nf_base + 8u * ((uint32_t)lane & (kTableCopies - 1));
+        constexpr int kUnroll = MODE == 2 ? kEvalUnrollStagnation : kEvalUnroll;
 #pragma unroll kUnroll
         for (uint32_t q = 0; q < groups; q++) {
           const uint4 w4 = g4[q];
-#if EG_LOOKUP_PREDICATED & 1
-          // only lanes in range touch the table (fewer shared-memory wavefronts); the others multiply by a register 1.0
-          const int d0 = __dp4a((int)sa, (int)w4.x, sq), d1 = __dp4a((int)sa, (int)w4.y, sq);
-          const int d2 = __dp4a((int)sa, (int)w4.z, sq), d3 = __dp4a((int)sa, (int)w4.w, sq);
-          double f0 = 1.0, f1 = 1.0, f2 = 1.0, f3 = 1.0;
-          if (d0 < lim) f0 = lds_f64(nf_lane + kStride * (uint32_t)d0);
-          if (d1 < lim) f1 = lds_f64(nf_lane + kStride * (uint32_t)d1);
-          if (d2 < lim) f2 = lds_f64(nf_lane + kStride * (uint32_t)d2);
-          if (d3 < lim) f3 = lds_f64(nf_lane + kStride * (uint32_t)d3);
-#else
           const int d0 = min(__dp4a((int)sa, (int)w4.x, sq), lim), d1 = min(__dp4a((int)sa, (int)w4.y, sq), lim);
           const int d2 = min(__dp4a((int)sa, (int)w4.z, sq), lim), d3 = min(__dp4a((int)sa, (int)w4.w, sq), lim);
           EG_CHECK(d0 >= nf_off && d1 >= nf_off && d2 >= nf_off && d3 >= nf_off);
-          const double f0 = lds_f64(nf_lane + kStride * (uint32_t)d0), f1 = lds_f64(nf_lane + kStride * (uint32_t)d1);
-          const double f2 = lds_f64(nf_lane + kStride * (uint32_t)d2), f3 = lds_f64(nf_lane + kStride * (uint32_t)d3);
-#endif
+          const double f0 = lds_f64(nf_base + 8u * (uint32_t)d0), f1 = lds_f64(nf_base + 8u * (uint32_t)d1);
+          const double f2 = lds_f64(nf_base + 8u * (uint32_t)d2), f3 = lds_f64(nf_base + 8u * (uint32_t)d3);
           sc *= f0;  // score *= distance / penalty_radius, in plant order
           sc *= f1;
           sc *= f2;
@@ -540,7 +488,10 @@ struct Warp {
       } else if (GEOM == 1) {
         // up to 181 sites per axis (|g|^2 fits 16 bits): the plant word is cell | |g|^2 << 16, and
         // |s - g|^2 = (|s|^2 - 2 s.g) + |g|^2 is one IDP.2A (16-bit (-2 sj, -2 si) times the word's two low bytes) and one add
-        // of the word's high half; same groups of four, same unpredicated lookups as on compact maps
+        // of the word's high half; same groups of four as on compact maps, but predicated lookups: only the lanes in range read
+        // the table, the others multiply by a register 1.0. On the 10x grid the shared-memory pipe is the limiter (97 % busy,
+        // half of its wavefronts bank conflicts of the random lookups), and fewer wavefronts are +3.4 % there
+        // (profiles/r02_eval_loop.md).
         const int si = packed >> 8, sj = packed & 0xFF;
         const uint32_t sa = ((uint32_t)(-2 * sj) & 0xFFFFu) | ((uint32_t)(-2 * si) << 16);
         const int sq = si * si + sj * sj + nf_off;
@@ -550,7 +501,6 @@ struct Warp {
 #pragma unroll kEvalUnroll
         for (uint32_t q = 0; q < groups; q++) {
           const uint4 w4 = g4[q];
-#if EG_LOOKUP_PREDICATED & 2
           const int d0 = dp2a_lo_su(sa, w4.x, sq) + (int)(w4.x >> 16), d1 = dp2a_lo_su(sa, w4.y, sq) + (int)(w4.y >> 16);
           const int d2 = dp2a_lo_su(sa, w4.z, sq) + (int)(w4.z >> 16), d3 = dp2a_lo_su(sa, w4.w, sq) + (int)(w4.w >> 16);
           double f0 = 1.0, f1 = 1.0, f2 = 1.0, f3 = 1.0;
@@ -558,13 +508,6 @@ struct Warp {
           if (d1 < lim) f1 = lds_f64(nf_base + 8u * (uint32_t)d1);
           if (d2 < lim) f2 = lds_f64(nf_base + 8u * (uint32_t)d2);
           if (d3 < lim) f3 = lds_f64(nf_base + 8u * (uint32_t)d3);
-#else
-          const int d0 = min(dp2a_lo_su(sa, w4.x, sq) + (int)(w4.x >> 16), lim), d1 = min(dp2a_lo_su(sa, w4.y, sq) + (int)(w4.y >> 16), lim);
-          const int d2 = min(dp2a_lo_su(sa, w4.z, sq) + (int)(w4.z >> 16), lim), d3 = min(dp2a_lo_su(sa, w4.w, sq) + (int)(w4.w >> 16), lim);
-          EG_CHECK(d0 >= nf_off && d1 >= nf_off && d2 >= nf_off && d3 >= nf_off);
-          const double f0 = lds_f64(nf_base + 8u * (uint32_t)d0), f1 = lds_f64(nf_base + 8u * (uint32_t)d1);
-          const double f2 = lds_f64(nf_base + 8u * (uint32_t)d2), f3 = lds_f64(nf_base + 8u * (uint32_t)d3);
-#endif
           sc *= f0;  // score *= distance / penalty_radius, in plant order
           sc *= f1;
           sc *= f2;
@@ -647,15 +590,9 @@ struct Warp {
   }
   // the rows of year y are complete (requested a year earlier); request those of year y+1
   __device__ __forceinline__ void load_rows(int y) {
-#ifdef EG_ROWS_SYNC
-    double* lw = LW(y);
-    for (int k = lane; k < EG_POLICY_ROW; k += 32) lw[k] = __ldg(&p.policy->rows[y][k]);
-    __syncwarp();
-#else
     asm volatile("cp.async.wait_group 0;" ::: "memory");
     __syncwarp();
     if (y + 1 < EG_NY) prefetch_rows(y + 1);
-#endif
     rows_dirty = false; dw_dirty = false; sorted_valid = false; total_valid = false;
     if (stagnation()) {  // the snapshot's sorted, scaled row of this year (host libm) for the stagnation sampler
       double* scl = (double*)(smem + sb + kOffScratch);
@@ -802,7 +739,6 @@ struct Warp {
       return (smem + sb + kOffSortIdx)[0];
     }
     double rv = f64() * total;
-#ifndef EG_SCAN_SEQUENTIAL
     {
       // Decide the scan from a warp-parallel prefix sum when no partial sum comes near
       // the draw. The sequential chain rv_k = fl(rv_{k-1} - w_k) and the tree sums S_k both differ from the exact
@@ -829,7 +765,6 @@ struct Warp {
         return min(f0, f1);
       }
     }
-#endif
     #pragma unroll kScanUnroll
     for (int k = 0; k < EG_N_ACTIONS; k++) {
       rv -= lw[k];
@@ -855,18 +790,13 @@ struct Warp {
     rng_id = p.same_stream ? 0ull : p.first_episode + ep;
     draw = 0; rbase = 0x80000000u; rbuf = 0ull;
     n_gens = 0; n_offs = 0; flags = 0;
-#ifdef EG_WALK_STATS
-    dbg_steps = dbg_evals = dbg_cands = dbg_pairs = 0;
-#endif
     gcost = 0.0; ocost = 0.0; gen0 = gen1 = gen2 = 0.0; co2 = 0.0;
     __syncwarp();
     const eg_traj* in = REPLAY ? p.replay_in + ep : nullptr;
     uint32_t n_def_total = 0, n_add_total = 0;
     double* vars = VARS();
     const bool learn = !REPLAY && !EG_OPT(p.replay_best);
-#ifndef EG_ROWS_SYNC
     if (!REPLAY) prefetch_rows(0);
-#endif
 
     for (int y = 0; y < EG_NY; y++) {
       year_start(y);
@@ -939,13 +869,9 @@ struct Warp {
         int site = -1;
         if (action < 45) {                                   // apply_action, actions.rs:42-76
           const int t = action / 3, m = action - 3 * t;
-#ifndef EG_NO_STASH
           stash(cur, remaining);
           const int cell = place(t, y);
           unstash(cur, remaining);
-#else
-          const int cell = place(t, y);
-#endif
           if (cell < 0) flags |= EG_FLAG_NO_SITE;
           else {
             site = (cell >> 8) * p.map.grid_n + (cell & 0xFF);
@@ -1071,12 +997,7 @@ struct Warp {
         case 4: word = (unsigned long long)__double_as_longlong(r_rel); break;
         case 5: word = (unsigned long long)n_gens | ((unsigned long long)n_offs << 32); break;
         case 6: word = (unsigned long long)(n_def_total & 0xFFFFu) | ((unsigned long long)(n_add_total & 0xFFFFu) << 16) | ((unsigned long long)flags << 32); break;
-#ifdef EG_WALK_STATS
-        // debug build: walk statistics instead of the reserved word (steps | evaluation steps << 16 | candidates << 32 | plant iterations / 16 << 48)
-        default: word = (unsigned long long)(dbg_steps & 0xFFFF) | ((unsigned long long)(dbg_evals & 0xFFFF) << 16) | ((unsigned long long)(dbg_cands & 0xFFFF) << 32) | ((unsigned long long)((dbg_pairs >> 4) & 0xFFFF) << 48); break;
-#else
         default: word = 0ull; break;
-#endif
       }
       ((unsigned long long*)(p.out + ep))[lane] = word;
     }
@@ -1100,14 +1021,18 @@ struct Warp {
   }
 };
 
-// blocks of 4 warps x 5 per SM, or (medium maps: one larger factor table per block) 10 warps x 2: 20 warps per SM, register cap 96
+// Blocks of 4 warps x 5 per SM, or (medium maps: one larger factor table per block) 10 warps x 2: 20 warps per SM, register cap 96.
+// The placement evaluation keeps four table lookups in flight per group of plants and needs ~115 registers to be scheduled that way
+// with the episode's state in registers; the state (13 doubles) therefore waits in shared memory while the placement walk runs
+// (Warp::stash), which brings the kernel to 94 registers without spills and 20 warps per SM: 3.15 ms per 65,536 episodes against
+// 3.39 ms with 4 blocks at 118 registers and 3.55 ms with 5 blocks and no stash (profiles/r02_eval_loop.md).
 template <int GEOM> struct Shape {
-  static constexpr bool kLarge = GEOM == 1 || (GEOM == 0 && kTableCopies > 1);  // one large table per block: fewer, larger blocks
-#ifndef EG_LARGE_WARPS
-#define EG_LARGE_WARPS (EG_EPISODE_WARPS * EG_EPISODE_MIN_BLOCKS / 2)
-#endif
-  static constexpr int kWarps = kLarge ? EG_LARGE_WARPS : EG_EPISODE_WARPS, kMinBlocks = kLarge ? 2 : EG_EPISODE_MIN_BLOCKS;
+  static constexpr int kWarps = GEOM == 1 ? 10 : 4, kMinBlocks = GEOM == 1 ? 2 : 5;
 };
+// kMinBlocks blocks fit in the 227 KB of shared memory of an SM with the largest factor table near_geom admits (the general form
+// has none); the system reserves 1 KB per block
+static_assert(Shape<0>::kMinBlocks * (Shape<0>::kWarps * kSliceBytes + 8 * EG_COMPACT_MAX_FACTORS + 1024) <= 227 * 1024, "compact maps");
+static_assert(Shape<1>::kMinBlocks * (Shape<1>::kWarps * kSliceBytes + 8 * EG_MEDIUM_MAX_FACTORS + 1024) <= 227 * 1024, "medium maps");
 
 template <bool REPLAY, int GEOM, int MODE>
 __global__ void __launch_bounds__(32 * Shape<GEOM>::kWarps, Shape<GEOM>::kMinBlocks) eg_episode_kernel(const __grid_constant__ EgEpisodeParams p, int slice_bytes, int table_bytes) {
@@ -1116,11 +1041,8 @@ __global__ void __launch_bounds__(32 * Shape<GEOM>::kWarps, Shape<GEOM>::kMinBlo
     double* nf_s = (double*)smem;  // compact: class rc holds its r2_limit[rc] entries from offset r2_limit[6 + rc], then a 1.0
     for (int rc = 0; rc < EG_N_RCLASS; rc++) {
       const int cnt = __ldg(&p.map.r2_limit[rc]), off = __ldg(&p.map.r2_limit[EG_N_RCLASS + rc]);
-      const int copies = GEOM == 0 ? kTableCopies : 1;
-      for (int i = threadIdx.x; i < (cnt + 1) * copies; i += blockDim.x) {
-        const int e = i / copies;
-        nf_s[(off + e) * copies + (i - e * copies)] = e < cnt ? __ldg(&p.map.near_factor[rc * p.map.r2_stride + e]) : 1.0;
-      }
+      for (int i = threadIdx.x; i < cnt + 1; i += blockDim.x)
+        nf_s[off + i] = i < cnt ? __ldg(&p.map.near_factor[rc * p.map.r2_stride + i]) : 1.0;
     }
     __syncthreads();
   }
@@ -1138,13 +1060,9 @@ __global__ void __launch_bounds__(32 * Shape<GEOM>::kWarps, Shape<GEOM>::kMinBlo
 
 template <bool REPLAY, int GEOM, int MODE>
 cudaError_t launch_as(const EgEpisodeParams& p, cudaStream_t stream) {
-  const bool wide = GEOM == 2;
-  const int slice = kSliceBytes;
-  const int shared_tab = wide ? 0 : (p.nf_entries * (int)sizeof(double) * (GEOM == 0 ? kTableCopies : 1) + 15) & ~15;
-  // as many warps per block as keep several blocks resident in the 227 KB of an SM
-  int warps = Shape<GEOM>::kWarps;
-  while (warps > 1 && (size_t)Shape<GEOM>::kMinBlocks * (warps * slice + shared_tab + 1024) > 227 * 1024) warps >>= 1;
-  const size_t smem_bytes = (size_t)warps * slice + shared_tab;
+  constexpr int warps = Shape<GEOM>::kWarps;
+  const int shared_tab = GEOM == 2 ? 0 : (p.nf_entries * (int)sizeof(double) + 15) & ~15;
+  const size_t smem_bytes = (size_t)warps * kSliceBytes + shared_tab;
   if (smem_bytes > 227 * 1024) return cudaErrorInvalidConfiguration;
   // function attributes and the occupancy query are per (device, shared-memory size): done once, then cached
   struct Cached { size_t smem = 0; int resident = 0; };
@@ -1157,9 +1075,8 @@ cudaError_t launch_as(const EgEpisodeParams& p, cudaStream_t stream) {
   if (shape.smem != smem_bytes || shape.resident == 0) {
     err = cudaFuncSetAttribute(eg_episode_kernel<REPLAY, GEOM, MODE>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_bytes);
     if (err != cudaSuccess) return err;
-    // shared-memory carveout: room for as many blocks as the register budget allows, the rest stays L1
-    const int resident_want = (int)std::min<size_t>(Shape<GEOM>::kMinBlocks * (Shape<GEOM>::kWarps / warps), (227 * 1024) / (smem_bytes + 1024));
-    const int carveout = std::min(100, (int)((resident_want * (smem_bytes + 1024) * 100 + 228 * 1024 - 1) / (228 * 1024)));
+    // shared-memory carveout: room for the kMinBlocks blocks the register budget allows, the rest stays L1
+    const int carveout = std::min(100, (int)((Shape<GEOM>::kMinBlocks * (smem_bytes + 1024) * 100 + 228 * 1024 - 1) / (228 * 1024)));
     cudaFuncSetAttribute(eg_episode_kernel<REPLAY, GEOM, MODE>, cudaFuncAttributePreferredSharedMemoryCarveout, carveout);
     // grid = every block the device can hold at once (a multiple of the SM count), never more warps than episodes
     int sms = 0, per_sm = 0;
@@ -1174,7 +1091,7 @@ cudaError_t launch_as(const EgEpisodeParams& p, cudaStream_t stream) {
   if (blocks == 0) return cudaErrorInvalidConfiguration;
   err = cudaMemsetAsync(p.next_episode, 0, sizeof(uint32_t), stream);
   if (err != cudaSuccess) return err;
-  eg_episode_kernel<REPLAY, GEOM, MODE><<<blocks, 32 * warps, smem_bytes, stream>>>(p, slice, shared_tab);
+  eg_episode_kernel<REPLAY, GEOM, MODE><<<blocks, 32 * warps, smem_bytes, stream>>>(p, kSliceBytes, shared_tab);
   return cudaGetLastError();
 }
 

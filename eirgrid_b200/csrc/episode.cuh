@@ -25,17 +25,5 @@ struct EgEpisodeParams {
   double ln100;                  // ln(MAX_ACCEPTABLE_COST*100/MAX_ACCEPTABLE_COST), host libm (scoring.rs:13,32)
 };
 
-#ifndef EG_EPISODE_WARPS
-#define EG_EPISODE_WARPS 4   // episodes (warps) per block for the Irish map; fewer when the per-warp slice is large
-#endif
-#ifndef EG_EPISODE_MIN_BLOCKS
-// 5 blocks of 4 warps: register cap 96. The placement evaluation keeps four table lookups in flight per group of plants and
-// needs ~115 registers to be scheduled that way with the episode's state in registers; the state (13 doubles) therefore waits in
-// shared memory while the placement walk runs (Warp::stash), which brings the kernel to 94 registers without spills and 20 warps
-// per SM: 3.15 ms per 65,536 episodes against 3.39 ms with 4 blocks at 118 registers and 3.55 ms with 5 blocks and no stash
-// (profiles/r02_eval_loop.md).
-#define EG_EPISODE_MIN_BLOCKS 5
-#endif
-
 cudaError_t eg_launch_rollout(const EgEpisodeParams& p, cudaStream_t stream);
 cudaError_t eg_launch_replay(const EgEpisodeParams& p, cudaStream_t stream);

@@ -411,10 +411,7 @@ void eg_host_build_tables(const EgHostMap& m, EgHostTables* out) {
   }
   {
     const int entries = out->r2_limit[2 * EG_N_RCLASS];
-    out->near_geom = (m.grid_n <= 64 && entries <= 2048) ? 0 : ((m.grid_n <= 181 && entries <= 5600) ? 1 : 2);
+    out->near_geom = (m.grid_n <= 64 && entries <= EG_COMPACT_MAX_FACTORS) ? 0 : ((m.grid_n <= 181 && entries <= EG_MEDIUM_MAX_FACTORS) ? 1 : 2);
   }
-#ifdef EG_GEOM_GENERAL  // A/B builds: every map through the general form
-  out->near_geom = 2;
-#endif
   (void)kRadius;
 }

@@ -12,6 +12,10 @@
 #define EG_NT EG_N_GEN_TYPES
 #define EG_N_RCLASS 6   // placement penalty radii 3,5,6,7,8,12 km (gpu/metal_location_search.rs:139-146)
 #define EG_N_PCLASS 7   // (radius, needs-coast-factor) combinations that occur among the 15 types
+// largest distance/radius factor table (all radius classes, each ending with its 1.0) of the forms that copy it into shared memory
+// (EgDeviceMap::near_geom); the episode kernel's block shapes are sized for them
+#define EG_COMPACT_MAX_FACTORS 2048  // compact form
+#define EG_MEDIUM_MAX_FACTORS 5600   // medium form
 
 // generation accumulator a plant's output is added to (map_handler.rs:852-865)
 enum { EG_ACC_PLAIN = 0, EG_ACC_INTERMITTENT = 1, EG_ACC_STORAGE = 2 };

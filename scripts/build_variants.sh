@@ -1,5 +1,5 @@
 #!/bin/bash
-# Build A/B variants of the library next to the default one:  scripts/build_variants.sh "tma:-DEG_ROWS_TMA" "scan:-DEG_SCAN_PARALLEL"
+# Build A/B variants of the library next to the default one:  scripts/build_variants.sh "bounds:-DEG_DEBUG_BOUNDS" "<name>:-D<switch>"
 # -> eirgrid_b200/libeg_<name>.so each (picked up by scripts/gpu_ab.sh, which times every libeg_*.so on both weight tables and
 # prints a hash of all outputs). Remove them with:  rm -f eirgrid_b200/libeg_*.so; rm -rf eirgrid_b200/build/libeg_*
 set -e
