@@ -120,6 +120,10 @@ def test_rollout_trained_weights_and_heuristic_counts(gpu_ctx, oracle_world):
     res, traj, sites, _ = gpu_ctx.rollout(gw, n, seed=5, want_sites=True)
     assert traj.tobytes() == etraj.tobytes()
     assert_results_equal(res, eres)
+    # without count weights the launch without optional outputs also takes the general form
+    res, traj, _, _ = gpu_ctx.rollout(gw, n, seed=5)
+    assert traj.tobytes() == etraj.tobytes()
+    assert_results_equal(res, eres)
 
 
 def test_same_stream_quirk_q8(gpu_ctx, oracle_world):
@@ -182,6 +186,10 @@ def test_rollout_stagnation_branch(gpu_ctx, oracle_world):
         # boundary would change one action; with 256 episodes x ~30 draws that has probability ~1e-12
         assert traj.tobytes() == etraj.tobytes()
         assert sites.tobytes() == esites.tobytes()
+        assert_results_equal(res, eres)
+        # the training launch (no optional outputs) runs the lean stagnation instantiation: same episodes
+        res, traj, _, _ = gpu_ctx.rollout(gw, 256, seed=32 + iwi)
+        assert traj.tobytes() == etraj.tobytes()
         assert_results_equal(res, eres)
 
 
@@ -290,6 +298,36 @@ def test_location_analysis_on_a_comb_coastline(oracle_world):
     ref = ctx.location_analysis(True, half_steps=50, step=1000.0, year_index=2).reshape(101, 101, 15)[50:, 50:].reshape(2601, 15)
     assert np.array_equal(sites[:, 2], ref)
     ctx.close()
+
+
+def test_suitability_rows_past_the_first_block(gpu_ctx, oracle_world):
+    """A block of the suitability kernel takes one site column j and 64 consecutive i; a 1,001-site grid has 16 such chunks,
+    the last one partial. Rows i on both sides of chunk boundaries, from one launch over the whole grid, against the oracle's
+    analysis of the same points (site (i, j) = analysis point (i + half) * (2 half + 1) + (j + half)): year 0 and year 25
+    (grown populations) on the shipped map, year 0 on the 10x map."""
+    from eirgrid_b200 import synthetic
+    side, half, step = 1001, 1000, 50.0
+    rows = (0, 63, 64, 127, 128, 999, 1000)
+
+    def check(ctx, world, year):
+        got = ctx.location_analysis_sites(True, side, step, year_first=year, n_years=1)[:, 0].reshape(side, side, 15)
+        for i in rows:
+            exp = world.location_analysis(True, half=half, step=step, first=(i + half) * (2 * half + 1) + half, n=side)
+            assert np.array_equal(got[i], exp), (year, i)
+
+    check(gpu_ctx, oracle_world, 0)
+    sx, sy, spop, ex, ey, et, ec, cx, cy = _ireland_arrays()
+    pop = spop.astype(np.float64)
+    for _ in range(25):
+        pop = np.floor(pop * 1.01 + 0.5)  # f64::round of positive values
+    check(gpu_ctx, O.World.from_arrays(sx, sy, pop.astype(np.uint32), ex, ey, et, ec, cx, cy, 51, 1000.0, fast=False), 25)
+    m = synthetic.scaled_map(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "ireland_map"), 10)
+    ctx = _lib.Context(0)
+    try:
+        ctx.map_set(*m)
+        check(ctx, O.World.from_arrays(*m, fast=False), 0)
+    finally:
+        ctx.close()
 
 
 def _ireland_arrays():

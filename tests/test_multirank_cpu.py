@@ -48,9 +48,9 @@ def _one_step(gw, ow, world, first, n_total, rank, world_size, use_dist):
     lo = first + offset
     res, traj, _, _ = world.rollout(ow, n_per_rank, seed=77, first_episode=lo, threads=2)
     t = gw.table()
-    consts = stats_ref.contrast_consts(t, stats_ref.default_score(*list(t.best_metrics)[:3]))
+    consts = stats_ref.contrast_consts(t)
     best, best_def = _best_lists(gw)
-    stats, scores = stats_ref.batch_stats(res, traj, consts, best, best_def)
+    stats, scores, _ = stats_ref.batch_stats(res, traj, consts, best, best_def)
     k = int(np.lexsort((np.arange(n_per_rank), -scores))[0])
     rec = T.pack_record(scores[k], lo + k, res[k:k + 1], traj[k:k + 1])
     pack = torch.from_numpy(T.pack_buffer(stats, rec))
@@ -90,9 +90,9 @@ def test_two_ranks_match_one_rank(tmp_path):
         from eirgrid_b200 import trainer as T
         res, traj, _, _ = world.rollout(ow, 65, seed=77, first_episode=first, threads=2)
         t = gw.table()
-        consts = stats_ref.contrast_consts(t, stats_ref.default_score(*list(t.best_metrics)[:3]))
+        consts = stats_ref.contrast_consts(t)
         best, best_def = _best_lists(gw)
-        stats, scores = stats_ref.batch_stats(res, traj, consts, best, best_def)
+        stats, scores, _ = stats_ref.batch_stats(res, traj, consts, best, best_def)
         k = int(np.lexsort((np.arange(65), -scores))[0])
         rec = T.pack_record(scores[k], first + k, res[k:k + 1], traj[k:k + 1])
         T.combine_and_apply(gw, stats, rec, 65, first)

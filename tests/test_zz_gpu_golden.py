@@ -46,5 +46,9 @@ def test_rollout_and_replay_equal_the_committed_vectors(gpu_ctx):
         assert hashlib.sha1(t2.tobytes()).digest() == g["iwi%d_traj_sha1" % iwi].tobytes(), iwi
         assert hashlib.sha1(s2.tobytes()).digest() == g["iwi%d_sites_sha1" % iwi].tobytes(), iwi
         _same_results(r2, g["iwi%d_results" % iwi])
+        if iwi > 500:  # the lean stagnation instantiation (no optional outputs): the same episodes
+            r3, t3, _, _ = gpu_ctx.rollout(w, 32, seed=7 + iwi, first_episode=1000)
+            assert hashlib.sha1(t3.tobytes()).digest() == g["iwi%d_traj_sha1" % iwi].tobytes(), iwi
+            _same_results(r3, g["iwi%d_results" % iwi])
     rr, _, _ = gpu_ctx.replay(g["initial_traj"][:8])
     _same_results(rr, g["replay_results"])
