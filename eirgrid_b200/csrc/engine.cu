@@ -3,18 +3,14 @@
 // EG_ERR_NO_DEVICE / EG_ERR_CUDA otherwise.
 #include <cuda_runtime.h>
 #include <cmath>
-#include <sys/stat.h>
-#include <sys/types.h>
-#include <cstdio>
-#include <cstdlib>
 #include <cstring>
-#include <ctime>
+#include <memory>
 #include <string>
 #include <vector>
 #include "common.hpp"
+#include "device_buffer.hpp"
 #include "episode.cuh"
 #include "host_tables.hpp"
-#include "json_min.hpp"
 #include "site_tables.cuh"
 #include "stats.cuh"
 #include "suitability.cuh"
@@ -38,7 +34,7 @@ int eg_fail(int code, const std::string& message) {
 struct eg_ctx {
   int device = 0;
   cudaStream_t stream = nullptr;
-  bool own_stream = false;
+  OwnedStream own_stream;              // set when eg_init created the stream; a stream passed in stays the caller's
   uint64_t launches = 0;
   bool map_ready = false;
   bool policy_ready = false;
@@ -46,176 +42,154 @@ struct eg_ctx {
   bool policy_stagnation = false;
   EgHostMap hmap;
   EgHostTables htab;
-  // device memory
-  EgSmallTables* d_small = nullptr;
-  double* d_plant_terms = nullptr;
-  double* d_site_opinion = nullptr;
-  double* d_coast = nullptr;
-  double* d_prefix = nullptr;          // [6][26][ns]
-  double* d_static_unsorted = nullptr; // [7][26][ns]
-  uint16_t* d_order = nullptr;
-  double* d_static_sorted = nullptr;
-  double* d_prefix_sorted = nullptr;
-  double* d_walk = nullptr;            // [7][26][ns][2]
-  double* d_near = nullptr;
-  int* d_r2_limit = nullptr;
-  double *d_sx = nullptr, *d_sy = nullptr, *d_ex = nullptr, *d_ey = nullptr, *d_cx = nullptr, *d_cy = nullptr;
-  uint32_t* d_pop = nullptr;
-  double* d_suit_rows = nullptr;       // scratch of the suitability kernel: crossing lists per site row
-  size_t suit_rows_cap = 0;
-  double* d_urban_r = nullptr;         // [26][S] sqrt(pop) * 5 (is_urban_area, map_handler.rs:1199-1209)
-  double urban_r_max = 0.0;
-  EgPolicyDevice* d_policy = nullptr;
-  EgPolicyDevice* h_policy[2] = {nullptr, nullptr};   // pinned staging of the snapshot, used in turn
-  cudaEvent_t policy_copied[2] = {nullptr, nullptr};  // the H2D copy issued from h_policy[b] has completed
+  EgDeviceMap dmap{};
+  // Device memory in groups that live equally long, each allocated all or nothing: built in a local and moved in only when
+  // every allocation succeeded, so a failed call leaves the group absent and the next call allocates it again.
+  struct MapTables {  // the loaded map (build_device_map)
+    DeviceArray<EgSmallTables> small;
+    DeviceArray<double> plant_terms, near, sx, sy, ex, ey, cx, cy, site_opinion, coast;
+    DeviceArray<double> prefix, walk;  // [6][26][ns], [7][26][ns][2]
+    DeviceArray<uint16_t> order;       // [7][26][ns]
+    DeviceArray<int> r2_limit;
+    DeviceArray<uint32_t> pop;
+    DeviceArray<double> urban_r;       // [26][S] sqrt(pop) * 5 (is_urban_area, map_handler.rs:1199-1209)
+    double urban_r_max = 0.0;
+  } map;
+  struct PolicyBuffers {  // the weights snapshot the rollouts read
+    DeviceArray<EgPolicyDevice> d;
+    PinnedArray<EgPolicyDevice> h[2];  // pinned staging of the snapshot, used in turn
+    Event copied[2];                   // the H2D copy issued from h[b] has completed
+  } policy;
   int policy_turn = 0;
-  uint32_t* d_next_episode = nullptr;  // work counter of the persistent episode kernels
-  // eg_train_batch_*: statistics table, shard best, winner record (device) and their pinned host mirrors
-  int64_t* d_stats = nullptr;
-  double* d_best_score = nullptr;
-  unsigned long long* d_best_index = nullptr;
-  unsigned char* d_record = nullptr;
-  int64_t* h_stats = nullptr;
-  unsigned char* h_record = nullptr;
+  struct Scratch {  // outputs of the host-buffer entry points, each grown on demand
+    DeviceArray<eg_result> out;
+    DeviceArray<eg_traj> traj, traj_in;
+    DeviceArray<eg_sites> sites;
+    DeviceArray<eg_yearly> yearly;
+  } scratch;
+  struct TrainBuffers {  // eg_train_batch_*: statistics table, shard best, winner record (device) and their pinned host mirrors
+    DeviceArray<int64_t> stats;
+    DeviceArray<double> best_score;
+    DeviceArray<unsigned long long> best_index;
+    DeviceArray<unsigned char> record;
+    PinnedArray<int64_t> h_stats;
+    PinnedArray<unsigned char> h_record;
+  } train;
   uint32_t train_n = 0;
   bool train_pending = false;
-  // eg_update_device: scratch of the in-order update (update.cu) and its pinned host mirrors
-  EgUpdBuffers upd{};
-  EgUpdState* h_upd_state = nullptr;
-  EgUpdSlot* h_upd_slot = nullptr;
-  EgUpdImprovement* h_upd_imp = nullptr;
-  EgDeviceMap dmap{};
-  // scratch for the host-buffer entry points
-  size_t cap = 0;
-  eg_result* s_out = nullptr;
-  eg_traj* s_traj = nullptr;
-  eg_traj* s_traj_in = nullptr;
-  eg_sites* s_sites = nullptr;
-  eg_yearly* s_yearly = nullptr;
-  size_t cap_yearly = 0, cap_sites = 0, cap_traj_in = 0;
+  struct UpdateBuffers {  // eg_update_device: scratch of the in-order update (update.cu) and its pinned host mirrors
+    DeviceArray<EgUpdState> state;
+    DeviceArray<EgUpdSlot> slots;
+    DeviceArray<double> score, factors;
+    DeviceArray<EgUpdPre> pre;
+    DeviceArray<EgUpdCtl> ctl;
+    DeviceArray<uint8_t> counts;
+    PinnedArray<EgUpdState> h_state;
+    PinnedArray<EgUpdSlot> h_slot;
+    PinnedArray<EgUpdImprovement> h_imp;
+  } upd;
+  DeviceArray<EgUpdImprovement> upd_improvements;  // grown with the batch, at least EG_UPD_IMP_INLINE
+  DeviceArray<double> suit_rows;       // scratch of the suitability kernel: crossing lists per site row
+  DeviceArray<uint32_t> next_episode;  // work counter of the persistent episode kernels
 };
 
 namespace {
 
-void free_map(eg_ctx* c) {
-  void* ptrs[] = {c->d_small, c->d_plant_terms, c->d_site_opinion, c->d_coast, c->d_prefix, c->d_static_unsorted, c->d_order,
-                  c->d_static_sorted, c->d_prefix_sorted, c->d_walk, c->d_near, c->d_r2_limit, c->d_sx, c->d_sy, c->d_ex, c->d_ey, c->d_cx, c->d_cy, c->d_pop, c->d_urban_r};
-  for (void* p : ptrs)
-    if (p) cudaFree(p);
-  c->d_urban_r = nullptr;
-  c->d_small = nullptr; c->d_plant_terms = nullptr; c->d_site_opinion = nullptr; c->d_coast = nullptr; c->d_prefix = nullptr;
-  c->d_static_unsorted = nullptr; c->d_order = nullptr; c->d_static_sorted = nullptr; c->d_prefix_sorted = nullptr; c->d_walk = nullptr;
-  c->d_near = nullptr; c->d_r2_limit = nullptr; c->d_sx = c->d_sy = c->d_ex = c->d_ey = c->d_cx = c->d_cy = nullptr; c->d_pop = nullptr;
-  c->map_ready = false;
-}
+// ln(MAX_ACCEPTABLE_COST * 100 / MAX_ACCEPTABLE_COST) of the score, host libm (scoring.rs:13,32)
+const double kLn100 = std::log(50000000000.0 * 100.0 / 50000000000.0);
+
+// makes the context's device current: every entry point that touches device memory calls this before its first CUDA call
+cudaError_t use_device(const eg_ctx* c) { return cudaSetDevice(c->device); }
 
 template <typename T>
-int upload(T** dst, const T* src, size_t n, cudaStream_t s) {
+int upload(DeviceArray<T>& dst, const T* src, size_t n, cudaStream_t s) {
   // two spare elements, zeroed: the suitability kernel stages these arrays with bulk copies in 16-byte units
-  EG_CUDA(cudaMalloc((void**)dst, (n + 2) * sizeof(T)));
-  EG_CUDA(cudaMemsetAsync(*dst, 0, (n + 2) * sizeof(T), s));
-  if (n) EG_CUDA(cudaMemcpyAsync(*dst, src, n * sizeof(T), cudaMemcpyHostToDevice, s));
+  EG_CUDA(dst.alloc(n + 2));
+  EG_CUDA(cudaMemsetAsync(dst.get(), 0, (n + 2) * sizeof(T), s));
+  if (n) EG_CUDA(cudaMemcpyAsync(dst.get(), src, n * sizeof(T), cudaMemcpyHostToDevice, s));
   return EG_OK;
 }
 
 int build_device_map(eg_ctx* c) {
   int rc = eg_host_map_validate(c->hmap);
   if (rc) return rc;
-  EG_CUDA(cudaSetDevice(c->device));
-  free_map(c);
+  EG_CUDA(use_device(c));
+  c->map = eg_ctx::MapTables();  // the old tables go first
+  c->map_ready = false;
   eg_host_build_tables(c->hmap, &c->htab);
   const EgHostMap& m = c->hmap;
   const int ns = m.grid_n * m.grid_n;
+  const size_t n_lists = (size_t)EG_N_PCLASS * EG_NY * ns;
   cudaStream_t s = c->stream;
-  if ((rc = upload(&c->d_small, &c->htab.small, 1, s))) return rc;
-  if ((rc = upload(&c->d_plant_terms, c->htab.plant_terms.data(), c->htab.plant_terms.size(), s))) return rc;
-  if ((rc = upload(&c->d_near, c->htab.near_factor.data(), c->htab.near_factor.size(), s))) return rc;
-  if ((rc = upload(&c->d_r2_limit, c->htab.r2_limit, (size_t)(2 * EG_N_RCLASS + 1), s))) return rc;
-  if ((rc = upload(&c->d_sx, m.sx.data(), m.sx.size(), s))) return rc;
-  if ((rc = upload(&c->d_sy, m.sy.data(), m.sy.size(), s))) return rc;
-  if ((rc = upload(&c->d_ex, m.ex.data(), m.ex.size(), s))) return rc;
-  if ((rc = upload(&c->d_ey, m.ey.data(), m.ey.size(), s))) return rc;
-  if ((rc = upload(&c->d_cx, m.cx.data(), m.cx.size(), s))) return rc;
-  if ((rc = upload(&c->d_cy, m.cy.data(), m.cy.size(), s))) return rc;
-  if ((rc = upload(&c->d_pop, c->htab.pop.data(), c->htab.pop.size(), s))) return rc;
+  eg_ctx::MapTables t;
+  if ((rc = upload(t.small, &c->htab.small, 1, s))) return rc;
+  if ((rc = upload(t.plant_terms, c->htab.plant_terms.data(), c->htab.plant_terms.size(), s))) return rc;
+  if ((rc = upload(t.near, c->htab.near_factor.data(), c->htab.near_factor.size(), s))) return rc;
+  if ((rc = upload(t.r2_limit, c->htab.r2_limit, (size_t)(2 * EG_N_RCLASS + 1), s))) return rc;
+  if ((rc = upload(t.sx, m.sx.data(), m.sx.size(), s))) return rc;
+  if ((rc = upload(t.sy, m.sy.data(), m.sy.size(), s))) return rc;
+  if ((rc = upload(t.ex, m.ex.data(), m.ex.size(), s))) return rc;
+  if ((rc = upload(t.ey, m.ey.data(), m.ey.size(), s))) return rc;
+  if ((rc = upload(t.cx, m.cx.data(), m.cx.size(), s))) return rc;
+  if ((rc = upload(t.cy, m.cy.data(), m.cy.size(), s))) return rc;
+  if ((rc = upload(t.pop, c->htab.pop.data(), c->htab.pop.size(), s))) return rc;
   {
     std::vector<double> urban_r(c->htab.pop.size());
-    c->urban_r_max = 0.0;
     for (size_t i = 0; i < urban_r.size(); i++) {
       urban_r[i] = std::sqrt((double)c->htab.pop[i]) * 5.0;
-      c->urban_r_max = std::max(c->urban_r_max, urban_r[i]);
+      t.urban_r_max = std::max(t.urban_r_max, urban_r[i]);
     }
-    if ((rc = upload(&c->d_urban_r, urban_r.data(), urban_r.size(), s))) return rc;
+    if ((rc = upload(t.urban_r, urban_r.data(), urban_r.size(), s))) return rc;
     EG_CUDA(cudaStreamSynchronize(s));  // urban_r is a local
   }
-  EG_CUDA(cudaMalloc((void**)&c->d_site_opinion, ns * sizeof(double)));
-  EG_CUDA(cudaMalloc((void**)&c->d_coast, ns * sizeof(double)));
-  EG_CUDA(cudaMalloc((void**)&c->d_prefix, (size_t)EG_N_RCLASS * EG_NY * ns * sizeof(double)));
-  EG_CUDA(cudaMalloc((void**)&c->d_static_unsorted, (size_t)EG_N_PCLASS * EG_NY * ns * sizeof(double)));
-  EG_CUDA(cudaMalloc((void**)&c->d_order, (size_t)EG_N_PCLASS * EG_NY * ns * sizeof(uint16_t)));
-  EG_CUDA(cudaMalloc((void**)&c->d_static_sorted, (size_t)EG_N_PCLASS * EG_NY * ns * sizeof(double)));
-  EG_CUDA(cudaMalloc((void**)&c->d_prefix_sorted, (size_t)EG_N_PCLASS * EG_NY * ns * sizeof(double)));
-  EG_CUDA(cudaMalloc((void**)&c->d_walk, (size_t)EG_N_PCLASS * EG_NY * ns * 2 * sizeof(double)));
+  DeviceArray<double> static_unsorted;  // [7][26][ns] static scores before the sort, needed by the build only
+  EG_CUDA(t.site_opinion.alloc(ns));
+  EG_CUDA(t.coast.alloc(ns));
+  EG_CUDA(t.prefix.alloc((size_t)EG_N_RCLASS * EG_NY * ns));
+  EG_CUDA(static_unsorted.alloc(n_lists));
+  EG_CUDA(t.order.alloc(n_lists));
+  EG_CUDA(t.walk.alloc(n_lists * 2));
   EgSiteBuildParams bp{};
   bp.grid_n = m.grid_n; bp.n_sites = ns; bp.step = m.step;
-  bp.n_settlements = (int)m.sx.size(); bp.sx = c->d_sx; bp.sy = c->d_sy; bp.pop = c->d_pop;
-  bp.n_existing = (int)m.ex.size(); bp.ex = c->d_ex; bp.ey = c->d_ey;
-  bp.n_coast = (int)m.cx.size(); bp.cx = c->d_cx; bp.cy = c->d_cy;
+  bp.n_settlements = (int)m.sx.size(); bp.sx = t.sx.get(); bp.sy = t.sy.get(); bp.pop = t.pop.get();
+  bp.n_existing = (int)m.ex.size(); bp.ex = t.ex.get(); bp.ey = t.ey.get();
+  bp.n_coast = (int)m.cx.size(); bp.cx = t.cx.get(); bp.cy = t.cy.get();
   bp.size_factor = c->htab.small.size_factor;
-  bp.prefix = c->d_prefix; bp.coast_factor = c->d_coast; bp.site_opinion = c->d_site_opinion;
-  bp.static_unsorted = c->d_static_unsorted; bp.order = c->d_order; bp.static_sorted = c->d_static_sorted;
-  bp.prefix_sorted = c->d_prefix_sorted;
-  bp.walk = (double2*)c->d_walk;
+  bp.prefix = t.prefix.get(); bp.coast_factor = t.coast.get(); bp.site_opinion = t.site_opinion.get();
+  bp.static_unsorted = static_unsorted.get(); bp.order = t.order.get();
+  bp.walk = (double2*)t.walk.get();
   int launches = 0;
   EG_CUDA(eg_build_site_tables(bp, s, &launches));
   c->launches += (uint64_t)launches;
   EG_CUDA(cudaStreamSynchronize(s));
-  c->dmap.small = c->d_small;
-  c->dmap.plant_terms = c->d_plant_terms;
-  c->dmap.near_geom = c->htab.near_geom;
-  c->dmap.site_opinion = c->d_site_opinion;
-  c->dmap.coast_factor = c->d_coast;
-  c->dmap.order = c->d_order;
-  c->dmap.static_score = c->d_static_sorted;
-  c->dmap.prefix_score = c->d_prefix_sorted;
-  c->dmap.walk = c->d_walk;
-  c->dmap.near_factor = c->d_near;
-  c->dmap.r2_limit = c->d_r2_limit;
-  c->dmap.r2_stride = c->htab.r2_stride;
-  c->dmap.n_sites = ns;
-  c->dmap.grid_n = m.grid_n;
-  c->dmap.kmax = c->htab.kmax;
+  EgDeviceMap& d = c->dmap;
+  d.small = t.small.get(); d.plant_terms = t.plant_terms.get(); d.near_geom = c->htab.near_geom;
+  d.site_opinion = t.site_opinion.get(); d.coast_factor = t.coast.get(); d.order = t.order.get(); d.walk = t.walk.get();
+  d.near_factor = t.near.get(); d.r2_limit = t.r2_limit.get(); d.r2_stride = c->htab.r2_stride;
+  d.n_sites = ns; d.grid_n = m.grid_n; d.kmax = c->htab.kmax;
+  c->map = std::move(t);
   c->map_ready = true;
   return EG_OK;
 }
 
 int ensure_scratch(eg_ctx* c, size_t n, bool sites, bool yearly, bool traj_in) {
-  if (n > c->cap) {
-    if (c->s_out) cudaFree(c->s_out);
-    if (c->s_traj) cudaFree(c->s_traj);
-    c->s_out = nullptr; c->s_traj = nullptr; c->cap = 0;
-    EG_CUDA(cudaMalloc((void**)&c->s_out, n * sizeof(eg_result)));
-    EG_CUDA(cudaMalloc((void**)&c->s_traj, n * sizeof(eg_traj)));
-    c->cap = n;
-  }
-  if (sites && n > c->cap_sites) {
-    if (c->s_sites) cudaFree(c->s_sites);
-    c->s_sites = nullptr; c->cap_sites = 0;
-    EG_CUDA(cudaMalloc((void**)&c->s_sites, n * sizeof(eg_sites)));
-    c->cap_sites = n;
-  }
-  if (yearly && n > c->cap_yearly) {
-    if (c->s_yearly) cudaFree(c->s_yearly);
-    c->s_yearly = nullptr; c->cap_yearly = 0;
-    EG_CUDA(cudaMalloc((void**)&c->s_yearly, n * sizeof(eg_yearly)));
-    c->cap_yearly = n;
-  }
-  if (traj_in && n > c->cap_traj_in) {
-    if (c->s_traj_in) cudaFree(c->s_traj_in);
-    c->s_traj_in = nullptr; c->cap_traj_in = 0;
-    EG_CUDA(cudaMalloc((void**)&c->s_traj_in, n * sizeof(eg_traj)));
-    c->cap_traj_in = n;
-  }
+  eg_ctx::Scratch& s = c->scratch;
+  if (n > s.out.size()) EG_CUDA(s.out.alloc(n));
+  if (n > s.traj.size()) EG_CUDA(s.traj.alloc(n));
+  if (sites && n > s.sites.size()) EG_CUDA(s.sites.alloc(n));
+  if (yearly && n > s.yearly.size()) EG_CUDA(s.yearly.alloc(n));
+  if (traj_in && n > s.traj_in.size()) EG_CUDA(s.traj_in.alloc(n));
+  return EG_OK;
+}
+
+// copies the first n episodes of the scratch outputs to the host buffers that are not NULL and waits for the copies
+int copy_scratch_out(eg_ctx* c, uint32_t n, eg_result* out, eg_traj* traj_out, eg_sites* sites_out, eg_yearly* yearly_out) {
+  const eg_ctx::Scratch& s = c->scratch;
+  EG_CUDA(cudaMemcpyAsync(out, s.out.get(), (size_t)n * sizeof(eg_result), cudaMemcpyDeviceToHost, c->stream));
+  if (traj_out) EG_CUDA(cudaMemcpyAsync(traj_out, s.traj.get(), (size_t)n * sizeof(eg_traj), cudaMemcpyDeviceToHost, c->stream));
+  if (sites_out) EG_CUDA(cudaMemcpyAsync(sites_out, s.sites.get(), (size_t)n * sizeof(eg_sites), cudaMemcpyDeviceToHost, c->stream));
+  if (yearly_out) EG_CUDA(cudaMemcpyAsync(yearly_out, s.yearly.get(), (size_t)n * sizeof(eg_yearly), cudaMemcpyDeviceToHost, c->stream));
+  EG_CUDA(cudaStreamSynchronize(c->stream));
   return EG_OK;
 }
 
@@ -234,7 +208,7 @@ int check_cfg(const eg_ctx* c, const eg_run_cfg* cfg) {
 EgEpisodeParams make_params(const eg_ctx* c, const eg_run_cfg* cfg, uint64_t seed, uint64_t first, uint32_t n) {
   EgEpisodeParams p{};
   p.map = c->dmap;
-  p.policy = c->d_policy;
+  p.policy = c->policy.d.get();
   p.seed = seed;
   p.first_episode = first;
   p.n = n;
@@ -244,10 +218,58 @@ EgEpisodeParams make_params(const eg_ctx* c, const eg_run_cfg* cfg, uint64_t see
   p.replay_best = cfg->replay_best;
   p.count_weights = c->policy_count_weights ? 1u : 0u;
   p.stagnation = c->policy_stagnation ? 1u : 0u;
-  p.ln100 = std::log(50000000000.0 * 100.0 / 50000000000.0);
-  p.next_episode = c->d_next_episode;
+  p.ln100 = kLn100;
+  p.next_episode = c->next_episode.get();
   p.nf_entries = c->htab.r2_limit[2 * EG_N_RCLASS];
   return p;
+}
+
+EgSuitabilityParams suitability_params(const eg_ctx* c, int use_loaded_map, int mode, int half, int side, double step, uint32_t year_first,
+                                       uint32_t n_years, uint32_t first, uint32_t n, double* d_scores) {
+  EgSuitabilityParams p{};
+  p.mode = mode; p.half = half; p.side = side; p.step = step; p.first = first; p.n = n;
+  p.year_first = (int)year_first; p.n_years = (int)n_years;
+  p.n_settlements = use_loaded_map ? (int)c->hmap.sx.size() : 0;
+  p.sx = c->map.sx.get(); p.sy = c->map.sy.get(); p.pop = c->map.pop.get(); p.urban_r = c->map.urban_r.get(); p.urban_r_max = c->map.urban_r_max;
+  p.n_generators = use_loaded_map ? (int)c->hmap.ex.size() : 0;
+  p.gx = c->map.ex.get(); p.gy = c->map.ey.get();
+  p.n_coast = (int)c->hmap.cx.size(); p.cx = c->map.cx.get(); p.cy = c->map.cy.get();
+  p.scores = d_scores;
+  return p;
+}
+
+// grows the kernel's scratch to what the launch needs, then queues the launch
+int launch_suitability(eg_ctx* c, const EgSuitabilityParams& p) {
+  const size_t rows = eg_suitability_rows_bytes(p.mode == 0 ? 2 * p.half + 1 : p.side) / sizeof(double);
+  if (rows > c->suit_rows.size()) EG_CUDA(c->suit_rows.alloc(rows));
+  EG_CUDA(eg_launch_suitability(p, c->suit_rows.get(), c->stream));
+  if (p.n && p.n_years) c->launches += 2;
+  return EG_OK;
+}
+
+// runs the kernel into a temporary device buffer and copies the scores to the host
+int suitability_to_host(eg_ctx* c, EgSuitabilityParams p, double* scores_out) {
+  EG_CUDA(use_device(c));
+  const size_t count = (size_t)p.n * p.n_years * EG_NT;
+  DeviceArray<double> d_scores;
+  EG_CUDA(d_scores.alloc(std::max<size_t>(count, 1)));
+  p.scores = d_scores.get();
+  const int rc = launch_suitability(c, p);
+  if (rc) return rc;
+  EG_CUDA(cudaMemcpyAsync(scores_out, d_scores.get(), count * sizeof(double), cudaMemcpyDeviceToHost, c->stream));
+  EG_CUDA(cudaStreamSynchronize(c->stream));
+  return EG_OK;
+}
+
+// argument checks of eg_location_analysis_sites and eg_location_analysis_sites_device (`name`)
+int check_sites_args(const eg_ctx* c, const double* scores, const char* name, uint32_t sites_per_axis, uint32_t year_first,
+                     uint32_t n_years, uint32_t first_site, uint32_t n_sites) {
+  if (!c || !scores) return eg_fail(EG_ERR_INVALID, std::string(name) + ": NULL argument");
+  if (!c->map_ready) return eg_fail(EG_ERR_STATE, "no map loaded (the coastline polygon is needed)");
+  if (year_first >= EG_NY || n_years > EG_NY - year_first) return eg_fail(EG_ERR_INVALID, "year range outside 2025..2050");
+  if (sites_per_axis == 0 || sites_per_axis > 65535u) return eg_fail(EG_ERR_INVALID, "sites_per_axis out of range");
+  if ((uint64_t)first_site + n_sites > (uint64_t)sites_per_axis * sites_per_axis) return eg_fail(EG_ERR_INVALID, "site range exceeds the grid");
+  return EG_OK;
 }
 
 }  // namespace
@@ -264,43 +286,24 @@ int eg_init(int device, void* cuda_stream, eg_ctx** out) {
     return eg_fail(EG_ERR_NO_DEVICE, std::string("no CUDA device (") + cudaGetErrorString(err) + "); eirgrid_b200 has no CPU fallback");
   if (device < 0 || device >= count) return eg_fail(EG_ERR_INVALID, "eg_init: device index out of range");
   EG_CUDA(cudaSetDevice(device));
-  eg_ctx* c = new eg_ctx();
+  std::unique_ptr<eg_ctx> c(new eg_ctx());
   c->device = device;
-  if (cuda_stream) {
-    c->stream = (cudaStream_t)cuda_stream;
-  } else {
-    cudaError_t e2 = cudaStreamCreateWithFlags(&c->stream, cudaStreamNonBlocking);
-    if (e2 != cudaSuccess) { delete c; return eg_fail(EG_ERR_CUDA, cudaGetErrorString(e2)); }
-    c->own_stream = true;
+  c->stream = (cudaStream_t)cuda_stream;
+  if (!cuda_stream) {
+    err = cudaStreamCreateWithFlags(&c->stream, cudaStreamNonBlocking);
+    if (err != cudaSuccess) return eg_fail(EG_ERR_CUDA, cudaGetErrorString(err));
+    c->own_stream.reset(c->stream);
   }
-  cudaError_t e3 = cudaMalloc((void**)&c->d_next_episode, sizeof(uint32_t));
-  if (e3 != cudaSuccess) { if (c->own_stream) cudaStreamDestroy(c->stream); delete c; return eg_fail(EG_ERR_CUDA, cudaGetErrorString(e3)); }
-  *out = c;
+  err = c->next_episode.alloc(1);
+  if (err != cudaSuccess) return eg_fail(EG_ERR_CUDA, cudaGetErrorString(err));
+  *out = c.release();
   return EG_OK;
 }
 
 void eg_destroy(eg_ctx* c) {
   if (!c) return;
-  cudaSetDevice(c->device);
+  use_device(c);
   cudaStreamSynchronize(c->stream);
-  free_map(c);
-  if (c->h_stats) cudaFreeHost(c->h_stats);
-  if (c->h_record) cudaFreeHost(c->h_record);
-  for (int b = 0; b < 2; b++) {
-    if (c->h_policy[b]) cudaFreeHost(c->h_policy[b]);
-    if (c->policy_copied[b]) cudaEventDestroy(c->policy_copied[b]);
-  }
-  if (c->h_upd_state) cudaFreeHost(c->h_upd_state);
-  if (c->h_upd_slot) cudaFreeHost(c->h_upd_slot);
-  if (c->h_upd_imp) cudaFreeHost(c->h_upd_imp);
-  if (c->d_suit_rows) cudaFree(c->d_suit_rows);
-  void* upd_ptrs[] = {c->upd.state, c->upd.slots, c->upd.score, c->upd.pre, c->upd.ctl, c->upd.counts, c->upd.factors, c->upd.improvements};
-  for (void* p : upd_ptrs)
-    if (p) cudaFree(p);
-  void* ptrs[] = {c->d_policy, c->d_next_episode, c->d_stats, c->d_best_score, c->d_best_index, c->d_record, c->s_out, c->s_traj, c->s_traj_in, c->s_sites, c->s_yearly};
-  for (void* p : ptrs)
-    if (p) cudaFree(p);
-  if (c->own_stream) cudaStreamDestroy(c->stream);
   delete c;
 }
 
@@ -342,15 +345,17 @@ int eg_map_site_tables(eg_ctx* c, uint32_t year_index, uint32_t rclass, uint32_t
   if (!c->map_ready) return eg_fail(EG_ERR_STATE, "no map loaded");
   if (year_index >= EG_NY || rclass >= EG_N_RCLASS || pclass >= EG_N_PCLASS) return eg_fail(EG_ERR_INVALID, "index out of range");
   const size_t ns = (size_t)c->dmap.n_sites;
-  EG_CUDA(cudaSetDevice(c->device));
+  const size_t list = ((size_t)pclass * EG_NY + year_index) * ns;
+  EG_CUDA(use_device(c));
   if (prefix_score)
-    EG_CUDA(cudaMemcpyAsync(prefix_score, c->d_prefix + ((size_t)rclass * EG_NY + year_index) * ns, ns * sizeof(double), cudaMemcpyDeviceToHost, c->stream));
-  if (static_score_sorted)
-    EG_CUDA(cudaMemcpyAsync(static_score_sorted, c->d_static_sorted + ((size_t)pclass * EG_NY + year_index) * ns, ns * sizeof(double), cudaMemcpyDeviceToHost, c->stream));
+    EG_CUDA(cudaMemcpyAsync(prefix_score, c->map.prefix.get() + ((size_t)rclass * EG_NY + year_index) * ns, ns * sizeof(double), cudaMemcpyDeviceToHost, c->stream));
+  if (static_score_sorted)  // the static score is the first half of each walk entry
+    EG_CUDA(cudaMemcpy2DAsync(static_score_sorted, sizeof(double), c->map.walk.get() + 2 * list, 2 * sizeof(double), sizeof(double), ns,
+                              cudaMemcpyDeviceToHost, c->stream));
   std::vector<uint16_t> tmp;
   if (order_sorted) {
     tmp.resize(ns);
-    EG_CUDA(cudaMemcpyAsync(tmp.data(), c->d_order + ((size_t)pclass * EG_NY + year_index) * ns, ns * sizeof(uint16_t), cudaMemcpyDeviceToHost, c->stream));
+    EG_CUDA(cudaMemcpyAsync(tmp.data(), c->map.order.get() + list, ns * sizeof(uint16_t), cudaMemcpyDeviceToHost, c->stream));
   }
   EG_CUDA(cudaStreamSynchronize(c->stream));
   if (order_sorted)
@@ -362,33 +367,37 @@ int eg_map_site_static(eg_ctx* c, double* coast_factor, double* site_opinion) {
   if (!c) return eg_fail(EG_ERR_INVALID, "ctx is NULL");
   if (!c->map_ready) return eg_fail(EG_ERR_STATE, "no map loaded");
   const size_t ns = (size_t)c->dmap.n_sites;
-  EG_CUDA(cudaSetDevice(c->device));
-  if (coast_factor) EG_CUDA(cudaMemcpyAsync(coast_factor, c->d_coast, ns * sizeof(double), cudaMemcpyDeviceToHost, c->stream));
-  if (site_opinion) EG_CUDA(cudaMemcpyAsync(site_opinion, c->d_site_opinion, ns * sizeof(double), cudaMemcpyDeviceToHost, c->stream));
+  EG_CUDA(use_device(c));
+  if (coast_factor) EG_CUDA(cudaMemcpyAsync(coast_factor, c->map.coast.get(), ns * sizeof(double), cudaMemcpyDeviceToHost, c->stream));
+  if (site_opinion) EG_CUDA(cudaMemcpyAsync(site_opinion, c->map.site_opinion.get(), ns * sizeof(double), cudaMemcpyDeviceToHost, c->stream));
   EG_CUDA(cudaStreamSynchronize(c->stream));
   return EG_OK;
 }
 
 int eg_weights_upload(eg_ctx* c, const eg_weights* w) {
   if (!c || !w) return eg_fail(EG_ERR_INVALID, "eg_weights_upload: NULL argument");
-  EG_CUDA(cudaSetDevice(c->device));
-  if (!c->d_policy) {
-    EG_CUDA(cudaMalloc((void**)&c->d_policy, sizeof(EgPolicyDevice)));
+  EG_CUDA(use_device(c));
+  if (!c->policy.d.get()) {
+    eg_ctx::PolicyBuffers p;
+    EG_CUDA(p.d.alloc(1));
     for (int b = 0; b < 2; b++) {
-      EG_CUDA(cudaMallocHost((void**)&c->h_policy[b], sizeof(EgPolicyDevice)));
-      EG_CUDA(cudaEventCreateWithFlags(&c->policy_copied[b], cudaEventDisableTiming));
+      EG_CUDA(p.h[b].alloc(1));
+      cudaEvent_t e = nullptr;
+      EG_CUDA(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
+      p.copied[b].reset(e);
     }
+    c->policy = std::move(p);
   }
   // two pinned staging buffers used in turn: the copy is queued on the stream and the call returns without waiting for it;
   // a buffer is refilled only after the copy issued from it two uploads ago has completed (normally long ago)
   const int b = c->policy_turn;
   c->policy_turn ^= 1;
-  EG_CUDA(cudaEventSynchronize(c->policy_copied[b]));
-  EgPolicyDevice& pol = *c->h_policy[b];
+  EG_CUDA(cudaEventSynchronize(c->policy.copied[b].get()));
+  EgPolicyDevice& pol = *c->policy.h[b].get();
   if (!eg_weights_fill_policy(*w, &pol))
     return eg_fail(EG_ERR_OVERFLOW, "eg_weights_upload: the best-strategy lists exceed the device snapshot's capacity (EG_BEST_CAPACITY / EG_TRAJ_CAPACITY actions)");
-  EG_CUDA(cudaMemcpyAsync(c->d_policy, &pol, sizeof(pol), cudaMemcpyHostToDevice, c->stream));
-  EG_CUDA(cudaEventRecord(c->policy_copied[b], c->stream));
+  EG_CUDA(cudaMemcpyAsync(c->policy.d.get(), &pol, sizeof(pol), cudaMemcpyHostToDevice, c->stream));
+  EG_CUDA(cudaEventRecord(c->policy.copied[b].get(), c->stream));
   c->policy_ready = true;
   c->policy_count_weights = pol.has_count_weights != 0;
   c->policy_stagnation = pol.iwi > 500;
@@ -401,7 +410,7 @@ int eg_rollout_batch_device(eg_ctx* c, const eg_run_cfg* cfg, uint64_t seed, uin
   if (rc) return rc;
   if (!c->policy_ready) return eg_fail(EG_ERR_STATE, "no weights uploaded: call eg_weights_upload first");
   if (!d_out) return eg_fail(EG_ERR_INVALID, "eg_rollout_batch_device: d_out is NULL");
-  EG_CUDA(cudaSetDevice(c->device));
+  EG_CUDA(use_device(c));
   EgEpisodeParams p = make_params(c, cfg, seed, first_episode, n);
   p.out = d_out; p.traj = d_traj; p.sites = d_sites; p.yearly = d_yearly;
   EG_CUDA(eg_launch_rollout(p, c->stream));
@@ -414,17 +423,14 @@ int eg_rollout_batch(eg_ctx* c, const eg_weights* w, const eg_run_cfg* cfg, uint
   int rc = check_cfg(c, cfg);
   if (rc) return rc;
   if (!w || !out) return eg_fail(EG_ERR_INVALID, "eg_rollout_batch: NULL argument");
+  EG_CUDA(use_device(c));
   if ((rc = eg_weights_upload(c, w))) return rc;
   if ((rc = ensure_scratch(c, n, sites_out != nullptr, yearly_out != nullptr, false))) return rc;
-  rc = eg_rollout_batch_device(c, cfg, seed, first_episode, n, c->s_out, traj_out ? c->s_traj : nullptr,
-                               sites_out ? c->s_sites : nullptr, yearly_out ? c->s_yearly : nullptr);
+  const eg_ctx::Scratch& s = c->scratch;
+  rc = eg_rollout_batch_device(c, cfg, seed, first_episode, n, s.out.get(), traj_out ? s.traj.get() : nullptr,
+                               sites_out ? s.sites.get() : nullptr, yearly_out ? s.yearly.get() : nullptr);
   if (rc) return rc;
-  EG_CUDA(cudaMemcpyAsync(out, c->s_out, (size_t)n * sizeof(eg_result), cudaMemcpyDeviceToHost, c->stream));
-  if (traj_out) EG_CUDA(cudaMemcpyAsync(traj_out, c->s_traj, (size_t)n * sizeof(eg_traj), cudaMemcpyDeviceToHost, c->stream));
-  if (sites_out) EG_CUDA(cudaMemcpyAsync(sites_out, c->s_sites, (size_t)n * sizeof(eg_sites), cudaMemcpyDeviceToHost, c->stream));
-  if (yearly_out) EG_CUDA(cudaMemcpyAsync(yearly_out, c->s_yearly, (size_t)n * sizeof(eg_yearly), cudaMemcpyDeviceToHost, c->stream));
-  EG_CUDA(cudaStreamSynchronize(c->stream));
-  return EG_OK;
+  return copy_scratch_out(c, n, out, traj_out, sites_out, yearly_out);
 }
 
 int eg_replay_batch_device(eg_ctx* c, const eg_run_cfg* cfg, const eg_traj* d_in, uint32_t n, eg_result* d_out,
@@ -432,7 +438,7 @@ int eg_replay_batch_device(eg_ctx* c, const eg_run_cfg* cfg, const eg_traj* d_in
   int rc = check_cfg(c, cfg);
   if (rc) return rc;
   if (!d_in || !d_out) return eg_fail(EG_ERR_INVALID, "eg_replay_batch_device: NULL argument");
-  EG_CUDA(cudaSetDevice(c->device));
+  EG_CUDA(use_device(c));
   EgEpisodeParams p = make_params(c, cfg, 0, 0, n);
   p.policy = nullptr;
   p.replay_in = d_in;
@@ -447,15 +453,13 @@ int eg_replay_batch(eg_ctx* c, const eg_run_cfg* cfg, const eg_traj* in, uint32_
   int rc = check_cfg(c, cfg);
   if (rc) return rc;
   if (!in || !out) return eg_fail(EG_ERR_INVALID, "eg_replay_batch: NULL argument");
+  EG_CUDA(use_device(c));
   if ((rc = ensure_scratch(c, n, sites_out != nullptr, yearly_out != nullptr, true))) return rc;
-  EG_CUDA(cudaMemcpyAsync(c->s_traj_in, in, (size_t)n * sizeof(eg_traj), cudaMemcpyHostToDevice, c->stream));
-  rc = eg_replay_batch_device(c, cfg, c->s_traj_in, n, c->s_out, sites_out ? c->s_sites : nullptr, yearly_out ? c->s_yearly : nullptr);
+  const eg_ctx::Scratch& s = c->scratch;
+  EG_CUDA(cudaMemcpyAsync(s.traj_in.get(), in, (size_t)n * sizeof(eg_traj), cudaMemcpyHostToDevice, c->stream));
+  rc = eg_replay_batch_device(c, cfg, s.traj_in.get(), n, s.out.get(), sites_out ? s.sites.get() : nullptr, yearly_out ? s.yearly.get() : nullptr);
   if (rc) return rc;
-  EG_CUDA(cudaMemcpyAsync(out, c->s_out, (size_t)n * sizeof(eg_result), cudaMemcpyDeviceToHost, c->stream));
-  if (sites_out) EG_CUDA(cudaMemcpyAsync(sites_out, c->s_sites, (size_t)n * sizeof(eg_sites), cudaMemcpyDeviceToHost, c->stream));
-  if (yearly_out) EG_CUDA(cudaMemcpyAsync(yearly_out, c->s_yearly, (size_t)n * sizeof(eg_yearly), cudaMemcpyDeviceToHost, c->stream));
-  EG_CUDA(cudaStreamSynchronize(c->stream));
-  return EG_OK;
+  return copy_scratch_out(c, n, out, nullptr, sites_out, yearly_out);
 }
 
 int eg_update_stats_device(eg_ctx* c, const eg_weights* w, const eg_result* d_results, const eg_traj* d_trajs, uint32_t n,
@@ -463,13 +467,13 @@ int eg_update_stats_device(eg_ctx* c, const eg_weights* w, const eg_result* d_re
   if (!c || !w || !d_results || !d_trajs || !d_stats || !d_best_score || !d_best_index)
     return eg_fail(EG_ERR_INVALID, "eg_update_stats_device: NULL argument");
   if (!c->policy_ready) return eg_fail(EG_ERR_STATE, "no weights uploaded: call eg_weights_upload first");
-  EG_CUDA(cudaSetDevice(c->device));
+  EG_CUDA(use_device(c));
   EgStatsParams p{};
   p.consts = eg_contrast_consts(*w);
-  p.policy = c->d_policy;
+  p.policy = c->policy.d.get();
   p.results = d_results; p.trajs = d_trajs; p.n = n;
   p.stats = d_stats; p.best_score = d_best_score; p.best_index = d_best_index;
-  p.ln100 = std::log(50000000000.0 * 100.0 / 50000000000.0);
+  p.ln100 = kLn100;
   EG_CUDA(eg_launch_stats(p, c->stream));
   c->launches += n ? 3 : 1;  // reset + accumulate + arg-best kernels
   return EG_OK;
@@ -477,7 +481,7 @@ int eg_update_stats_device(eg_ctx* c, const eg_weights* w, const eg_result* d_re
 
 int eg_update_stats_clear_device(eg_ctx* c, int64_t* d_stats) {
   if (!c || !d_stats) return eg_fail(EG_ERR_INVALID, "eg_update_stats_clear_device: NULL argument");
-  EG_CUDA(cudaSetDevice(c->device));
+  EG_CUDA(use_device(c));
   EG_CUDA(cudaMemsetAsync(d_stats, 0, (size_t)EG_STATS_WORDS * sizeof(int64_t), c->stream));
   return EG_OK;
 }
@@ -486,7 +490,7 @@ int eg_update_pack_best_device(eg_ctx* c, const eg_result* d_results, const eg_t
                                const unsigned long long* d_best_index, uint64_t first_global_episode, void* d_record) {
   if (!c || !d_results || !d_trajs || !d_best_score || !d_best_index || !d_record)
     return eg_fail(EG_ERR_INVALID, "eg_update_pack_best_device: NULL argument");
-  EG_CUDA(cudaSetDevice(c->device));
+  EG_CUDA(use_device(c));
   EG_CUDA(eg_launch_pack_best(d_results, d_trajs, n, d_best_score, d_best_index, first_global_episode, d_record, c->stream));
   c->launches++;
   return EG_OK;
@@ -499,7 +503,7 @@ int eg_update_pack_exchange_device(eg_ctx* c, const eg_result* d_results, const 
   if (!c || !d_results || !d_trajs || !d_stats || !d_best_score || !d_best_index || !peer_buffers || !peer_flags || !d_error)
     return eg_fail(EG_ERR_INVALID, "eg_update_pack_exchange_device: NULL argument");
   if (world == 0 || world > EG_MAX_PEERS || rank >= world) return eg_fail(EG_ERR_INVALID, "eg_update_pack_exchange_device: bad world / rank");
-  EG_CUDA(cudaSetDevice(c->device));
+  EG_CUDA(use_device(c));
   EgExchangeParams p{};
   p.results = d_results; p.trajs = d_trajs; p.n = n; p.best_score = d_best_score; p.best_index = d_best_index;
   p.first_global = first_global_episode; p.stats = d_stats; p.world = world; p.rank = rank; p.epoch = epoch; p.error = d_error;
@@ -514,23 +518,27 @@ int eg_train_batch_begin(eg_ctx* c, const eg_weights* w, const eg_run_cfg* cfg, 
   if (rc) return rc;
   if (!w) return eg_fail(EG_ERR_INVALID, "eg_train_batch_begin: weights are NULL");
   if (c->train_pending) return eg_fail(EG_ERR_STATE, "eg_train_batch_begin: a batch is already in flight on this context");
-  EG_CUDA(cudaSetDevice(c->device));
-  if (!c->d_stats) {
-    EG_CUDA(cudaMalloc((void**)&c->d_stats, EG_STATS_WORDS * sizeof(int64_t)));
-    EG_CUDA(cudaMalloc((void**)&c->d_best_score, sizeof(double)));
-    EG_CUDA(cudaMalloc((void**)&c->d_best_index, sizeof(unsigned long long)));
-    EG_CUDA(cudaMalloc((void**)&c->d_record, EG_BEST_RECORD_BYTES));
-    EG_CUDA(cudaMallocHost((void**)&c->h_stats, EG_STATS_WORDS * sizeof(int64_t)));
-    EG_CUDA(cudaMallocHost((void**)&c->h_record, EG_BEST_RECORD_BYTES));
+  EG_CUDA(use_device(c));
+  if (!c->train.stats.get()) {
+    eg_ctx::TrainBuffers t;
+    EG_CUDA(t.stats.alloc(EG_STATS_WORDS));
+    EG_CUDA(t.best_score.alloc(1));
+    EG_CUDA(t.best_index.alloc(1));
+    EG_CUDA(t.record.alloc(EG_BEST_RECORD_BYTES));
+    EG_CUDA(t.h_stats.alloc(EG_STATS_WORDS));
+    EG_CUDA(t.h_record.alloc(EG_BEST_RECORD_BYTES));
+    c->train = std::move(t);
   }
   if ((rc = eg_weights_upload(c, w))) return rc;
   if ((rc = ensure_scratch(c, n, false, false, false))) return rc;
-  if ((rc = eg_rollout_batch_device(c, cfg, seed, first_episode, n, c->s_out, c->s_traj, nullptr, nullptr))) return rc;
-  if ((rc = eg_update_stats_clear_device(c, c->d_stats))) return rc;
-  if ((rc = eg_update_stats_device(c, w, c->s_out, c->s_traj, n, c->d_stats, c->d_best_score, c->d_best_index))) return rc;
-  if ((rc = eg_update_pack_best_device(c, c->s_out, c->s_traj, n, c->d_best_score, c->d_best_index, first_episode, c->d_record))) return rc;
-  EG_CUDA(cudaMemcpyAsync(c->h_stats, c->d_stats, EG_STATS_WORDS * sizeof(int64_t), cudaMemcpyDeviceToHost, c->stream));
-  EG_CUDA(cudaMemcpyAsync(c->h_record, c->d_record, EG_BEST_RECORD_BYTES, cudaMemcpyDeviceToHost, c->stream));
+  const eg_ctx::Scratch& s = c->scratch;
+  const eg_ctx::TrainBuffers& t = c->train;
+  if ((rc = eg_rollout_batch_device(c, cfg, seed, first_episode, n, s.out.get(), s.traj.get(), nullptr, nullptr))) return rc;
+  if ((rc = eg_update_stats_clear_device(c, t.stats.get()))) return rc;
+  if ((rc = eg_update_stats_device(c, w, s.out.get(), s.traj.get(), n, t.stats.get(), t.best_score.get(), t.best_index.get()))) return rc;
+  if ((rc = eg_update_pack_best_device(c, s.out.get(), s.traj.get(), n, t.best_score.get(), t.best_index.get(), first_episode, t.record.get()))) return rc;
+  EG_CUDA(cudaMemcpyAsync(t.h_stats.get(), t.stats.get(), EG_STATS_WORDS * sizeof(int64_t), cudaMemcpyDeviceToHost, c->stream));
+  EG_CUDA(cudaMemcpyAsync(t.h_record.get(), t.record.get(), EG_BEST_RECORD_BYTES, cudaMemcpyDeviceToHost, c->stream));
   c->train_n = n;
   c->train_pending = true;
   return EG_OK;
@@ -539,84 +547,70 @@ int eg_train_batch_begin(eg_ctx* c, const eg_weights* w, const eg_run_cfg* cfg, 
 int eg_train_batch_end(eg_ctx* c, int64_t* stats_out, void* record_out) {
   if (!c || !stats_out || !record_out) return eg_fail(EG_ERR_INVALID, "eg_train_batch_end: NULL argument");
   if (!c->train_pending) return eg_fail(EG_ERR_STATE, "eg_train_batch_end: no batch in flight");
-  EG_CUDA(cudaSetDevice(c->device));
+  EG_CUDA(use_device(c));
   c->train_pending = false;
   EG_CUDA(cudaStreamSynchronize(c->stream));
-  std::memcpy(stats_out, c->h_stats, EG_STATS_WORDS * sizeof(int64_t));
-  std::memcpy(record_out, c->h_record, EG_BEST_RECORD_BYTES);
+  std::memcpy(stats_out, c->train.h_stats.get(), EG_STATS_WORDS * sizeof(int64_t));
+  std::memcpy(record_out, c->train.h_record.get(), EG_BEST_RECORD_BYTES);
   return EG_OK;
 }
 
 int eg_train_batch_results(eg_ctx* c, eg_result* out, eg_traj* traj_out) {
   if (!c || !out) return eg_fail(EG_ERR_INVALID, "eg_train_batch_results: NULL argument");
   if (c->train_pending || !c->train_n) return eg_fail(EG_ERR_STATE, "eg_train_batch_results: no finished batch");
-  EG_CUDA(cudaSetDevice(c->device));
-  EG_CUDA(cudaMemcpyAsync(out, c->s_out, (size_t)c->train_n * sizeof(eg_result), cudaMemcpyDeviceToHost, c->stream));
-  if (traj_out) EG_CUDA(cudaMemcpyAsync(traj_out, c->s_traj, (size_t)c->train_n * sizeof(eg_traj), cudaMemcpyDeviceToHost, c->stream));
-  EG_CUDA(cudaStreamSynchronize(c->stream));
-  return EG_OK;
+  EG_CUDA(use_device(c));
+  return copy_scratch_out(c, c->train_n, out, traj_out, nullptr, nullptr);
 }
 
 // ---- in-order update on the device (update.cu) ----------------------------------------------------------------------
-namespace {
-
-int ensure_update_buffers(eg_ctx* c, uint32_t n) {
-  EgUpdBuffers& u = c->upd;
-  if (!u.state) {
-    EG_CUDA(cudaMalloc((void**)&u.state, sizeof(EgUpdState)));
-    EG_CUDA(cudaMalloc((void**)&u.slots, (size_t)(EG_UPD_CHUNK + 1) * sizeof(EgUpdSlot)));
-    EG_CUDA(cudaMalloc((void**)&u.score, (size_t)EG_UPD_CHUNK * sizeof(double)));
-    EG_CUDA(cudaMalloc((void**)&u.pre, (size_t)EG_UPD_CHUNK * sizeof(EgUpdPre)));
-    EG_CUDA(cudaMalloc((void**)&u.ctl, (size_t)EG_UPD_CHUNK * sizeof(EgUpdCtl)));
-    EG_CUDA(cudaMalloc((void**)&u.counts, (size_t)EG_NY * EG_UPD_CHUNK * EG_UPD_ROW));
-    EG_CUDA(cudaMalloc((void**)&u.factors, (size_t)EG_NY * EG_UPD_CHUNK * EG_UPD_ENTRIES * sizeof(double)));
-    EG_CUDA(cudaMallocHost((void**)&c->h_upd_state, sizeof(EgUpdState)));
-    EG_CUDA(cudaMallocHost((void**)&c->h_upd_slot, sizeof(EgUpdSlot)));
-    EG_CUDA(cudaMallocHost((void**)&c->h_upd_imp, (size_t)EG_UPD_IMP_INLINE * sizeof(EgUpdImprovement)));
-  }
-  if (n > u.improvements_capacity) {
-    if (u.improvements) cudaFree(u.improvements);
-    u.improvements = nullptr; u.improvements_capacity = 0;
-    const uint32_t cap = std::max<uint32_t>(n, EG_UPD_IMP_INLINE);
-    EG_CUDA(cudaMalloc((void**)&u.improvements, (size_t)cap * sizeof(EgUpdImprovement)));
-    u.improvements_capacity = cap;
-  }
-  return EG_OK;
-}
-
-}  // namespace
-
 int eg_update_device(eg_ctx* c, eg_weights* w, const eg_result* d_results, const eg_traj* d_trajs, uint32_t n, uint32_t replay_best,
                      uint64_t rng_seed, eg_update_stats* stats_out) {
   if (!c || !w || (n && (!d_results || !d_trajs))) return eg_fail(EG_ERR_INVALID, "eg_update_device: NULL argument");
-  EG_CUDA(cudaSetDevice(c->device));
-  int rc = ensure_update_buffers(c, n);
-  if (rc) return rc;
+  EG_CUDA(use_device(c));
+  if (!c->upd.state.get()) {
+    eg_ctx::UpdateBuffers u;
+    EG_CUDA(u.state.alloc(1));
+    EG_CUDA(u.slots.alloc((size_t)EG_UPD_CHUNK + 1));
+    EG_CUDA(u.score.alloc(EG_UPD_CHUNK));
+    EG_CUDA(u.pre.alloc(EG_UPD_CHUNK));
+    EG_CUDA(u.ctl.alloc(EG_UPD_CHUNK));
+    EG_CUDA(u.counts.alloc((size_t)EG_NY * EG_UPD_CHUNK * EG_UPD_ROW));
+    EG_CUDA(u.factors.alloc((size_t)EG_NY * EG_UPD_CHUNK * EG_UPD_ENTRIES));
+    EG_CUDA(u.h_state.alloc(1));
+    EG_CUDA(u.h_slot.alloc(1));
+    EG_CUDA(u.h_imp.alloc(EG_UPD_IMP_INLINE));
+    c->upd = std::move(u);
+  }
+  if (n > c->upd_improvements.size()) EG_CUDA(c->upd_improvements.alloc(std::max<uint32_t>(n, EG_UPD_IMP_INLINE)));
+  const eg_ctx::UpdateBuffers& u = c->upd;
+  const EgUpdBuffers view{u.state.get(), u.slots.get(), u.score.get(), u.pre.get(), u.ctl.get(), u.counts.get(), u.factors.get(),
+                          c->upd_improvements.get(), (uint32_t)c->upd_improvements.size()};
   // the pinned mirrors are free again: every call ends with a stream synchronisation
-  if (!eg_weights_fill_update_state(*w, c->h_upd_state, c->h_upd_slot))
+  if (!eg_weights_fill_update_state(*w, u.h_state.get(), u.h_slot.get()))
     return eg_fail(EG_ERR_OVERFLOW, "eg_update_device: the best-strategy lists exceed EG_UPD_CAT_CAPACITY entries");
   const uint32_t iteration0 = w->iteration_count;
-  EG_CUDA(cudaMemcpyAsync(c->upd.state, c->h_upd_state, sizeof(EgUpdState), cudaMemcpyHostToDevice, c->stream));
-  EG_CUDA(cudaMemcpyAsync(c->upd.slots, c->h_upd_slot, sizeof(EgUpdSlot), cudaMemcpyHostToDevice, c->stream));
+  EG_CUDA(cudaMemcpyAsync(view.state, u.h_state.get(), sizeof(EgUpdState), cudaMemcpyHostToDevice, c->stream));
+  EG_CUDA(cudaMemcpyAsync(view.slots, u.h_slot.get(), sizeof(EgUpdSlot), cudaMemcpyHostToDevice, c->stream));
   for (uint32_t base = 0; base < n; base += EG_UPD_CHUNK) {
     const uint32_t cnt = std::min<uint32_t>(EG_UPD_CHUNK, n - base);
     int launches = 0;
-    EG_CUDA(eg_launch_update_pass(c->upd, d_results + base, d_trajs + base, cnt, base, replay_best, rng_seed, c->stream, &launches));
+    EG_CUDA(eg_launch_update_pass(view, d_results + base, d_trajs + base, cnt, base, replay_best, rng_seed, c->stream, &launches));
     c->launches += (uint64_t)launches;
   }
-  EG_CUDA(cudaMemcpyAsync(c->h_upd_state, c->upd.state, sizeof(EgUpdState), cudaMemcpyDeviceToHost, c->stream));
-  EG_CUDA(cudaMemcpyAsync(c->h_upd_slot, c->upd.slots, sizeof(EgUpdSlot), cudaMemcpyDeviceToHost, c->stream));
-  EG_CUDA(cudaMemcpyAsync(c->h_upd_imp, c->upd.improvements, (size_t)EG_UPD_IMP_INLINE * sizeof(EgUpdImprovement), cudaMemcpyDeviceToHost, c->stream));
+  EG_CUDA(cudaMemcpyAsync(u.h_state.get(), view.state, sizeof(EgUpdState), cudaMemcpyDeviceToHost, c->stream));
+  EG_CUDA(cudaMemcpyAsync(u.h_slot.get(), view.slots, sizeof(EgUpdSlot), cudaMemcpyDeviceToHost, c->stream));
+  EG_CUDA(cudaMemcpyAsync(u.h_imp.get(), view.improvements, (size_t)EG_UPD_IMP_INLINE * sizeof(EgUpdImprovement), cudaMemcpyDeviceToHost, c->stream));
   EG_CUDA(cudaStreamSynchronize(c->stream));
-  const EgUpdState& st = *c->h_upd_state;
+  const EgUpdState& st = *u.h_state.get();
   std::vector<EgUpdImprovement> more;
-  const EgUpdImprovement* imps = c->h_upd_imp;
+  const EgUpdImprovement* imps = u.h_imp.get();
   if (st.n_improvements > EG_UPD_IMP_INLINE) {  // rare: more improving episodes than the inline window
     more.resize(st.n_improvements);
-    EG_CUDA(cudaMemcpy(more.data(), c->upd.improvements, (size_t)st.n_improvements * sizeof(EgUpdImprovement), cudaMemcpyDeviceToHost));
+    EG_CUDA(cudaMemcpyAsync(more.data(), view.improvements, (size_t)st.n_improvements * sizeof(EgUpdImprovement), cudaMemcpyDeviceToHost, c->stream));
+    EG_CUDA(cudaStreamSynchronize(c->stream));
     imps = more.data();
   }
-  eg_weights_apply_update_state(*w, st, *c->h_upd_slot, imps, st.n_improvements, iteration0);
+  eg_weights_apply_update_state(*w, st, *u.h_slot.get(), imps, st.n_improvements, iteration0);
   if (stats_out) {
     eg_update_stats so;
     std::memset(&so, 0, sizeof(so));
@@ -639,69 +633,16 @@ int eg_train_batch_inorder(eg_ctx* c, eg_weights* w, const eg_run_cfg* cfg, uint
   if (rc) return rc;
   if (!w) return eg_fail(EG_ERR_INVALID, "eg_train_batch_inorder: weights are NULL");
   if (c->train_pending) return eg_fail(EG_ERR_STATE, "eg_train_batch_inorder: a batch is already in flight on this context");
+  EG_CUDA(use_device(c));
   if ((rc = eg_weights_upload(c, w))) return rc;
   if ((rc = ensure_scratch(c, n, false, false, false))) return rc;
-  if ((rc = eg_rollout_batch_device(c, cfg, seed, first_episode, n, c->s_out, c->s_traj, nullptr, nullptr))) return rc;
+  const eg_ctx::Scratch& s = c->scratch;
+  if ((rc = eg_rollout_batch_device(c, cfg, seed, first_episode, n, s.out.get(), s.traj.get(), nullptr, nullptr))) return rc;
   c->train_n = n;
-  return eg_update_device(c, w, c->s_out, c->s_traj, n, cfg->replay_best, rng_seed, stats_out);
+  return eg_update_device(c, w, s.out.get(), s.traj.get(), n, cfg->replay_best, rng_seed, stats_out);
 }
 
-// ---- CSV export of the best run (utils/csv_export.rs) ------------------------------------------------------------
-namespace {
-
-const char* const kCsvGenNames[EG_NT] = {"OnshoreWind", "OffshoreWind", "DomesticSolar", "CommercialSolar", "UtilitySolar", "Nuclear", "CoalPlant",
-                                         "GasCombinedCycle", "GasPeaker", "Biomass", "HydroDam", "PumpedStorage", "BatteryStorage",
-                                         "TidalGenerator", "WaveEnergy"};
-const char* const kCsvOffsetNames[EG_N_OFFSET_TYPES] = {"Forest", "Wetland", "ActiveCapture", "CarbonCredit"};
-
-// Rust's `{}` for f64: shortest digits that round-trip, never scientific notation
-std::string rust_display(double v) {
-  char buf[400];
-  for (int prec = 1; prec <= 17; prec++) {
-    std::snprintf(buf, sizeof(buf), "%.*g", prec, v);
-    if (std::strtod(buf, nullptr) == v) break;
-  }
-  if (!std::strpbrk(buf, "eE")) return buf;
-  // re-print without exponent: enough fixed digits to round-trip
-  for (int prec = 0; prec <= 340; prec++) {
-    std::snprintf(buf, sizeof(buf), "%.*f", prec, v);
-    if (std::strtod(buf, nullptr) == v) break;
-  }
-  return buf;
-}
-
-std::string fixed(double v, int prec) {
-  char buf[400];
-  std::snprintf(buf, sizeof(buf), "%.*f", prec, v);
-  return buf;
-}
-
-// uniform in [0,1) for the exported offset coordinates: Philox4x32-10, counter (index, axis, 0, "CSVO")
-double csv_uniform(uint32_t index, uint32_t axis) {
-  uint32_t a0 = index, a1 = axis, a2 = 0u, a3 = 0x4353564Fu, x0 = 0x45495247u, x1 = 0x52494442u;
-  for (int r = 0; r < 10; r++) {
-    const uint64_t p0 = (uint64_t)0xD2511F53u * a0, p1 = (uint64_t)0xCD9E8D57u * a2;
-    const uint32_t n0 = (uint32_t)(p1 >> 32) ^ a1 ^ x0, n1 = (uint32_t)p1, n2 = (uint32_t)(p0 >> 32) ^ a3 ^ x1, n3 = (uint32_t)p0;
-    a0 = n0; a1 = n1; a2 = n2; a3 = n3;
-    x0 += 0x9E3779B9u; x1 += 0xBB67AE85u;
-  }
-  return (double)(((uint64_t)a0 | ((uint64_t)a1 << 32)) >> 11) * (1.0 / 9007199254740992.0);
-}
-
-bool mkdir_p(const std::string& p) {
-  std::string cur;
-  for (size_t i = 0; i <= p.size(); i++) {
-    if ((i == p.size() || p[i] == '/') && !cur.empty()) {
-      struct stat st;
-      if (stat(cur.c_str(), &st) != 0 && mkdir(cur.c_str(), 0777) != 0 && stat(cur.c_str(), &st) != 0) return false;
-    }
-    if (i < p.size()) cur += p[i];
-  }
-  return true;
-}
-
-}  // namespace
-
+// ---- CSV export of the best run (utils/csv_export.rs): the replay here, the files in report_files.cpp ----------------
 int eg_export_best_run_csv(eg_ctx* c, const eg_weights* w, const eg_run_cfg* cfg, const char* output_dir, char* written_dir) {
   int rc = check_cfg(c, cfg);
   if (rc) return rc;
@@ -726,241 +667,8 @@ int eg_export_best_run_csv(eg_ctx* c, const eg_weights* w, const eg_run_cfg* cfg
   rcfg.replay_best = 0;
   eg_sites sites;
   if ((rc = eg_replay_batch(c, &rcfg, &traj, 1, &res, &sites, &yearly))) return rc;
-
-  char ts[32];
-  const std::time_t t = std::time(nullptr);
-  std::tm tmv;
-  localtime_r(&t, &tmv);
-  std::strftime(ts, sizeof(ts), "%Y%m%d_%H%M%S", &tmv);  // CsvExporter::new, csv_export.rs:114-128
-  const std::string dir = std::string(output_dir) + "/" + ts;
-  if (!mkdir_p(dir + "/yearly_details")) return eg_fail(EG_ERR_IO, "cannot create " + dir);
-  const EgSmallTables& T = c->htab.small;
-
-  {  // simulation_summary.csv, csv_export.rs:215-432
-    std::FILE* f = std::fopen((dir + "/simulation_summary.csv").c_str(), "w");
-    if (!f) return eg_fail(EG_ERR_IO, "cannot write simulation_summary.csv in " + dir);
-    std::fprintf(f, "Simulation Summary\nTimestamp,%s\n\n", ts);
-    std::fprintf(f, "Final Metrics\nFinal Net Emissions (tonnes CO2),%s\n", rust_display(res.net_emissions).c_str());
-    std::fprintf(f, "Average Public Opinion (%%),%s\n", fixed(res.public_opinion * 100.0, 2).c_str());
-    std::fprintf(f, "Total Cost (\xE2\x82\xAC),%s\n", fixed(res.total_cost, 2).c_str());
-    std::fprintf(f, "Power Reliability (%%),%s\n\n", fixed(res.power_reliability * 100.0, 2).c_str());
-    std::fprintf(f, "Actions Taken\nYear,Action Type,Generator Type,Generator ID,Operation %%,Offset Type,Estimated Cost (\xE2\x82\xAC)\n");
-    for (int y = 0; y < EG_NY; y++) {
-      // SimulationResult.actions holds the additional actions only (simulation.rs:193, iteration.rs:90)
-      for (int i = traj.n_deficit[y]; i < traj.n_deficit[y] + traj.n_additional[y]; i++) {
-        const int a = traj.actions[row[y] + i];
-        const int year = EG_BASE_YEAR + y;
-        if (a < 45) {
-          const int tp = a / 3, m = a % 3;
-          // calc_generator_cost(type, base_cost(year), year, can_be_urban, requires_water, requires_water) * multiplier / 100
-          const double cost = c->htab.plant_terms[(size_t)EG_OPC_INDEX(y, tp, 0, y) * 2 + 1] * T.mult[m];
-          std::fprintf(f, "%d,AddGenerator,%s,,,,%s\n", year, kCsvGenNames[tp], fixed(cost, 2).c_str());
-        } else if (a < 57) {
-          const int o = (a - 45) / 3, m = (a - 45) % 3;
-          const double cost = (T.off_base_cost[o] * T.year[y].inflation) * T.mult[m];
-          std::fprintf(f, "%d,AddCarbonOffset,,,,%s,%s\n", year, kCsvOffsetNames[o], fixed(cost, 2).c_str());
-        } else if (a == EG_ACT_UPGRADE) std::fprintf(f, "%d,UpgradeEfficiency,,,,,0.00\n", year);   // empty id: no generator found
-        else if (a == EG_ACT_ADJUST) std::fprintf(f, "%d,AdjustOperation,,,0,,0.00\n", year);
-        else if (a == EG_ACT_CLOSE) std::fprintf(f, "%d,CloseGenerator,,,,,0.00\n", year);
-        else std::fprintf(f, "%d,DoNothing,,,,,0.00\n", year);
-      }
-    }
-    std::fprintf(f, "\nYearly Summary Metrics\n");
-    std::fprintf(f, "Year,Population,PowerUsage,PowerGeneration,PowerBalance,PublicOpinion,YearlyCapitalCost,TotalCapitalCost,Inflation,CO2Emissions,"
-                    "CarbonOffset,NetEmissions,YearlyRevenue,TotalRevenue,ActiveGenerators,YearlyUpgradeCosts,YearlyClosureCosts,YearlyTotalCost,TotalCost\n");
-    for (int y = 0; y < EG_NY; y++) {
-      const eg_year_metrics& m = yearly.y[y];
-      std::fprintf(f, "%d,%u,%.2f,%.2f,%.2f,%.4f,%.2f,%.2f,%.4f,%.2f,%.2f,%.2f,%.2f,%.2f,%u,%.2f,%.2f,%.2f,%.2f\n", EG_BASE_YEAR + y, m.total_population,
-                   m.total_power_usage, m.total_power_generation, m.power_balance, m.average_public_opinion, m.yearly_capital_cost,
-                   m.total_capital_cost, m.inflation_factor, m.total_co2_emissions, m.total_carbon_offset, m.net_co2_emissions,
-                   m.yearly_carbon_credit_revenue, m.total_carbon_credit_revenue, m.active_generators, 0.0, 0.0, m.yearly_total_cost, m.total_cost);
-    }
-    std::fclose(f);
-  }
-  if (!w->history.empty()) {  // improvement_history.csv, csv_export.rs:155-212
-    std::FILE* f = std::fopen((dir + "/improvement_history.csv").c_str(), "w");
-    if (!f) return eg_fail(EG_ERR_IO, "cannot write improvement_history.csv in " + dir);
-    std::fprintf(f, "Iteration,Score,Net Emissions (tonnes),Total Cost (\xE2\x82\xAC),Public Opinion (%%),Power Reliability (%%),Score Improvement (%%),Timestamp\n");
-    double prev = 0.0;
-    for (size_t i = 0; i < w->history.size(); i++) {
-      const EgImprovement& h = w->history[i];
-      const double imp = (i > 0 && prev > 0.0) ? ((h.score - prev) / prev) * 100.0 : 0.0;
-      std::fprintf(f, "%u,%.6f,%.2f,%.2f,%.2f,%.2f,%.2f,%s\n", h.iteration, h.score, h.net_emissions, h.total_cost, h.public_opinion * 100.0,
-                   h.power_reliability * 100.0, imp, h.timestamp.c_str());
-      prev = h.score;
-    }
-    std::fclose(f);
-  }
-  {  // yearly_details/settlements.csv, csv_export.rs:456-530 (population and usage re-derived from the 2025 values, as there)
-    std::FILE* f = std::fopen((dir + "/yearly_details/settlements.csv").c_str(), "w");
-    if (!f) return eg_fail(EG_ERR_IO, "cannot write settlements.csv in " + dir);
-    std::fprintf(f, "Year,Name,Longitude,Latitude,Population,PowerUsage\n");
-    const EgHostMap& m = c->hmap;
-    for (int y = 0; y < EG_NY; y++) {
-      // f64::powi lowers to repeated squaring (compiler-rt __powidf2); reproduce it for 1.01^n and 1.02^n
-      auto powi = [](double a, int b) { double r = 1.0; bool recip = b < 0; for (;;) { if (b & 1) r *= a; b /= 2; if (b == 0) break; a *= a; } return recip ? 1.0 / r : r; };
-      for (size_t s = 0; s < m.sx.size(); s++) {
-        const double xv = std::min(std::max(m.sx[s], 0.0), 50000.0), yv = std::min(std::max(m.sy[s], 0.0), 50000.0);
-        const double lon = -10.6 + ((-5.9 - -10.6) * (xv / 50000.0)), lat = 51.4 + ((55.4 - 51.4) * (yv / 50000.0));  // transform_grid_to_lat_lon, csv_export.rs:42-83
-        const uint32_t pop = (uint32_t)std::round((double)m.spop[s] * powi(1.01, y));
-        const double usage = ((double)m.spop[s] * 0.001) * powi(1.02, y);  // settlement power usage of the loader: population x 1 kW in MW
-        std::fprintf(f, "%d,%s,%.6f,%.6f,%u,%s\n", EG_BASE_YEAR + y, s < m.sname.size() ? m.sname[s].c_str() : ("Settlement_" + std::to_string(s)).c_str(),
-                     lon, lat, pop, rust_display(usage).c_str());
-      }
-    }
-    std::fclose(f);
-  }
-  {  // yearly_details/generators.csv, csv_export.rs:532-984
-    // `Generator.eol` holds a lifespan in years, so the exporter's first pass (`year > eol`, :701) skips every plant of the
-    // map and all rows come from its second pass (:813-979): one row per generator listed as active in that year's
-    // metrics, with type, commissioning year and end of life parsed back out of the id and the remaining columns filled
-    // from per-type defaults; plants added during the run get the id-hash coordinates of :867-869, pre-existing plants
-    // their real ones. Row order inside a year is HashMap order there; here: pre-existing plants, then build order.
-    std::FILE* f = std::fopen((dir + "/yearly_details/generators.csv").c_str(), "w");
-    if (!f) return eg_fail(EG_ERR_IO, "cannot write generators.csv in " + dir);
-    std::fprintf(f, "Year,Generator ID,Type,Longitude,Latitude,Power Output (MW),Efficiency (%%),Operation (%%),CO2 Output (tonnes),Is Active,"
-                    "Commissioning Year,End of Life Year,Size,Capital Cost (\xE2\x82\xAC),Operating Cost (\xE2\x82\xAC),Total Annual Cost (\xE2\x82\xAC),"
-                    "Reliability Factor,Planning Time (years),Construction Time (years),Construction Speed\n");
-    static const double kDefPower[EG_NT] = {50.0, 200.0, 0.01, 0.5, 50.0, 1000.0, 500.0, 400.0, 100.0, 50.0, 250.0, 200.0, 50.0, 30.0, 20.0};
-    static const double kDefCo2PerKwh[EG_NT] = {0, 0, 0, 0, 0, 0, 3.0, 0.4, 0.5, 0.1, 0, 0, 0, 0, 0};
-    static const double kDefCostPerMw[EG_NT] = {1500000.0, 3500000.0, 1000000.0, 800000.0, 600000.0, 6000000.0, 2000000.0, 1000000.0,
-                                                500000.0, 3000000.0, 2500000.0, 2000000.0, 400000.0, 5000000.0, 4000000.0};
-    static const double kDefReliability[EG_NT] = {0.35, 0.35, 0.25, 0.25, 0.25, 0.95, 0.90, 0.85, 0.90, 0.80, 0.75, 0.95, 0.98, 0.45, 0.40};
-    struct Plant { std::string id; int type, first_year, commissioning; double x, y; };
-    std::vector<Plant> plants;
-    const EgHostMap& m = c->hmap;
-    for (size_t g = 0; g < m.ex.size(); g++)  // "Existing_{type}_{n}" (generators_loader.rs:190): the third id field is the row number
-      plants.push_back({std::string("Existing_") + kCsvGenNames[m.etype[g]] + "_" + std::to_string(g), m.etype[g],
-                        g < c->htab.ex_online_year.size() && c->htab.ex_online_year[g] ? c->htab.ex_online_year[g] : 1 << 30, (int)g, m.ex[g], m.ey[g]});
-    for (int y = 0; y < EG_NY; y++)
-      for (int i = 0; i < traj.n_deficit[y] + traj.n_additional[y]; i++) {
-        const int a = traj.actions[row[y] + i];
-        if (a >= 45 || sites.site[row[y] + i] == EG_SITE_NONE) continue;
-        const int year = EG_BASE_YEAR + y;
-        Plant p{std::string("Gen_") + kCsvGenNames[a / 3] + "_" + std::to_string(year) + "_" + std::to_string(plants.size()), a / 3, year, year, 0, 0};
-        uint32_t h = 0;
-        for (unsigned char ch : p.id) h += ch;
-        p.x = 5000.0 + (double)(h % 100) / 100.0 * (50000.0 - 10000.0);
-        p.y = 5000.0 + (double)((h / 100) % 100) / 100.0 * (50000.0 - 10000.0);
-        plants.push_back(p);
-      }
-    for (int y = 0; y < EG_NY; y++) {
-      const int year = EG_BASE_YEAR + y;
-      for (const Plant& p : plants) {
-        if (p.first_year > year) continue;
-        const int t = p.type;
-        const double xv = std::min(std::max(p.x, 0.0), 50000.0), yv = std::min(std::max(p.y, 0.0), 50000.0);
-        const double lon = -10.6 + ((-5.9 - -10.6) * (xv / 50000.0)), lat = 51.4 + ((55.4 - 51.4) * (yv / 50000.0));
-        const double power = kDefPower[t];
-        const double co2 = kDefCo2PerKwh[t] == 0 ? 0.0 : power * kDefCo2PerKwh[t] * 8760.0 / 1000.0;
-        const double size = t == 0 ? power / 3.0 : t == 1 ? power / 8.0 : t == 2 ? power * 8.0 : t == 3 ? power * 6.0 : t == 4 ? power * 2.0 : power / 50.0;
-        const double capital = power * kDefCostPerMw[t], operating = capital * 0.03;
-        double planning, construction;
-        eg_host_tech_durations(t, p.commissioning, &planning, &construction);
-        // efficiency 0.99 and operation 100 (get_operation_percentage, a 0..100 value that the exporter scales by 100 again)
-        std::fprintf(f, "%d,%s,%s,%.6f,%.6f,%.2f,%.2f,%.2f,%.2f,true,%d,%d,%.2f,%.2f,%.2f,%.2f,%.2f,%.2f,%.2f,Normal\n", year, p.id.c_str(), kCsvGenNames[t],
-                     lon, lat, power, 0.99 * 100.0, 100.0 * 100.0, co2, p.commissioning, p.commissioning + 25, size * 100.0, capital, operating,
-                     capital + operating, kDefReliability[t], planning, construction);
-      }
-    }
-    std::fclose(f);
-  }
-  {  // yearly_details/carbon_offsets.csv, csv_export.rs:987-1093
-    // The exporter rebuilds the offsets on a copy of the base map, whose construction delays are on and whose clock stands
-    // at 2024 (multi_simulation.rs:862-888, map_handler.rs:785-811): every offset is still `Planned` when the rows are
-    // written, so calc_carbon_offset is 0 in every year and the size column, derived from it (:1353-1366), is 0 as well.
-    // Coordinates are thread_rng draws there (actions.rs:142-144); here a Philox stream keyed by the offset's position.
-    std::FILE* f = std::fopen((dir + "/yearly_details/carbon_offsets.csv").c_str(), "w");
-    if (!f) return eg_fail(EG_ERR_IO, "cannot write carbon_offsets.csv in " + dir);
-    std::fprintf(f, "Year,Offset ID,Type,X,Y,Size,Capture Efficiency (%%),Power Consumption (MW),CO2 Offset (tonnes),Negative CO2 Emissions (tonnes),"
-                    "Cost (\xE2\x82\xAC),Operating Cost (\xE2\x82\xAC),Total Annual Cost (\xE2\x82\xAC),Cost Per Tonne (\xE2\x82\xAC)\n");
-    static const double kOffOperating[EG_N_OFFSET_TYPES] = {10000.0, 15000.0, 100000.0, 5000.0};
-    static const double kOffOpTrend[EG_N_OFFSET_TYPES] = {1.0, 1.01, 0.97, 1.02};
-    struct Offset { std::string id; int type, year, mult; double x, y; };
-    std::vector<Offset> offs;
-    for (int y = 0; y < EG_NY; y++)
-      for (int i = traj.n_deficit[y]; i < traj.n_deficit[y] + traj.n_additional[y]; i++) {
-        const int a = traj.actions[row[y] + i];
-        if (a < 45 || a >= 57) continue;
-        const int o = (a - 45) / 3, year = EG_BASE_YEAR + y;
-        Offset r{std::string("Offset_") + kCsvOffsetNames[o] + "_" + std::to_string(year) + "_" + std::to_string(offs.size()), o, year, (a - 45) % 3, 0, 0};
-        r.x = csv_uniform((uint32_t)offs.size(), 0) * 50000.0;
-        r.y = csv_uniform((uint32_t)offs.size(), 1) * 50000.0;
-        offs.push_back(r);
-      }
-    auto powi = [](double a, int b) { double r = 1.0; for (;;) { if (b & 1) r *= a; b /= 2; if (b == 0) break; a *= a; } return r; };
-    for (int y = 0; y < EG_NY; y++) {
-      const int year = EG_BASE_YEAR + y;
-      for (const Offset& r : offs) {
-        if (year < r.year) continue;
-        const double lon = -10.6 + ((-5.9 - -10.6) * (r.x / 50000.0)), lat = 51.4 + ((55.4 - 51.4) * (r.y / 50000.0));
-        const double cost = (T.off_base_cost[r.type] * powi(1.0 + 0.0185, y)) * T.mult[r.mult];                       // carbon_offset.rs:188-195
-        const double operating = kOffOperating[r.type] * T.year[y].inflation * std::pow(kOffOpTrend[r.type], (double)y);  // :197-209
-        std::fprintf(f, "%d,%s,%s,%.6f,%.6f,0,%.2f,%s,0.00,-0.00,%.2f,%.2f,%.2f,0.00\n", year, r.id.c_str(), kCsvOffsetNames[r.type], lon, lat,
-                     0.85 * 100.0, r.type == 2 ? "50" : "0", cost, operating, cost + operating);
-      }
-    }
-    std::fclose(f);
-  }
-  {  // operation_logs/generator_operation_logs.csv, csv_export.rs:1096-1310: the year loop there runs over
-     // commissioning_year..=min(eol, 2050) with eol a lifespan (25..60 years), an empty range, so only the header is written
-    if (!mkdir_p(dir + "/operation_logs")) return eg_fail(EG_ERR_IO, "cannot create " + dir + "/operation_logs");
-    std::FILE* f = std::fopen((dir + "/operation_logs/generator_operation_logs.csv").c_str(), "w");
-    if (!f) return eg_fail(EG_ERR_IO, "cannot write generator_operation_logs.csv in " + dir);
-    std::fprintf(f, "Year,Month,Day,Hour,Generator ID,Type,Power Output (MW),Operation %%,Actual Output (MW),Weather Factor,CO2 Emissions (tonnes)\n");
-    std::fclose(f);
-  }
-  if (written_dir) std::snprintf(written_dir, 512, "%s", dir.c_str());
-  return EG_OK;
+  return eg_write_best_run_csv(output_dir, w, c->hmap, c->htab, traj, row, res, yearly, sites, written_dir);
 }
-
-namespace {
-
-EgSuitabilityParams suitability_params(const eg_ctx* c, int use_loaded_map, int mode, int half, int side, double step, uint32_t year_first,
-                                       uint32_t n_years, uint32_t first, uint32_t n, double* d_scores) {
-  EgSuitabilityParams p{};
-  p.mode = mode; p.half = half; p.side = side; p.step = step; p.first = first; p.n = n;
-  p.year_first = (int)year_first; p.n_years = (int)n_years;
-  p.n_settlements = use_loaded_map ? (int)c->hmap.sx.size() : 0;
-  p.sx = c->d_sx; p.sy = c->d_sy; p.pop = c->d_pop; p.urban_r = c->d_urban_r; p.urban_r_max = c->urban_r_max;
-  p.n_generators = use_loaded_map ? (int)c->hmap.ex.size() : 0;
-  p.gx = c->d_ex; p.gy = c->d_ey;
-  p.n_coast = (int)c->hmap.cx.size(); p.cx = c->d_cx; p.cy = c->d_cy;
-  p.scores = d_scores;
-  return p;
-}
-
-int ensure_suit_rows(eg_ctx* c, const EgSuitabilityParams& p) {
-  const size_t need = eg_suitability_rows_bytes(p.mode == 0 ? 2 * p.half + 1 : p.side);
-  if (need > c->suit_rows_cap) {
-    if (c->d_suit_rows) cudaFree(c->d_suit_rows);
-    c->d_suit_rows = nullptr; c->suit_rows_cap = 0;
-    EG_CUDA(cudaMalloc((void**)&c->d_suit_rows, need));
-    c->suit_rows_cap = need;
-  }
-  return EG_OK;
-}
-
-// runs the kernel into a temporary device buffer and copies the scores to the host
-int suitability_to_host(eg_ctx* c, const EgSuitabilityParams& p0, double* scores_out) {
-  EG_CUDA(cudaSetDevice(c->device));
-  EgSuitabilityParams p = p0;
-  const size_t count = (size_t)p.n * p.n_years * EG_NT;
-  double* d_scores = nullptr;
-  EG_CUDA(cudaMalloc((void**)&d_scores, std::max<size_t>(count, 1) * sizeof(double)));
-  p.scores = d_scores;
-  cudaError_t err = cudaSuccess;
-  if (ensure_suit_rows(c, p) != EG_OK) err = cudaErrorMemoryAllocation;
-  if (err == cudaSuccess) err = eg_launch_suitability(p, c->d_suit_rows, c->stream);
-  if (err == cudaSuccess && count) c->launches += 2;
-  if (err == cudaSuccess) err = cudaMemcpyAsync(scores_out, d_scores, count * sizeof(double), cudaMemcpyDeviceToHost, c->stream);
-  if (err == cudaSuccess) err = cudaStreamSynchronize(c->stream);
-  cudaFree(d_scores);
-  if (err != cudaSuccess) return eg_fail(EG_ERR_CUDA, cudaGetErrorString(err));
-  return EG_OK;
-}
-
-}  // namespace
 
 int eg_location_analysis(eg_ctx* c, int use_loaded_map, int32_t half_steps, double step, double* scores_out,
                          uint32_t first_point, uint32_t n_points) {
@@ -980,27 +688,16 @@ int eg_location_analysis_year(eg_ctx* c, int use_loaded_map, uint32_t year_index
 
 int eg_location_analysis_sites_device(eg_ctx* c, int use_loaded_map, uint32_t sites_per_axis, double step, uint32_t year_first,
                                       uint32_t n_years, uint32_t first_site, uint32_t n_sites, double* d_scores) {
-  if (!c || !d_scores) return eg_fail(EG_ERR_INVALID, "eg_location_analysis_sites_device: NULL argument");
-  if (!c->map_ready) return eg_fail(EG_ERR_STATE, "no map loaded (the coastline polygon is needed)");
-  if (year_first >= EG_NY || n_years > EG_NY - year_first) return eg_fail(EG_ERR_INVALID, "year range outside 2025..2050");
-  if (sites_per_axis == 0 || sites_per_axis > 65535u) return eg_fail(EG_ERR_INVALID, "sites_per_axis out of range");
-  if ((uint64_t)first_site + n_sites > (uint64_t)sites_per_axis * sites_per_axis) return eg_fail(EG_ERR_INVALID, "site range exceeds the grid");
-  EG_CUDA(cudaSetDevice(c->device));
-  const EgSuitabilityParams p = suitability_params(c, use_loaded_map, 1, 0, (int)sites_per_axis, step, year_first, n_years, first_site, n_sites, d_scores);
-  int rc = ensure_suit_rows(c, p);
+  const int rc = check_sites_args(c, d_scores, "eg_location_analysis_sites_device", sites_per_axis, year_first, n_years, first_site, n_sites);
   if (rc) return rc;
-  EG_CUDA(eg_launch_suitability(p, c->d_suit_rows, c->stream));
-  if (n_sites && n_years) c->launches += 2;
-  return EG_OK;
+  EG_CUDA(use_device(c));
+  return launch_suitability(c, suitability_params(c, use_loaded_map, 1, 0, (int)sites_per_axis, step, year_first, n_years, first_site, n_sites, d_scores));
 }
 
 int eg_location_analysis_sites(eg_ctx* c, int use_loaded_map, uint32_t sites_per_axis, double step, uint32_t year_first, uint32_t n_years,
                                uint32_t first_site, uint32_t n_sites, double* scores_out) {
-  if (!c || !scores_out) return eg_fail(EG_ERR_INVALID, "eg_location_analysis_sites: NULL argument");
-  if (!c->map_ready) return eg_fail(EG_ERR_STATE, "no map loaded (the coastline polygon is needed)");
-  if (year_first >= EG_NY || n_years > EG_NY - year_first) return eg_fail(EG_ERR_INVALID, "year range outside 2025..2050");
-  if (sites_per_axis == 0 || sites_per_axis > 65535u) return eg_fail(EG_ERR_INVALID, "sites_per_axis out of range");
-  if ((uint64_t)first_site + n_sites > (uint64_t)sites_per_axis * sites_per_axis) return eg_fail(EG_ERR_INVALID, "site range exceeds the grid");
+  const int rc = check_sites_args(c, scores_out, "eg_location_analysis_sites", sites_per_axis, year_first, n_years, first_site, n_sites);
+  if (rc) return rc;
   return suitability_to_host(c, suitability_params(c, use_loaded_map, 1, 0, (int)sites_per_axis, step, year_first, n_years, first_site, n_sites, nullptr), scores_out);
 }
 
@@ -1013,103 +710,7 @@ int eg_location_analysis_write(eg_ctx* c, int use_loaded_map, double min_suitabi
   std::vector<double> scores((size_t)side * side * EG_NT);
   int rc = eg_location_analysis_year(c, use_loaded_map, 0, half, step, scores.data(), 0, (uint32_t)(side * side));
   if (rc) return rc;
-  struct Loc { double x, y; std::vector<int> types; };
-  std::vector<Loc> locations;
-  size_t type_counts[EG_NT] = {0};
-  std::vector<size_t> type_to_locations[EG_NT];
-  size_t multi = 0;
-  auto clamp_map = [](double v) { return std::min(std::max(v, 0.0), 50000.0); };  // Coordinate::new, data/poi.rs:11-15
-  for (int i = -half; i <= half; i++)
-    for (int j = -half; j <= half; j++) {
-      const double* sc = &scores[((size_t)(i + half) * side + (size_t)(j + half)) * EG_NT];
-      Loc loc{clamp_map((double)i * step), clamp_map((double)j * step), {}};
-      for (int t = 0; t < EG_NT; t++)
-        if (sc[t] >= min_suitability) {
-          loc.types.push_back(t);
-          type_counts[t]++;
-          type_to_locations[t].push_back(locations.size());
-        }
-      if (!loc.types.empty()) {
-        if (loc.types.size() > 1) multi++;
-        locations.push_back(loc);
-      }
-    }
-  // scores of a stored location, by its position in the scan
-  auto score_of = [&](const Loc& l, int t) {
-    // locations keep their coordinates only; find the scan cell again through the coordinate (first cell with it: the
-    // clamped duplicates share their scores)
-    const int i = (int)(l.x / step), j = (int)(l.y / step);
-    return scores[((size_t)(i + half) * side + (size_t)(j + half)) * EG_NT + t];
-  };
-  if (cache_dir) {
-    if (!mkdir_p(cache_dir)) return eg_fail(EG_ERR_IO, std::string("cannot create ") + cache_dir);
-    // serde_json::to_string_pretty(LocationAnalysis): fields in declaration order; the HashMaps (unordered in the
-    // reference) are written in generator-type order
-    std::string o = "{\n  \"locations\": [";
-    for (size_t k = 0; k < locations.size(); k++) {
-      const Loc& l = locations[k];
-      o += k ? ",\n    {\n" : "\n    {\n";
-      o += "      \"coordinate\": {\n        \"x\": " + egjson::fmt_double(l.x) + ",\n        \"y\": " + egjson::fmt_double(l.y) + "\n      },\n";
-      o += "      \"suitability_scores\": {";
-      for (size_t q = 0; q < l.types.size(); q++)
-        o += std::string(q ? ",\n" : "\n") + "        \"" + kCsvGenNames[l.types[q]] + "\": " + egjson::fmt_double(score_of(l, l.types[q]));
-      o += "\n      }\n    }";
-    }
-    o += locations.empty() ? "],\n" : "\n  ],\n";
-    auto count_map = [&](const char* name) {
-      o += std::string("  \"") + name + "\": {";
-      bool first = true;
-      for (int t = 0; t < EG_NT; t++)
-        if (type_counts[t]) {
-          o += std::string(first ? "\n" : ",\n") + "    \"" + kCsvGenNames[t] + "\": " + std::to_string(type_counts[t]);
-          first = false;
-        }
-      o += first ? "},\n" : "\n  },\n";
-    };
-    count_map("type_counts");
-    o += "  \"multi_type_locations\": [";
-    bool first_multi = true;
-    for (const Loc& l : locations) {
-      if (l.types.size() < 2) continue;
-      o += first_multi ? "\n    [\n" : ",\n    [\n";
-      first_multi = false;
-      o += "      {\n        \"x\": " + egjson::fmt_double(l.x) + ",\n        \"y\": " + egjson::fmt_double(l.y) + "\n      },\n      [";
-      for (size_t q = 0; q < l.types.size(); q++) o += std::string(q ? ",\n" : "\n") + "        \"" + kCsvGenNames[l.types[q]] + "\"";
-      o += "\n      ]\n    ]";
-    }
-    o += first_multi ? "],\n" : "\n  ],\n";
-    count_map("remaining_spaces");
-    o += "  \"exhausted_types\": [],\n  \"type_to_locations\": {";
-    bool first_type = true;
-    for (int t = 0; t < EG_NT; t++) {
-      if (type_to_locations[t].empty()) continue;
-      o += std::string(first_type ? "\n" : ",\n") + "    \"" + kCsvGenNames[t] + "\": [";
-      first_type = false;
-      for (size_t q = 0; q < type_to_locations[t].size(); q++) o += std::string(q ? ",\n" : "\n") + "      " + std::to_string(type_to_locations[t][q]);
-      o += "\n    ]";
-    }
-    o += first_type ? "}\n}" : "\n  }\n}";
-    const std::string path = std::string(cache_dir) + "/location_analysis.json";
-    FILE* f = std::fopen(path.c_str(), "wb");
-    if (!f || std::fwrite(o.data(), 1, o.size(), f) != o.size()) { if (f) std::fclose(f); return eg_fail(EG_ERR_IO, "cannot write " + path); }
-    std::fclose(f);
-  }
-  if (text_path) {
-    std::string o = "Location Analysis Results\n========================\n\n";
-    o += "Total suitable locations: " + std::to_string(locations.size()) + "\nMulti-type locations: " + std::to_string(multi) + "\n\n";
-    o += "Locations by Generator Type:\n--------------------------\n";
-    for (int t = 0; t < EG_NT; t++)
-      if (type_counts[t]) o += std::string(kCsvGenNames[t]) + ": " + std::to_string(type_counts[t]) + "\n";
-    o += "\nDetailed Location Data:\n---------------------\n";
-    for (const Loc& l : locations) {
-      o += "\nCoordinate: (" + rust_display(l.x) + ", " + rust_display(l.y) + ")\n";
-      for (int t : l.types) o += std::string("  ") + kCsvGenNames[t] + ": " + fixed(score_of(l, t), 3) + "\n";
-    }
-    FILE* f = std::fopen(text_path, "wb");
-    if (!f || std::fwrite(o.data(), 1, o.size(), f) != o.size()) { if (f) std::fclose(f); return eg_fail(EG_ERR_IO, std::string("cannot write ") + text_path); }
-    std::fclose(f);
-  }
-  return EG_OK;
+  return eg_write_location_analysis(scores, half, step, min_suitability, cache_dir, text_path);
 }
 
 }  // extern "C"

@@ -1,4 +1,4 @@
-// host_tables.hpp — host-side map (as loaded) and the small host-built tables.
+// host_tables.hpp — host-side map (as loaded), the small host-built tables, and the output files written from them.
 #pragma once
 #include <cstdint>
 #include <string>
@@ -34,3 +34,11 @@ int eg_host_map_validate(const EgHostMap& m);
 void eg_host_build_tables(const EgHostMap& m, EgHostTables* out);
 // planning_duration / construction_duration of config/tech_type.rs:70-200 for a generator type registered in `year`
 void eg_host_tech_durations(int type, int year, double* planning, double* construction);
+
+// report_files.cpp: the six CSV files of the best run under <output_dir>/<timestamp>/ from its replay (`traj`, year y from
+// slot row[y]; the directory goes to `written_dir`, 512 bytes, unless NULL), and location_analysis.json in `cache_dir` and
+// the text report at `text_path` (either may be NULL) from the scores [(2 half + 1)^2][EG_NT] of analyze_map's grid
+int eg_write_best_run_csv(const char* output_dir, const eg_weights* w, const EgHostMap& hmap, const EgHostTables& htab, const eg_traj& traj,
+                          const int* row, const eg_result& res, const eg_yearly& yearly, const eg_sites& sites, char* written_dir);
+int eg_write_location_analysis(const std::vector<double>& scores, int half, double step, double min_suitability, const char* cache_dir,
+                               const char* text_path);

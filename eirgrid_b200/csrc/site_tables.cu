@@ -102,9 +102,7 @@ __global__ void __launch_bounds__(256) eg_site_rank_kernel(const EgSiteBuildPara
   if (me < p.n_sites) {
     const int mi = me / p.grid_n;
     p.order[base + rank] = (uint16_t)((mi << 8) | (me - mi * p.grid_n));  // packed (i, j) of the site
-    p.static_sorted[base + rank] = mine;
     const double pre = p.prefix[((size_t)c_pc_rclass[pc] * EG_NY + y) * p.n_sites + me];
-    p.prefix_sorted[base + rank] = pre;
     p.walk[base + rank] = make_double2(mine, pre);
   }
 }

@@ -22,11 +22,9 @@ struct EgSiteBuildParams {
   double* prefix;          // [6][26][n_sites]  score after settlements and existing plants per radius class
   double* coast_factor;    // [n_sites]
   double* site_opinion;    // [n_sites]
-  double* static_unsorted; // [7][26][n_sites]
+  double* static_unsorted; // [7][26][n_sites] scratch: static scores in site order
   uint16_t* order;         // [7][26][n_sites]
-  double* static_sorted;   // [7][26][n_sites]
-  double* prefix_sorted;   // [7][26][n_sites]
-  double2* walk;           // [7][26][n_sites] (static_sorted, prefix_sorted) interleaved: one 16-byte read per walk entry
+  double2* walk;           // [7][26][n_sites] (static score, prefix score) in `order`: one 16-byte read per walk entry
 };
 
 // launches 3 kernels on `stream`; returns the number of launches in *launches

@@ -76,9 +76,9 @@ struct EgDeviceMap {      // device pointers + sizes, passed by value to the ker
   const double* coast_factor;     // [n_sites] 1/(1+min_coast_distance/5000)                  metal_location_search.rs:157-162
   // placement lists, sorted by static score (descending, ties by scan order), per (pclass, year)
   const uint16_t* order;          // [7][26][n_sites] candidate site as (i << 8) | j
-  const double* static_score;     // [7][26][n_sites] score of the site when no simulation-built plant is in range
-  const double* prefix_score;     // [7][26][n_sites] score after settlements + existing plants (before new plants)
-  const double* walk;             // [7][26][n_sites][2] (static_score, prefix_score) interleaved, what the placement walk reads
+  const void* unused[2];          // read by no kernel, but without these 16 bytes `order` and `walk` share one 16-byte constant
+                                  // load and the episode kernels compile to a different instruction schedule
+  const double* walk;             // [7][26][n_sites][2] (static score, prefix score) of the sorted site, what the placement walk reads
   const double* near_factor;      // [6][r2_stride] distance/radius by squared cell distance d2 (valid for d2 < r2_limit[rc])
   const int* r2_limit;            // [6] first squared cell distance that is NOT inside the penalty radius, followed by
                                   // [6] start of the class in the compact table (prefix sums of the limits) and [1] its size

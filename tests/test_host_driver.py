@@ -137,6 +137,32 @@ def test_host_two_gpus_equal_one_gpu(host_binary, tmp_path):
     assert list(out[0].best_metrics) == list(out[1].best_metrics)
 
 
+@pytest.mark.gpu
+def test_host_two_gpus_export_best_run_csv(host_binary, tmp_path):
+    """The CSV export replays the best run on the first GPU's context while the second GPU, which ran the last training batch,
+    is still the current device: the replay must run on the first context's device and export what one GPU exports."""
+    import torch
+    if torch.cuda.device_count() < 2:
+        pytest.skip("needs 2 GPUs")
+    cache = str(tmp_path / "cache")
+    os.makedirs(cache)
+    open(os.path.join(cache, "location_analysis.json"), "w").write("{}")
+    summaries = []
+    for devs, ck in (("0", "ck1"), ("0,1", "ck2")):
+        r = subprocess.run([host_binary, "--assets", ASSETS, "-c", str(tmp_path / ck), "-C", cache, "--master-seed", "5", "-n", "9",
+                            "--no-continue", "--devices", devs], capture_output=True, text=True)
+        assert r.returncode == 0, r.stderr
+        s = json.loads(r.stdout.strip().split("\n")[-1])
+        assert s["training_batches"]["episodes"] == 9 and "Enhanced simulation results exported to" in r.stdout
+        (export,) = os.listdir(os.path.join(s["run_dir"], "enhanced_csv"))
+        out = os.path.join(s["run_dir"], "enhanced_csv", export)
+        for f in ("yearly_details/settlements.csv", "yearly_details/generators.csv", "yearly_details/carbon_offsets.csv",
+                  "operation_logs/generator_operation_logs.csv"):
+            assert os.path.exists(os.path.join(out, f)), f
+        summaries.append([l for l in open(os.path.join(out, "simulation_summary.csv")) if not l.startswith("Timestamp,")])
+    assert summaries[0] == summaries[1]
+
+
 def test_analyze_locations_tool_flags_and_failure_without_gpu(host_binary):
     """host/analyze_locations.cpp mirrors aiSimulator/bin/analyze_locations.rs:7-17 (flags -m / -o / -c with the same defaults)"""
     tool = os.path.join(os.path.dirname(host_binary), "analyze_locations")
