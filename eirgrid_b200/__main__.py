@@ -47,7 +47,7 @@ def parse_args(argv=None):
     # additions of this implementation
     ap.add_argument("--assets", default=os.path.join("aiSimulator", "assets"), help="directory with settlements.json, ireland_generators.csv, coastline_points.json")
     ap.add_argument("--batch-size", type=_positive, default=65536, help="episodes in flight per GPU")
-    ap.add_argument("--update-mode", choices=["batch", "sequential", "sequential-host"], default="batch")
+    ap.add_argument("--update-mode", choices=["batch", "sequential"], default="batch")
     ap.add_argument("--master-seed", type=_unsigned, default=None, help="seed of the per-episode RNG streams when --seed is not given")
     return ap.parse_args(argv)
 

@@ -1,4 +1,4 @@
-// eg_math.hpp — exp / ln / pow for the weight-update rule, ONE source for the host and the device.
+// eg_math.hpp — exp / ln / pow for the weight-update rule and Philox4x32-10, ONE source for the host and the device.
 //
 // The reference's update (ai/learning/weights/learning.rs:131-373) calls f64::exp, f64::powf and (through score_metrics,
 // ai/metrics/scoring.rs:12-13) f64::ln with per-episode arguments: the deterioration of every episode goes through
@@ -217,5 +217,19 @@ EGM_HD double pow(double x, double y) {
   if (y == 1.0) return sign * x;
   return sign * exp_dd(mul_d(log_dd(x), y));
 }
+
+// Philox4x32-10 (Salmon et al., SC '11) of the counter x under the key (k0, k1), in place: every counter-based stream
+// outside the episode kernel (whose philox_u64 is its own, tuned form) draws from this one
+EGM_HD void philox4x32_10(uint32_t x[4], uint32_t k0, uint32_t k1) {
+  for (int r = 0; r < 10; r++) {
+    const uint64_t p0 = (uint64_t)0xD2511F53u * x[0], p1 = (uint64_t)0xCD9E8D57u * x[2];
+    const uint32_t n0 = (uint32_t)(p1 >> 32) ^ x[1] ^ k0, n1 = (uint32_t)p1, n2 = (uint32_t)(p0 >> 32) ^ x[3] ^ k1, n3 = (uint32_t)p0;
+    x[0] = n0; x[1] = n1; x[2] = n2; x[3] = n3;
+    k0 += 0x9E3779B9u; k1 += 0xBB67AE85u;
+  }
+}
+
+// the low 64 bits of a Philox output, words (lo, hi), as a 53-bit uniform in [0, 1)
+EGM_HD double uniform53(uint32_t lo, uint32_t hi) { return (double)((((uint64_t)hi << 32) | lo) >> 11) * (1.0 / 9007199254740992.0); }
 
 }  // namespace egm

@@ -6,16 +6,12 @@
 #include <cstring>
 #include <ctime>
 #include "common.hpp"
+#include "eg_math.hpp"
 #include "host_tables.hpp"
 #include "json_min.hpp"
 #include "weights.hpp"
 
 namespace {
-
-const char* const kCsvGenNames[EG_NT] = {"OnshoreWind", "OffshoreWind", "DomesticSolar", "CommercialSolar", "UtilitySolar", "Nuclear", "CoalPlant",
-                                         "GasCombinedCycle", "GasPeaker", "Biomass", "HydroDam", "PumpedStorage", "BatteryStorage",
-                                         "TidalGenerator", "WaveEnergy"};
-const char* const kCsvOffsetNames[EG_N_OFFSET_TYPES] = {"Forest", "Wetland", "ActiveCapture", "CarbonCredit"};
 
 // Rust's `{}` for f64: shortest digits that round-trip, never scientific notation
 std::string rust_display(double v) {
@@ -41,14 +37,9 @@ std::string fixed(double v, int prec) {
 
 // uniform in [0,1) for the exported offset coordinates: Philox4x32-10, counter (index, axis, 0, "CSVO")
 double csv_uniform(uint32_t index, uint32_t axis) {
-  uint32_t a0 = index, a1 = axis, a2 = 0u, a3 = 0x4353564Fu, x0 = 0x45495247u, x1 = 0x52494442u;
-  for (int r = 0; r < 10; r++) {
-    const uint64_t p0 = (uint64_t)0xD2511F53u * a0, p1 = (uint64_t)0xCD9E8D57u * a2;
-    const uint32_t n0 = (uint32_t)(p1 >> 32) ^ a1 ^ x0, n1 = (uint32_t)p1, n2 = (uint32_t)(p0 >> 32) ^ a3 ^ x1, n3 = (uint32_t)p0;
-    a0 = n0; a1 = n1; a2 = n2; a3 = n3;
-    x0 += 0x9E3779B9u; x1 += 0xBB67AE85u;
-  }
-  return (double)(((uint64_t)a0 | ((uint64_t)a1 << 32)) >> 11) * (1.0 / 9007199254740992.0);
+  uint32_t x[4] = {index, axis, 0u, 0x4353564Fu};
+  egm::philox4x32_10(x, 0x45495247u, 0x52494442u);
+  return egm::uniform53(x[0], x[1]);
 }
 
 bool mkdir_p(const std::string& p) {
@@ -97,11 +88,11 @@ int eg_write_best_run_csv(const char* output_dir, const eg_weights* w, const EgH
           const int tp = a / 3, m = a % 3;
           // calc_generator_cost(type, base_cost(year), year, can_be_urban, requires_water, requires_water) * multiplier / 100
           const double cost = htab.plant_terms[(size_t)EG_OPC_INDEX(y, tp, 0, y) * 2 + 1] * T.mult[m];
-          std::fprintf(f, "%d,AddGenerator,%s,,,,%s\n", year, kCsvGenNames[tp], fixed(cost, 2).c_str());
+          std::fprintf(f, "%d,AddGenerator,%s,,,,%s\n", year, kGenNames[tp], fixed(cost, 2).c_str());
         } else if (a < 57) {
           const int o = (a - 45) / 3, m = (a - 45) % 3;
           const double cost = (T.off_base_cost[o] * T.year[y].inflation) * T.mult[m];
-          std::fprintf(f, "%d,AddCarbonOffset,,,,%s,%s\n", year, kCsvOffsetNames[o], fixed(cost, 2).c_str());
+          std::fprintf(f, "%d,AddCarbonOffset,,,,%s,%s\n", year, kOffsetNames[o], fixed(cost, 2).c_str());
         } else if (a == EG_ACT_UPGRADE) std::fprintf(f, "%d,UpgradeEfficiency,,,,,0.00\n", year);   // empty id: no generator found
         else if (a == EG_ACT_ADJUST) std::fprintf(f, "%d,AdjustOperation,,,0,,0.00\n", year);
         else if (a == EG_ACT_CLOSE) std::fprintf(f, "%d,CloseGenerator,,,,,0.00\n", year);
@@ -171,14 +162,14 @@ int eg_write_best_run_csv(const char* output_dir, const eg_weights* w, const EgH
     std::vector<Plant> plants;
     const EgHostMap& m = hmap;
     for (size_t g = 0; g < m.ex.size(); g++)  // "Existing_{type}_{n}" (generators_loader.rs:190): the third id field is the row number
-      plants.push_back({std::string("Existing_") + kCsvGenNames[m.etype[g]] + "_" + std::to_string(g), m.etype[g],
+      plants.push_back({std::string("Existing_") + kGenNames[m.etype[g]] + "_" + std::to_string(g), m.etype[g],
                         g < htab.ex_online_year.size() && htab.ex_online_year[g] ? htab.ex_online_year[g] : 1 << 30, (int)g, m.ex[g], m.ey[g]});
     for (int y = 0; y < EG_NY; y++)
       for (int i = 0; i < traj.n_deficit[y] + traj.n_additional[y]; i++) {
         const int a = traj.actions[row[y] + i];
         if (a >= 45 || sites.site[row[y] + i] == EG_SITE_NONE) continue;
         const int year = EG_BASE_YEAR + y;
-        Plant p{std::string("Gen_") + kCsvGenNames[a / 3] + "_" + std::to_string(year) + "_" + std::to_string(plants.size()), a / 3, year, year, 0, 0};
+        Plant p{std::string("Gen_") + kGenNames[a / 3] + "_" + std::to_string(year) + "_" + std::to_string(plants.size()), a / 3, year, year, 0, 0};
         uint32_t h = 0;
         for (unsigned char ch : p.id) h += ch;
         p.x = 5000.0 + (double)(h % 100) / 100.0 * (50000.0 - 10000.0);
@@ -199,7 +190,7 @@ int eg_write_best_run_csv(const char* output_dir, const eg_weights* w, const EgH
         double planning, construction;
         eg_host_tech_durations(t, p.commissioning, &planning, &construction);
         // efficiency 0.99 and operation 100 (get_operation_percentage, a 0..100 value that the exporter scales by 100 again)
-        std::fprintf(f, "%d,%s,%s,%.6f,%.6f,%.2f,%.2f,%.2f,%.2f,true,%d,%d,%.2f,%.2f,%.2f,%.2f,%.2f,%.2f,%.2f,Normal\n", year, p.id.c_str(), kCsvGenNames[t],
+        std::fprintf(f, "%d,%s,%s,%.6f,%.6f,%.2f,%.2f,%.2f,%.2f,true,%d,%d,%.2f,%.2f,%.2f,%.2f,%.2f,%.2f,%.2f,Normal\n", year, p.id.c_str(), kGenNames[t],
                      lon, lat, power, 0.99 * 100.0, 100.0 * 100.0, co2, p.commissioning, p.commissioning + 25, size * 100.0, capital, operating,
                      capital + operating, kDefReliability[t], planning, construction);
       }
@@ -224,7 +215,7 @@ int eg_write_best_run_csv(const char* output_dir, const eg_weights* w, const EgH
         const int a = traj.actions[row[y] + i];
         if (a < 45 || a >= 57) continue;
         const int o = (a - 45) / 3, year = EG_BASE_YEAR + y;
-        Offset r{std::string("Offset_") + kCsvOffsetNames[o] + "_" + std::to_string(year) + "_" + std::to_string(offs.size()), o, year, (a - 45) % 3, 0, 0};
+        Offset r{std::string("Offset_") + kOffsetNames[o] + "_" + std::to_string(year) + "_" + std::to_string(offs.size()), o, year, (a - 45) % 3, 0, 0};
         r.x = csv_uniform((uint32_t)offs.size(), 0) * 50000.0;
         r.y = csv_uniform((uint32_t)offs.size(), 1) * 50000.0;
         offs.push_back(r);
@@ -236,7 +227,7 @@ int eg_write_best_run_csv(const char* output_dir, const eg_weights* w, const EgH
         const double lon = -10.6 + ((-5.9 - -10.6) * (r.x / 50000.0)), lat = 51.4 + ((55.4 - 51.4) * (r.y / 50000.0));
         const double cost = (T.off_base_cost[r.type] * powi(1.0 + 0.0185, y)) * T.mult[r.mult];                       // carbon_offset.rs:188-195
         const double operating = kOffOperating[r.type] * T.year[y].inflation * std::pow(kOffOpTrend[r.type], (double)y);  // :197-209
-        std::fprintf(f, "%d,%s,%s,%.6f,%.6f,0,%.2f,%s,0.00,-0.00,%.2f,%.2f,%.2f,0.00\n", year, r.id.c_str(), kCsvOffsetNames[r.type], lon, lat,
+        std::fprintf(f, "%d,%s,%s,%.6f,%.6f,0,%.2f,%s,0.00,-0.00,%.2f,%.2f,%.2f,0.00\n", year, r.id.c_str(), kOffsetNames[r.type], lon, lat,
                      0.85 * 100.0, r.type == 2 ? "50" : "0", cost, operating, cost + operating);
       }
     }
@@ -296,7 +287,7 @@ int eg_write_location_analysis(const std::vector<double>& scores, int half, doub
       o += "      \"coordinate\": {\n        \"x\": " + egjson::fmt_double(l.x) + ",\n        \"y\": " + egjson::fmt_double(l.y) + "\n      },\n";
       o += "      \"suitability_scores\": {";
       for (size_t q = 0; q < l.types.size(); q++)
-        o += std::string(q ? ",\n" : "\n") + "        \"" + kCsvGenNames[l.types[q]] + "\": " + egjson::fmt_double(score_of(l, l.types[q]));
+        o += std::string(q ? ",\n" : "\n") + "        \"" + kGenNames[l.types[q]] + "\": " + egjson::fmt_double(score_of(l, l.types[q]));
       o += "\n      }\n    }";
     }
     o += locations.empty() ? "],\n" : "\n  ],\n";
@@ -305,7 +296,7 @@ int eg_write_location_analysis(const std::vector<double>& scores, int half, doub
       bool first = true;
       for (int t = 0; t < EG_NT; t++)
         if (type_counts[t]) {
-          o += std::string(first ? "\n" : ",\n") + "    \"" + kCsvGenNames[t] + "\": " + std::to_string(type_counts[t]);
+          o += std::string(first ? "\n" : ",\n") + "    \"" + kGenNames[t] + "\": " + std::to_string(type_counts[t]);
           first = false;
         }
       o += first ? "},\n" : "\n  },\n";
@@ -318,7 +309,7 @@ int eg_write_location_analysis(const std::vector<double>& scores, int half, doub
       o += first_multi ? "\n    [\n" : ",\n    [\n";
       first_multi = false;
       o += "      {\n        \"x\": " + egjson::fmt_double(l.x) + ",\n        \"y\": " + egjson::fmt_double(l.y) + "\n      },\n      [";
-      for (size_t q = 0; q < l.types.size(); q++) o += std::string(q ? ",\n" : "\n") + "        \"" + kCsvGenNames[l.types[q]] + "\"";
+      for (size_t q = 0; q < l.types.size(); q++) o += std::string(q ? ",\n" : "\n") + "        \"" + kGenNames[l.types[q]] + "\"";
       o += "\n      ]\n    ]";
     }
     o += first_multi ? "],\n" : "\n  ],\n";
@@ -327,7 +318,7 @@ int eg_write_location_analysis(const std::vector<double>& scores, int half, doub
     bool first_type = true;
     for (int t = 0; t < EG_NT; t++) {
       if (type_to_locations[t].empty()) continue;
-      o += std::string(first_type ? "\n" : ",\n") + "    \"" + kCsvGenNames[t] + "\": [";
+      o += std::string(first_type ? "\n" : ",\n") + "    \"" + kGenNames[t] + "\": [";
       first_type = false;
       for (size_t q = 0; q < type_to_locations[t].size(); q++) o += std::string(q ? ",\n" : "\n") + "      " + std::to_string(type_to_locations[t][q]);
       o += "\n    ]";
@@ -343,11 +334,11 @@ int eg_write_location_analysis(const std::vector<double>& scores, int half, doub
     o += "Total suitable locations: " + std::to_string(locations.size()) + "\nMulti-type locations: " + std::to_string(multi) + "\n\n";
     o += "Locations by Generator Type:\n--------------------------\n";
     for (int t = 0; t < EG_NT; t++)
-      if (type_counts[t]) o += std::string(kCsvGenNames[t]) + ": " + std::to_string(type_counts[t]) + "\n";
+      if (type_counts[t]) o += std::string(kGenNames[t]) + ": " + std::to_string(type_counts[t]) + "\n";
     o += "\nDetailed Location Data:\n---------------------\n";
     for (const Loc& l : locations) {
       o += "\nCoordinate: (" + rust_display(l.x) + ", " + rust_display(l.y) + ")\n";
-      for (int t : l.types) o += std::string("  ") + kCsvGenNames[t] + ": " + fixed(score_of(l, t), 3) + "\n";
+      for (int t : l.types) o += std::string("  ") + kGenNames[t] + ": " + fixed(score_of(l, t), 3) + "\n";
     }
     FILE* f = std::fopen(text_path, "wb");
     if (!f || std::fwrite(o.data(), 1, o.size(), f) != o.size()) { if (f) std::fclose(f); return eg_fail(EG_ERR_IO, std::string("cannot write ") + text_path); }

@@ -11,30 +11,18 @@
 //             [183,198) occurrences of deficit key k in current_deficit_actions
 // Integer sums make the result independent of the reduction order and of the number of GPUs.
 #include "stats.cuh"
+#include "update_rule.hpp"
 #include <algorithm>
 
 namespace {
 
-constexpr double kMaxAcceptableCost = 50000000000.0, kMaxAcceptableEmissions = 1000000.0;
-
 __device__ __forceinline__ double default_score(const eg_result& r, double ln100, bool cost_only = false) {  // scoring.rs:5-44
-  if (cost_only) return 2.0 - fmin(log(fmax(r.total_cost / kMaxAcceptableCost, 1.0)) / ln100, 1.0);
-  if (r.net_emissions > 0.0) return 1.0 - fmin(r.net_emissions / kMaxAcceptableEmissions, 1.0);
-  const double normalized_cost = fmax(r.total_cost / kMaxAcceptableCost, 1.0);
+  if (cost_only) return 2.0 - fmin(log(fmax(r.total_cost / egrule::kMaxCost, 1.0)) / ln100, 1.0);
+  if (r.net_emissions > 0.0) return 1.0 - fmin(r.net_emissions / egrule::kMaxEmissions, 1.0);
+  const double normalized_cost = fmax(r.total_cost / egrule::kMaxCost, 1.0);
   const double cost_score = 1.0 - fmin(log(normalized_cost) / ln100, 1.0);
   const double cost_weight = normalized_cost > 8.0 ? 0.8 : 0.5;
   return 1.0 + (cost_score * cost_weight + r.public_opinion * (1.0 - cost_weight));
-}
-
-__device__ __forceinline__ int deficit_key_of_action(int code) {
-  if (code == EG_ACT_DO_NOTHING) return 14;
-  if (code >= 45 || code % 3) return -1;
-  switch (code / 3) {
-    case 8: return 0; case 7: return 1; case 12: return 2; case 11: return 3; case 9: return 4; case 0: return 5;
-    case 1: return 6; case 4: return 7; case 10: return 8; case 5: return 9; case 2: return 10; case 3: return 11;
-    case 13: return 12; case 14: return 13;
-  }
-  return -1;
 }
 
 __global__ void eg_stats_reset_kernel(double* best_score, unsigned long long* best_index) {
@@ -138,7 +126,7 @@ __global__ void __launch_bounds__(256) eg_stats_kernel(const EgStatsParams p) {
       unsigned long long* ys = acc + EG_STATS_HEADER + y * EG_STATS_YEAR_STRIDE;
       if (i < y_nrun) atomicAdd(&ys[2 * EG_N_ACTIONS + a], 1ull);
       else {
-        const int k = deficit_key_of_action(a);
+        const int k = egrule::deficit_key_of_action(a);
         if (k >= 0) atomicAdd(&ys[3 * EG_N_ACTIONS + k], 1ull);
       }
       if (!pass) continue;

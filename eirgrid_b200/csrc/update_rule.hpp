@@ -6,9 +6,11 @@
 // handful of factors — boost, penalty, mild penalty — that are then multiplied into the table entries of the actions
 // the episode and the best strategy recorded. Everything up to those factors is here, written once, so that the two
 // forms execute the same IEEE operations in the same order (host: -ffp-contract=off, device: --fmad=false) and end with
-// the same bits. exp / ln / pow come from eg_math.hpp for the same reason.
+// the same bits. exp / ln / pow come from eg_math.hpp for the same reason. The weight clamps, the scoring constants and the
+// deficit-key order are defined here only: the episode kernel, the batch statistics and the file writers use them too.
 #pragma once
 #include "eg_math.hpp"
+#include "tables.h"
 
 namespace egrule {
 
@@ -87,18 +89,12 @@ EGM_HD Contrast deficit_contrast(uint32_t iwi, double learning_rate) {
 }
 
 // The randomisation branch draws from a counter-based stream of our own (the reference uses thread_rng there, which no
-// run can reproduce): draw d of the episode with iteration counter c is the low 64 bits of
-// Philox4x32-10(counter = (c, 0, d, "UPDT"), key = rng_seed), as a 53-bit uniform in [0, 1).
+// run can reproduce): draw d of the episode with iteration counter c is Philox4x32-10(counter = (c, 0, d, "UPDT"),
+// key = rng_seed) as a 53-bit uniform.
 EGM_HD double update_uniform(uint32_t key_lo, uint32_t key_hi, uint32_t iteration, uint32_t draw) {
-  uint32_t a0 = iteration, a1 = 0u, a2 = draw, a3 = 0x55504454u, x0 = key_lo, x1 = key_hi;
-  for (int r = 0; r < 10; r++) {
-    const uint64_t p0 = (uint64_t)0xD2511F53u * a0, p1 = (uint64_t)0xCD9E8D57u * a2;
-    const uint32_t n0 = (uint32_t)(p1 >> 32) ^ a1 ^ x0, n1 = (uint32_t)p1, n2 = (uint32_t)(p0 >> 32) ^ a3 ^ x1, n3 = (uint32_t)p0;
-    a0 = n0; a1 = n1; a2 = n2; a3 = n3;
-    x0 += 0x9E3779B9u; x1 += 0xBB67AE85u;
-  }
-  const uint64_t u = (uint64_t)a0 | ((uint64_t)a1 << 32);
-  return (double)(u >> 11) * (1.0 / 9007199254740992.0);
+  uint32_t x[4] = {iteration, 0u, draw, 0x55504454u};
+  egm::philox4x32_10(x, key_lo, key_hi);
+  return egm::uniform53(x[0], x[1]);
 }
 
 // one randomisation step of a weight: w * (1 + 0.25 * (2u - 1)) clamped like learning.rs:275-277
@@ -106,16 +102,33 @@ EGM_HD double random_factor(double u) { return 1.0 + 0.25 * (u * 2.0 - 1.0); }
 EGM_HD double apply_random_factor(double w, double f) { return min_std(max_std(w * f, kMinWeight), kMaxWeight); }
 EGM_HD double randomise(double w, double u) { return apply_random_factor(w, random_factor(u)); }
 
-// deficit key (weights/core.rs:130-152 insertion order) of an action code, -1 if the action is not a deficit key
+// Deficit keys in the insertion order of weights/core.rs:130-152: key k < 14 is AddGenerator(kDeficitKeyTypes[k], 100 %),
+// key 14 is DoNothing.
+constexpr int kDeficitKeyTypes[14] = {8, 7, 12, 11, 9, 0, 1, 4, 10, 5, 2, 3, 13, 14};
+
+// The same order as 4-bit fields of one word each, for branch-free lookups: the type of key k, and the key of type t
+// (0xF: CoalPlant, the one type without a key).
+constexpr uint64_t pack_types_of_keys() {
+  uint64_t v = 0;
+  for (int k = 0; k < 14; k++) v |= (uint64_t)kDeficitKeyTypes[k] << (4 * k);
+  return v;
+}
+constexpr uint64_t pack_keys_of_types() {
+  uint64_t v = (1ull << (4 * EG_NT)) - 1;
+  for (int k = 0; k < 14; k++) v ^= (uint64_t)(0xF ^ k) << (4 * kDeficitKeyTypes[k]);
+  return v;
+}
+constexpr uint64_t kTypeOfKey = pack_types_of_keys(), kKeyOfType = pack_keys_of_types();
+
+// action code of deficit key k (k >= 14: DoNothing)
+EGM_HD int deficit_key_action(uint32_t k) { return k < 14 ? 3 * (int)((kTypeOfKey >> (4 * k)) & 0xF) : EG_ACT_DO_NOTHING; }
+
+// deficit key of an action code, -1 if the action is not a deficit key
 EGM_HD int deficit_key_of_action(int code) {
-  if (code == 60) return 14;
-  if (code >= 45 || code % 3) return -1;
-  switch (code / 3) {
-    case 8: return 0; case 7: return 1; case 12: return 2; case 11: return 3; case 9: return 4; case 0: return 5;
-    case 1: return 6; case 4: return 7; case 10: return 8; case 5: return 9; case 2: return 10; case 3: return 11;
-    case 13: return 12; case 14: return 13;
-  }
-  return -1;
+  if (code == EG_ACT_DO_NOTHING) return 14;
+  if ((unsigned)code >= 45u || code % 3) return -1;
+  const int k = (int)((kKeyOfType >> (4 * (code / 3))) & 0xF);
+  return k == 0xF ? -1 : k;
 }
 
 }  // namespace egrule

@@ -31,9 +31,13 @@ struct eg_weights {
   eg_weights();
 };
 
-// default-mode score_metrics on the host (scoring.rs:18-44)
-double eg_score_default(const double m[4]);
-double eg_score(const double m[4], bool cost_only);
+// names the reference prints for the parts of an action key: GeneratorType and CarbonOffsetType variants in key order, cost
+// multipliers in percent
+constexpr const char* kGenNames[EG_NT] = {"OnshoreWind", "OffshoreWind", "DomesticSolar", "CommercialSolar", "UtilitySolar",
+                                          "Nuclear", "CoalPlant", "GasCombinedCycle", "GasPeaker", "Biomass", "HydroDam",
+                                          "PumpedStorage", "BatteryStorage", "TidalGenerator", "WaveEnergy"};
+constexpr const char* kOffsetNames[EG_N_OFFSET_TYPES] = {"Forest", "Wetland", "ActiveCapture", "CarbonCredit"};
+constexpr int kMultPercent[EG_N_MULTS] = {100, 120, 150};
 
 // fills the device-side snapshot (weights + per-batch constants of update_weights + best lists); false when the best
 // lists are longer than the snapshot's capacity (EG_BEST_CAPACITY / EG_TRAJ_CAPACITY slots) and were cut

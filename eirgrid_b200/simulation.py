@@ -121,7 +121,6 @@ def run_multi_simulation(asset_dir, num_iterations, parallel=True, continue_from
     update_mode "batch": device-side statistics + one allreduce per batch (DESIGN.md §update).
     update_mode "sequential": the reference's per-episode update in episode order, applied on the GPU (eg_update_device:
     exact reference rule with `batch_size` episodes sampled per snapshot; replicated on every rank).
-    update_mode "sequential-host": the same rule through eg_update on the host (every record copied back; the slow twin).
     The replay phase (last 10 % of the iterations) always runs the per-episode rule.
     Returns a summary dict; checkpoints are written like the reference's.
     """
@@ -132,8 +131,8 @@ def run_multi_simulation(asset_dir, num_iterations, parallel=True, continue_from
     distributed = dist.is_available() and dist.is_initialized()
     rank = dist.get_rank() if distributed else 0
     world = dist.get_world_size() if distributed else 1
-    if update_mode not in ("batch", "sequential", "sequential-host"):
-        raise ValueError("update_mode must be 'batch', 'sequential' or 'sequential-host'")
+    if update_mode not in ("batch", "sequential"):
+        raise ValueError("update_mode must be 'batch' or 'sequential'")
     os.makedirs(checkpoint_dir, exist_ok=True)
     # Everything a run derives from the clock or from the checkpoint directory is decided by rank 0 and broadcast: ranks that
     # looked for themselves could pick different seeds, or see rank 0's new (empty) run directory as the one to resume from.
@@ -188,21 +187,12 @@ def run_multi_simulation(asset_dir, num_iterations, parallel=True, continue_from
             trainer.set_batch(advance)
             st = trainer.step()
         else:
-            # Replay batches and the sequential modes run the reference's per-episode rule (it rebuilds the doubled records of
+            # Replay batches and the sequential mode run the reference's per-episode rule (it rebuilds the doubled records of
             # replay iterations, quirk Q10). The rule is sequential in the episodes: with several ranks the ROLLOUT of the batch is
             # sharded and the records are all-gathered, then every rank applies the same in-order update to the whole batch on
-            # its own GPU (identical inputs, identical tables, no further exchange). "sequential-host" replicates everything.
-            if update_mode == "sequential-host":
-                advance = min(per_gpu, phase_end - completed)
-                trainer.n = advance
-                trainer.upload_weights()
-                trainer.launch_rollout(first_episode=trainer.next_episode)
-                res, traj = trainer.fetch_results()
-                st = weights.update(res, traj, replay_best=replay_best, rng_seed=rng_seed)
-                trainer.next_episode += advance
-            else:
-                advance = min(per_gpu * world, phase_end - completed)
-                st = trainer.step_inorder_sharded(advance, rng_seed=rng_seed)
+            # its own GPU (identical inputs, identical tables, no further exchange).
+            advance = min(per_gpu * world, phase_end - completed)
+            st = trainer.step_inorder_sharded(advance, rng_seed=rng_seed)
         completed += advance
         n_flagged += int(st.n_flagged)
         if st.n_flagged and rank == 0:

@@ -89,7 +89,7 @@ void usage() {
       "      --enable-csv-export         (always on: summary, improvement history and settlements CSVs of the best run)\n"
       "      --debug-logging, --debug-weights, --track-weight-history\n"
       "      --enable-construction-delays\n"
-      "additions: --assets <DIR> --batch-size <N> --update-mode batch|sequential|sequential-host --master-seed <S> --devices 0,1,..");
+      "additions: --assets <DIR> --batch-size <N> --update-mode batch|sequential --master-seed <S> --devices 0,1,..");
 }
 
 Args parse(int argc, char** argv) {
@@ -146,8 +146,7 @@ Args parse(int argc, char** argv) {
     } else if (f == "-h" || f == "--help") { usage(); std::exit(0); }
     else die("unknown argument " + f);
   }
-  if (a.update_mode != "batch" && a.update_mode != "sequential" && a.update_mode != "sequential-host")
-    die("--update-mode must be batch, sequential or sequential-host");
+  if (a.update_mode != "batch" && a.update_mode != "sequential") die("--update-mode must be batch or sequential");
   if (a.update_mode != "batch" && a.devices.size() > 1) die("--update-mode sequential is single-GPU");
   if (a.batch_size == 0) die("--batch-size must be positive");
   return a;
@@ -310,8 +309,6 @@ int main(int argc, char** argv) {
   std::printf("Starting multi-simulation optimization with %llu iterations (%llu completed, %llu remaining) in directory %s\n",
               (unsigned long long)a.iterations, (unsigned long long)start_iteration, (unsigned long long)remaining0, run_dir.c_str());
 
-  std::vector<eg_result> results;
-  std::vector<eg_traj> trajs;
   std::vector<int64_t> stats(EG_STATS_WORDS), shard_stats(EG_STATS_WORDS);
   std::vector<unsigned char> records(G * EG_BEST_RECORD_BYTES);
   uint64_t completed = start_iteration;
@@ -327,8 +324,6 @@ int main(int argc, char** argv) {
   while (completed < a.iterations) {
     const double t_batch = now_s();
     const bool is_full_run = a.force_full_simulation || !cache_loaded || completed + final_full >= a.iterations;
-    bool has_best = false;
-    best_score_of(weights, &has_best);
     uint32_t nb[EG_N_YEARS], nbd[EG_N_YEARS];
     const bool has_best_actions = eg_weights_get_best(weights, nb, nullptr, 0, nbd, nullptr, 0) == 1;
     eg_run_cfg cfg{};
@@ -356,19 +351,11 @@ int main(int argc, char** argv) {
       t_train += now_s() - t_batch;
       n_train += done_now;
     } else {
-      // replay batches and the sequential modes: the reference's per-episode update in episode order (it rebuilds the doubled
-      // records of replay iterations, quirk Q10) — on the GPU (eg_update_device behind eg_train_batch_inorder), or with
-      // --update-mode sequential-host on the host after copying every record back (eg_update, the slow twin)
+      // replay batches and --update-mode sequential: the reference's per-episode update in episode order on the GPU
+      // (eg_update_device behind eg_train_batch_inorder; it rebuilds the doubled records of replay iterations, quirk Q10)
       const uint64_t phase_end = (is_full_run || final_full >= a.iterations) ? a.iterations : a.iterations - final_full;
       const uint32_t n_s = (uint32_t)std::min<uint64_t>(per_gpu, phase_end - completed);
-      if (a.update_mode == "sequential-host") {
-        results.resize(n_s);
-        trajs.resize(n_s);
-        check(eg_rollout_batch(ctx[0], weights, &cfg, rng_seed, completed, n_s, results.data(), trajs.data(), nullptr, nullptr), "eg_rollout_batch");
-        check(eg_update(weights, results.data(), trajs.data(), n_s, cfg.replay_best, rng_seed, &st), "eg_update");
-      } else {
-        check(eg_train_batch_inorder(ctx[0], weights, &cfg, rng_seed, completed, n_s, rng_seed, &st), "eg_train_batch_inorder");
-      }
+      check(eg_train_batch_inorder(ctx[0], weights, &cfg, rng_seed, completed, n_s, rng_seed, &st), "eg_train_batch_inorder");
       done_now = n_s;
       t_inorder += now_s() - t_batch;
       n_inorder += done_now;

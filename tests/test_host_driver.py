@@ -45,7 +45,7 @@ def test_host_fails_loudly_without_gpu(host_binary):
 def test_host_rejects_malformed_arguments(host_binary):
     """Like clap on the reference's Args (cli/cli.rs:4-62): a usage error, never an abort or a wrapped-around number."""
     for args in (["-n", "abc"], ["-n", "-5"], ["-n", "99999999999999999999"], ["--devices", "x"], ["--batch-size", "5000000000"],
-                 ["--batch-size", "0"], ["--update-mode", "weird"], ["--seed", "1.5"], ["--nonexistent"], ["-n"]):
+                 ["--batch-size", "0"], ["--update-mode", "weird"], ["--update-mode", "sequential-host"], ["--seed", "1.5"], ["--nonexistent"], ["-n"]):
         r = subprocess.run([host_binary] + args, capture_output=True, text=True)
         assert r.returncode == 2 and r.stderr.startswith("error: "), (args, r.returncode, r.stderr[:200])
         assert "terminate called" not in r.stderr
