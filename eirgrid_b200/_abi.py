@@ -132,6 +132,55 @@ class UpdateStats(C.Structure):
                 ("batch_best_score", C.c_double), ("batch_best_episode", C.c_int64), ("n_flagged", C.c_uint32), ("reserved", C.c_uint32)]
 
 
+EVAL_CHUNK = 65536
+EVAL_SCORE_BINS = 2048
+EVAL_N_FLAGS = 4
+FINAL_FIELDS = ["score", "net_emissions", "public_opinion", "total_cost", "power_reliability", "n_generators", "n_offsets",
+                "n_deficit_actions", "n_additional_actions"]
+EVAL_YEAR_FIELDS = ["total_population", "active_generators"] + YEAR_FIELDS[:-1]  # every field of eg_year_metrics but `reserved`
+MOMENTS = ["mean", "m2", "min", "max"]
+
+
+class EvalStats(C.Structure):
+    """eg_eval_stats: statistics of an evaluation (Context.evaluate). Moment arrays are [..., 4] = (mean, m2, min, max); the
+    numpy views share the structure's memory. The all-zero structure is the empty statistics."""
+    _fields_ = [("n_episodes", C.c_uint64), ("best_episode", C.c_uint64), ("worst_episode", C.c_uint64),
+                ("has_yearly", C.c_uint32), ("reserved", C.c_uint32),
+                ("final_metrics", (C.c_double * 4) * len(FINAL_FIELDS)),
+                ("yearly", ((C.c_double * 4) * len(EVAL_YEAR_FIELDS)) * N_YEARS),
+                ("n_flagged", C.c_uint64), ("flag_counts", C.c_uint64 * EVAL_N_FLAGS),
+                ("score_hist", C.c_uint64 * EVAL_SCORE_BINS), ("score_out_of_range", C.c_uint64),
+                ("net_zero_or_below", C.c_uint64 * N_YEARS), ("in_deficit", C.c_uint64 * N_YEARS),
+                ("first_net_zero_year", C.c_uint64 * (N_YEARS + 1)),
+                ("additional_actions", (C.c_uint64 * N_ACTIONS) * N_YEARS), ("deficit_actions", (C.c_uint64 * N_ACTIONS) * N_YEARS)]
+
+    def view(self, name):
+        """numpy view of an array field (e.g. view("final_metrics")[FINAL_FIELDS.index("score"), 0] is the mean score)"""
+        return np.ctypeslib.as_array(getattr(self, name))
+
+    def moments(self, field, year=None):
+        """{mean, m2, min, max} of a final metric, or of a yearly field in year index `year`"""
+        row = self.view("final_metrics")[FINAL_FIELDS.index(field)] if year is None else \
+            self.view("yearly")[year, EVAL_YEAR_FIELDS.index(field)]
+        return dict(zip(MOMENTS, (float(v) for v in row)))
+
+    def merge(self, other):
+        """self <- self followed by other (eg_eval_stats_merge); returns self"""
+        from . import _lib
+        _lib.check(_lib.lib().eg_eval_stats_merge(C.byref(self), C.byref(other)))
+        return self
+
+    def write_json(self, path):
+        """the record as JSON (eg_eval_stats_write_json)"""
+        import os
+        from . import _lib
+        _lib.check(_lib.lib().eg_eval_stats_write_json(C.byref(self), os.fsencode(path)))
+
+    @classmethod
+    def from_bytes(cls, data):
+        return cls.from_buffer_copy(bytes(data))
+
+
 def action_name(code):
     """Human-readable GridAction for an action code (ai/actions/grid_action.rs:18-40 Display format)."""
     if code < 45:

@@ -23,7 +23,7 @@ EXPORTS = [
     "eg_location_analysis_year", "eg_microbench_fp64", "eg_export_best_run_csv", "eg_weights_history_append", "eg_train_batch_begin", "eg_train_batch_end", "eg_train_batch_results", "eg_update_combine_apply",
     "eg_update_device", "eg_train_batch_inorder", "eg_rule_math",
     "eg_location_analysis_sites", "eg_location_analysis_sites_device", "eg_location_analysis_write",
-    "eg_update_pack_exchange_device",
+    "eg_update_pack_exchange_device", "eg_evaluate", "eg_eval_accumulate_device", "eg_eval_stats_merge", "eg_eval_stats_write_json",
 ]
 
 
@@ -96,6 +96,10 @@ def lib():
     L.eg_update_apply_stats.argtypes = [vp, vp, u64, vp, vp, i64, C.POINTER(_abi.UpdateStats)]
     L.eg_location_analysis.argtypes = [vp, C.c_int, C.c_int32, C.c_double, vp, u32, u32]
     L.eg_location_analysis_year.argtypes = [vp, C.c_int, u32, C.c_int32, C.c_double, vp, u32, u32]
+    L.eg_evaluate.argtypes = [vp, vp, C.POINTER(_abi.RunCfg), u64, u64, u64, u32, C.POINTER(_abi.EvalStats)]
+    L.eg_eval_accumulate_device.argtypes = [vp, vp, vp, vp, u32, u64, vp]
+    L.eg_eval_stats_merge.argtypes = [C.POINTER(_abi.EvalStats), C.POINTER(_abi.EvalStats)]
+    L.eg_eval_stats_write_json.argtypes = [C.POINTER(_abi.EvalStats), C.c_char_p]
     _lib = L
     return L
 
@@ -379,6 +383,20 @@ class Context:
         traj = np.zeros(n, _abi.TRAJ_DTYPE) if want_traj else None
         check(self.L.eg_train_batch_results(self.h, _abi.ptr(res), _abi.ptr(traj)))
         return res, traj
+
+    # ---- policy evaluation ----
+    def evaluate(self, weights, n, seed=1, first_episode=0, cfg=None, with_yearly=True):
+        """Statistics of episodes first_episode .. first_episode + n - 1 sampled from `weights`, reduced on the GPU."""
+        cfg = cfg or _abi.RunCfg()
+        st = _abi.EvalStats()
+        check(self.L.eg_evaluate(self.h, weights.h, C.byref(cfg), int(seed), int(first_episode), int(n), int(bool(with_yearly)),
+                                 C.byref(st)))
+        return st
+
+    def eval_accumulate_device(self, n, d_results, d_traj, d_yearly, first_global_episode, d_acc):
+        """Fold n episodes already on the device into the device record d_acc (eg_eval_stats bytes), on the ctx stream."""
+        check(self.L.eg_eval_accumulate_device(self.h, _dev_ptr(d_results), _dev_ptr(d_traj), _dev_ptr(d_yearly), int(n),
+                                               int(first_global_episode), _dev_ptr(d_acc)))
 
     def sync(self):
         check(self.L.eg_sync(self.h))

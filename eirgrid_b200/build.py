@@ -12,7 +12,7 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, os.environ.get("EIRGRID_LIB_NAME", "libeirgrid_b200.so"))
-SOURCES = ["engine.cu", "episode.cu", "site_tables.cu", "stats.cu", "update.cu", "suitability.cu", "microbench.cu", "weights.cpp", "host_tables.cpp", "report_files.cpp"]
+SOURCES = ["engine.cu", "episode.cu", "site_tables.cu", "stats.cu", "evaluate.cu", "update.cu", "suitability.cu", "microbench.cu", "weights.cpp", "host_tables.cpp", "report_files.cpp"]
 NVCC = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
 EXTRA = os.environ.get("EIRGRID_NVCC_EXTRA", "").split()
 FLAGS = EXTRA + ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "--fmad=false", "-std=c++17",

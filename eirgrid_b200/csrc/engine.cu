@@ -10,6 +10,7 @@
 #include "common.hpp"
 #include "device_buffer.hpp"
 #include "episode.cuh"
+#include "evaluate.cuh"
 #include "host_tables.hpp"
 #include "site_tables.cuh"
 #include "stats.cuh"
@@ -88,6 +89,11 @@ struct eg_ctx {
     PinnedArray<EgUpdSlot> h_slot;
     PinnedArray<EgUpdImprovement> h_imp;
   } upd;
+  struct EvalBuffers {  // eg_evaluate / eg_eval_accumulate_device: block partials of one chunk, eg_evaluate's record and its pinned host mirror
+    DeviceArray<EgEvalPartial> partials;
+    DeviceArray<eg_eval_stats> acc;
+    PinnedArray<eg_eval_stats> h_acc;
+  } eval;
   DeviceArray<EgUpdImprovement> upd_improvements;  // grown with the batch, at least EG_UPD_IMP_INLINE
   DeviceArray<double> suit_rows;       // scratch of the suitability kernel: crossing lists per site row
   DeviceArray<uint32_t> next_episode;  // work counter of the persistent episode kernels
@@ -179,6 +185,16 @@ int ensure_scratch(eg_ctx* c, size_t n, bool sites, bool yearly, bool traj_in) {
   if (sites && n > s.sites.size()) EG_CUDA(s.sites.alloc(n));
   if (yearly && n > s.yearly.size()) EG_CUDA(s.yearly.alloc(n));
   if (traj_in && n > s.traj_in.size()) EG_CUDA(s.traj_in.alloc(n));
+  return EG_OK;
+}
+
+int ensure_eval(eg_ctx* c) {
+  if (c->eval.partials.get()) return EG_OK;
+  eg_ctx::EvalBuffers e;
+  EG_CUDA(e.partials.alloc(EG_EVAL_CHUNK / EG_EVAL_SLICE));
+  EG_CUDA(e.acc.alloc(1));
+  EG_CUDA(e.h_acc.alloc(1));
+  c->eval = std::move(e);
   return EG_OK;
 }
 
@@ -640,6 +656,47 @@ int eg_train_batch_inorder(eg_ctx* c, eg_weights* w, const eg_run_cfg* cfg, uint
   if ((rc = eg_rollout_batch_device(c, cfg, seed, first_episode, n, s.out.get(), s.traj.get(), nullptr, nullptr))) return rc;
   c->train_n = n;
   return eg_update_device(c, w, s.out.get(), s.traj.get(), n, cfg->replay_best, rng_seed, stats_out);
+}
+
+// ---- policy evaluation (evaluate.cu) ----------------------------------------------------------------------------------
+int eg_eval_accumulate_device(eg_ctx* c, const eg_result* d_results, const eg_traj* d_traj, const eg_yearly* d_yearly, uint32_t n,
+                              uint64_t first_global_episode, eg_eval_stats* d_acc) {
+  if (!c || !d_results || !d_traj || !d_acc) return eg_fail(EG_ERR_INVALID, "eg_eval_accumulate_device: NULL argument");
+  EG_CUDA(use_device(c));
+  const int rc = ensure_eval(c);
+  if (rc) return rc;
+  // the chunks of eg_evaluate, so that both partition a range alike
+  for (uint32_t base = 0; base < n; base += EG_EVAL_CHUNK) {
+    const EgEvalParams p{d_results + base, d_traj + base, d_yearly ? d_yearly + base : nullptr, std::min<uint32_t>(EG_EVAL_CHUNK, n - base),
+                         first_global_episode + base, d_acc, c->eval.partials.get()};
+    EG_CUDA(eg_launch_eval(p, c->stream));
+    c->launches += 2;
+  }
+  return EG_OK;
+}
+
+int eg_evaluate(eg_ctx* c, const eg_weights* w, const eg_run_cfg* cfg, uint64_t seed, uint64_t first_episode, uint64_t n,
+                uint32_t with_yearly, eg_eval_stats* out) {
+  int rc = check_cfg(c, cfg);
+  if (rc) return rc;
+  if (!w || !out) return eg_fail(EG_ERR_INVALID, "eg_evaluate: NULL argument");
+  EG_CUDA(use_device(c));
+  if ((rc = eg_weights_upload(c, w))) return rc;
+  if ((rc = ensure_scratch(c, (size_t)std::min<uint64_t>(n, EG_EVAL_CHUNK), false, with_yearly != 0, false))) return rc;
+  const eg_ctx::Scratch& s = c->scratch;
+  eg_yearly* d_yearly = with_yearly ? s.yearly.get() : nullptr;
+  if ((rc = ensure_eval(c))) return rc;
+  eg_eval_stats* d_acc = c->eval.acc.get();
+  EG_CUDA(cudaMemsetAsync(d_acc, 0, sizeof(eg_eval_stats), c->stream));
+  for (uint64_t base = 0; base < n; base += EG_EVAL_CHUNK) {
+    const uint32_t cnt = (uint32_t)std::min<uint64_t>(EG_EVAL_CHUNK, n - base);
+    if ((rc = eg_rollout_batch_device(c, cfg, seed, first_episode + base, cnt, s.out.get(), s.traj.get(), nullptr, d_yearly))) return rc;
+    if ((rc = eg_eval_accumulate_device(c, s.out.get(), s.traj.get(), d_yearly, cnt, first_episode + base, d_acc))) return rc;
+  }
+  EG_CUDA(cudaMemcpyAsync(c->eval.h_acc.get(), d_acc, sizeof(eg_eval_stats), cudaMemcpyDeviceToHost, c->stream));
+  EG_CUDA(cudaStreamSynchronize(c->stream));
+  std::memcpy(out, c->eval.h_acc.get(), sizeof(eg_eval_stats));
+  return EG_OK;
 }
 
 // ---- CSV export of the best run (utils/csv_export.rs): the replay here, the files in report_files.cpp ----------------

@@ -346,3 +346,122 @@ int eg_write_location_analysis(const std::vector<double>& scores, int half, doub
   }
   return EG_OK;
 }
+
+// ---- the evaluation record as JSON (eg_eval_stats_write_json) -----------------------------------------------------------
+namespace {
+
+// shortest text that reads back as the same double; JSON has no NaN or infinity: null
+std::string json_number(double v) {
+  if (!std::isfinite(v)) return "null";
+  char buf[40];
+  for (int prec = 1; prec <= 17; prec++) {
+    std::snprintf(buf, sizeof(buf), "%.*g", prec, v);
+    if (std::strtod(buf, nullptr) == v) break;
+  }
+  return buf;
+}
+
+std::string json_moments(const eg_moments& m, uint64_t n) {
+  if (n == 0) return "null";
+  const double sd = n < 2 ? 0.0 : std::sqrt(m.m2 / (double)(n - 1));
+  return "{\"mean\": " + json_number(m.mean) + ", \"std\": " + json_number(sd) + ", \"min\": " + json_number(m.min) +
+         ", \"max\": " + json_number(m.max) + "}";
+}
+
+std::string json_fraction(uint64_t k, uint64_t n) { return n ? json_number((double)k / (double)n) : "null"; }
+
+const char* const kFinalNames[EG_EVAL_N_FINAL] = {"score", "net_emissions", "public_opinion", "total_cost", "power_reliability",
+                                                  "n_generators", "n_offsets", "n_deficit_actions", "n_additional_actions"};
+const char* const kYearFieldNames[EG_EVAL_N_YEAR_FIELDS] = {
+    "total_population", "active_generators", "total_power_usage", "total_power_generation", "power_balance", "average_public_opinion",
+    "yearly_capital_cost", "total_capital_cost", "inflation_factor", "total_co2_emissions", "total_carbon_offset", "net_co2_emissions",
+    "yearly_carbon_credit_revenue", "total_carbon_credit_revenue", "yearly_energy_sales_revenue", "total_energy_sales_revenue",
+    "yearly_total_cost", "total_cost"};
+const char* const kFlagNames[EG_EVAL_N_FLAGS] = {"gen_overflow", "offset_overflow", "record_overflow", "no_site"};
+
+}  // namespace
+
+extern "C" int eg_eval_stats_write_json(const eg_eval_stats* s, const char* path) {
+  if (!s || !path) return eg_fail(EG_ERR_INVALID, "eg_eval_stats_write_json: NULL argument");
+  const uint64_t n = s->n_episodes;
+  const bool yearly = s->has_yearly != 0;
+  const auto year_key = [](int y) { return "\"" + std::to_string(EG_BASE_YEAR + y) + "\""; };
+  std::string o = "{\n  \"episodes\": " + std::to_string(n) + ",\n  \"flagged\": {\"any\": " + std::to_string(s->n_flagged);
+  for (int b = 0; b < EG_EVAL_N_FLAGS; b++) o += std::string(", \"") + kFlagNames[b] + "\": " + std::to_string(s->flag_counts[b]);
+  o += "},\n  \"final\": {";
+  for (int f = 0; f < EG_EVAL_N_FINAL; f++)
+    o += std::string(f ? ",\n    \"" : "\n    \"") + kFinalNames[f] + "\": " + json_moments(s->final_metrics[f], n);
+  // quantile q of the scores in [0, 2]: lower edge of the bin that holds the ceil(q * m)-th smallest of those m scores
+  uint64_t in_range = 0;
+  for (int b = 0; b < EG_EVAL_SCORE_BINS; b++) in_range += s->score_hist[b];
+  o += "\n  },\n  \"score_quantiles\": {";
+  const int pct[7] = {1, 5, 25, 50, 75, 95, 99};
+  for (int q = 0; q < 7; q++) {
+    std::string v = "null";
+    if (in_range) {
+      const uint64_t rank = (pct[q] * in_range + 99) / 100;
+      uint64_t cum = 0;
+      for (int b = 0; b < EG_EVAL_SCORE_BINS; b++) {
+        cum += s->score_hist[b];
+        if (cum >= rank) { v = json_number(b / 1024.0); break; }
+      }
+    }
+    char key[8];
+    std::snprintf(key, sizeof(key), "p%02d", pct[q]);
+    o += std::string(q ? ", \"" : "\"") + key + "\": " + v;
+  }
+  o += "},\n  \"score_histogram\": {\"bin_width\": " + json_number(1.0 / 1024.0) + ", \"counts\": [";
+  for (int b = 0; b < EG_EVAL_SCORE_BINS; b++) o += (b ? ", " : "") + std::to_string(s->score_hist[b]);
+  o += "], \"out_of_range\": " + std::to_string(s->score_out_of_range) + "},\n";
+  o += "  \"best_episode\": " + (n ? std::to_string(s->best_episode) : std::string("null")) + ",\n";
+  o += "  \"worst_episode\": " + (n ? std::to_string(s->worst_episode) : std::string("null")) + ",\n";
+  o += "  \"yearly\": ";
+  if (!yearly) o += "null";
+  else {
+    o += "{";
+    for (int y = 0; y < EG_NY; y++) {
+      o += (y ? ",\n    " : "\n    ") + year_key(y) + ": {";
+      for (int f = 0; f < EG_EVAL_N_YEAR_FIELDS; f++)
+        o += std::string(f ? ", \"" : "\"") + kYearFieldNames[f] + "\": " + json_moments(s->yearly[y][f], n);
+      o += "}";
+    }
+    o += "\n  }";
+  }
+  const auto year_fractions = [&](const uint64_t* k) {
+    if (!yearly) return std::string("null");
+    std::string a = "[";
+    for (int y = 0; y < EG_NY; y++) a += (y ? ", " : "") + json_fraction(k[y], n);
+    return a + "]";
+  };
+  o += ",\n  \"p_net_zero_or_below\": " + year_fractions(s->net_zero_or_below);
+  o += ",\n  \"p_in_deficit\": " + year_fractions(s->in_deficit);
+  o += ",\n  \"first_net_zero_year\": ";
+  if (!yearly) o += "null";
+  else {
+    o += "{";
+    for (int y = 0; y <= EG_NY; y++)
+      o += (y ? ", " : "") + (y < EG_NY ? year_key(y) : std::string("\"never\"")) + ": " + std::to_string(s->first_net_zero_year[y]);
+    o += "}";
+  }
+  o += ",\n  \"actions\": {";
+  for (int y = 0; y < EG_NY; y++) {
+    o += (y ? ",\n    " : "\n    ") + year_key(y) + ": {";
+    const uint64_t* parts[2] = {s->additional_actions[y], s->deficit_actions[y]};
+    for (int k = 0; k < 2; k++) {
+      o += k ? ", \"deficit\": {" : "\"additional\": {";
+      bool first = true;
+      for (int a = 0; a < EG_N_ACTIONS; a++) {
+        if (!parts[k][a]) continue;
+        o += (first ? "\"" : ", \"") + eg_action_display(a) + "\": " + std::to_string(parts[k][a]);
+        first = false;
+      }
+      o += "}";
+    }
+    o += "}";
+  }
+  o += "\n  }\n}\n";
+  FILE* f = std::fopen(path, "wb");
+  if (!f || std::fwrite(o.data(), 1, o.size(), f) != o.size()) { if (f) std::fclose(f); return eg_fail(EG_ERR_IO, std::string("cannot write ") + path); }
+  if (std::fclose(f) != 0) return eg_fail(EG_ERR_IO, std::string("cannot write ") + path);
+  return EG_OK;
+}

@@ -11,6 +11,7 @@
 //             [183,198) occurrences of deficit key k in current_deficit_actions
 // Integer sums make the result independent of the reduction order and of the number of GPUs.
 #include "stats.cuh"
+#include "traj_items.cuh"
 #include "update_rule.hpp"
 #include <algorithm>
 
@@ -84,58 +85,22 @@ __global__ void __launch_bounds__(256) eg_stats_kernel(const EgStatsParams p) {
       if (pass) atomicAdd(&acc[1], 1ull);
       if (rp->flags) atomicAdd(&acc[2], 1ull);  // capacity overflow / no site: counted so that a driver can report it
     }
-    // The episode's records: current_run_actions ++ current_deficit_actions of every year, ~40 items in all, most of them
-    // in 2025. Lane y holds year y's counts; the items are numbered through all years (warp prefix sum) and dealt out 32 at
-    // a time, each lane finding its item's year by binary search over the prefix sums.
-    const eg_traj* t = p.trajs + ep;
-    int nd = 0, nrun = 0;
-    if (lane < EG_NY) { nd = t->n_deficit[lane]; nrun = nd + t->n_additional[lane]; }
-    // first slot of each year's row in the record (rows are stored back to back); counts that run past the capacity
-    // (never written by the episode kernels) are cut
-    int row_end = nrun;
-#pragma unroll
-    for (int o = 1; o < 32; o <<= 1) {
-      const int v = __shfl_up_sync(0xFFFFFFFFu, row_end, o);
-      if (lane >= o) row_end += v;
-    }
-    int row = row_end - nrun;
-    if (row > EG_TRAJ_CAPACITY) row = EG_TRAJ_CAPACITY;
-    if (row + nrun > EG_TRAJ_CAPACITY) { nrun = EG_TRAJ_CAPACITY - row; nd = min(nd, nrun); }
-    const int cnt = nrun + nd;
-    int incl = cnt;
-#pragma unroll
-    for (int o = 1; o < 32; o <<= 1) {
-      const int v = __shfl_up_sync(0xFFFFFFFFu, incl, o);
-      if (lane >= o) incl += v;
-    }
-    const int total = __shfl_sync(0xFFFFFFFFu, incl, 31);
-    for (int base = 0; base < total; base += 32) {
-      const int q = base + lane;
-      int y = 0;  // number of years whose items all come before item q
-#pragma unroll
-      for (int step = 16; step > 0; step >>= 1) {
-        const int v = __shfl_sync(0xFFFFFFFFu, incl, y + step - 1);
-        if (v <= q) y += step;
-      }
-      const int y_incl = __shfl_sync(0xFFFFFFFFu, incl, y), y_cnt = __shfl_sync(0xFFFFFFFFu, cnt, y);
-      const int y_nrun = __shfl_sync(0xFFFFFFFFu, nrun, y), y_row = __shfl_sync(0xFFFFFFFFu, row, y);
-      if (q >= total) continue;
-      const int i = q - (y_incl - y_cnt);
-      const int a = t->actions[y_row + (i < y_nrun ? i : i - y_nrun)];
-      if (a >= EG_N_ACTIONS) continue;  // not an action code (records are produced by the episode kernels; defensive)
+    // the episode's records: current_run_actions ++ current_deficit_actions of every year, dealt out to the lanes
+    eg_warp_traj_items(p.trajs + ep, lane, [&](int y, int i, int y_nrun, int, int a) {
+      if (a >= EG_N_ACTIONS) return;  // not an action code (records are produced by the episode kernels; defensive)
       unsigned long long* ys = acc + EG_STATS_HEADER + y * EG_STATS_YEAR_STRIDE;
       if (i < y_nrun) atomicAdd(&ys[2 * EG_N_ACTIONS + a], 1ull);
       else {
         const int k = egrule::deficit_key_of_action(a);
         if (k >= 0) atomicAdd(&ys[3 * EG_N_ACTIONS + k], 1ull);
       }
-      if (!pass) continue;
+      if (!pass) return;
       if (!((best_mask[y] >> a) & 1ull)) {
         atomicAdd(&ys[a], (unsigned long long)log_pen);
       } else if (i < (int)best_len[y]) {
         if (best_cat[best_start[y] + i] != a) atomicAdd(&ys[EG_N_ACTIONS + a], (unsigned long long)log_mild);
       }
-    }
+    });
   }
   if (lane == 0 && warp_best >= 0.0) atomicMax((long long*)p.best_score, __double_as_longlong(warp_best));  // scores are >= 0: bit order == value order
   __syncthreads();

@@ -470,6 +470,15 @@ EgContrastConsts eg_contrast_consts(const eg_weights& W) {
   return c;
 }
 
+std::string eg_action_display(int code) {  // impl Display for GridAction, ai/actions/grid_action.rs:18-41
+  if (code < 45) return std::string("AddGenerator(") + kGenNames[code / 3] + ", " + std::to_string(kMultPercent[code % 3]) + "%)";
+  if (code < 57) return std::string("AddCarbonOffset(") + kOffsetNames[(code - 45) / 3] + ", " + std::to_string(kMultPercent[(code - 45) % 3]) + "%)";
+  if (code == EG_ACT_UPGRADE) return "UpgradeEfficiency()";
+  if (code == EG_ACT_ADJUST) return "AdjustOperation(, 0%)";
+  if (code == EG_ACT_CLOSE) return "CloseGenerator()";
+  return "DoNothing";
+}
+
 extern "C" {
 
 uint8_t eg_deficit_key_action(uint32_t k) { return (uint8_t)deficit_key_action(k); }
@@ -788,14 +797,6 @@ int eg_update_apply_stats(eg_weights* w, const int64_t* stats, uint64_t n_total,
 
 int eg_weights_history_append(const eg_weights* w, uint64_t iteration, const char* history_path) {
   if (!w || !history_path) return eg_fail(EG_ERR_INVALID, "eg_weights_history_append: NULL argument");
-  auto action_display = [](int code) -> std::string {  // impl Display for GridAction, ai/actions/grid_action.rs:18-41
-    if (code < 45) return std::string("AddGenerator(") + kGenNames[code / 3] + ", " + std::to_string(kMultPercent[code % 3]) + "%)";
-    if (code < 57) return std::string("AddCarbonOffset(") + kOffsetNames[(code - 45) / 3] + ", " + std::to_string(kMultPercent[(code - 45) % 3]) + "%)";
-    if (code == EG_ACT_UPGRADE) return "UpgradeEfficiency()";
-    if (code == EG_ACT_ADJUST) return "AdjustOperation(, 0%)";
-    if (code == EG_ACT_CLOSE) return "CloseGenerator()";
-    return "DoNothing";
-  };
   const double best_score = w->has_best ? score_w(*w, w->best_metrics) : 0.0;
   char ts[48];
   {
@@ -824,7 +825,7 @@ int eg_weights_history_append(const eg_weights* w, uint64_t iteration, const cha
     }
     o += "}";
   };
-  rows("weights", EG_N_ACTIONS, &w->w[0][0], [&](int k) { return action_display(k); }, true);
+  rows("weights", EG_N_ACTIONS, &w->w[0][0], [&](int k) { return eg_action_display(k); }, true);
   o += ",\n";
   rows("action_count_weights", EG_N_COUNT_KEYS, &w->cw[0][0], [&](int k) { return std::to_string(k); }, w->has_count_weights);
   o += ",\n" + i3 + "\"learning_rate\": " + egjson::fmt_double(w->learning_rate);
@@ -833,7 +834,7 @@ int eg_weights_history_append(const eg_weights* w, uint64_t iteration, const cha
   o += ",\n" + i3 + "\"exploration_rate\": " + egjson::fmt_double(w->exploration_rate);
   o += ",\n" + i3 + "\"force_best_actions\": false";
   o += ",\n";
-  rows("deficit_weights", EG_N_DEFICIT_KEYS, &w->dw[0][0], [&](int k) { return action_display(deficit_key_action(k)); }, true);
+  rows("deficit_weights", EG_N_DEFICIT_KEYS, &w->dw[0][0], [&](int k) { return eg_action_display(deficit_key_action(k)); }, true);
   o += ",\n" + i3 + "\"guaranteed_best_actions\": false";
   o += ",\n" + i3 + "\"optimization_mode\": " + (w->optimization_mode.empty() ? std::string("null") : "\"" + w->optimization_mode + "\"");
   o += ",\n" + i3 + "\"best_score\": " + egjson::fmt_double(best_score) + "\n" + i2 + "},\n";

@@ -38,6 +38,8 @@ constexpr const char* kGenNames[EG_NT] = {"OnshoreWind", "OffshoreWind", "Domest
                                           "PumpedStorage", "BatteryStorage", "TidalGenerator", "WaveEnergy"};
 constexpr const char* kOffsetNames[EG_N_OFFSET_TYPES] = {"Forest", "Wetland", "ActiveCapture", "CarbonCredit"};
 constexpr int kMultPercent[EG_N_MULTS] = {100, 120, 150};
+// an action code as the reference prints the GridAction (impl Display, ai/actions/grid_action.rs:18-41)
+std::string eg_action_display(int code);
 
 // fills the device-side snapshot (weights + per-batch constants of update_weights + best lists); false when the best
 // lists are longer than the snapshot's capacity (EG_BEST_CAPACITY / EG_TRAJ_CAPACITY slots) and were cut

@@ -333,6 +333,60 @@ int eg_train_batch_results(eg_ctx* ctx, eg_result* out, eg_traj* traj_out /* nul
 int eg_update_combine_apply(eg_weights* w, const int64_t* stats_sum, const void* records, uint32_t n_records,
                             uint64_t n_total, uint64_t first_episode, eg_update_stats* stats_out);
 
+/* ---- policy evaluation: statistics of n episodes sampled from one table, reduced on the device -------------------------
+ * A fixed-size record; the all-zero record is the empty statistics. Moments are {mean, m2 = sum of squared deviations, min,
+ * max}, folded with Welford's update inside a block and merged with Chan et al.'s pairwise formula everywhere else. For fixed
+ * (weights, cfg, seed, first_episode, n) the record is the same bytes on every run. Integer parts, min/max and the best/worst ids
+ * do not depend on how the episode range is split; the moments of a split range differ from the unsplit ones in the last bits. */
+#define EG_EVAL_CHUNK 65536            /* episodes rolled out and reduced per step of eg_evaluate */
+#define EG_EVAL_SCORE_BINS 2048        /* score histogram over [0, 2]: bin = min(floor(score * 1024), 2047) */
+#define EG_EVAL_N_FLAGS 4              /* one counter per EG_FLAG_* bit */
+#define EG_EVAL_N_FINAL 9              /* score, net_emissions, public_opinion, total_cost, power_reliability, n_generators, n_offsets,
+                                          n_deficit_actions, n_additional_actions (the fields of eg_result in order) */
+#define EG_EVAL_N_YEAR_FIELDS 18       /* total_population, active_generators and the 16 f64 fields of eg_year_metrics before `reserved` */
+#define EG_EVAL_COUNTER_WORDS (1 + EG_EVAL_N_FLAGS + EG_EVAL_SCORE_BINS + 1 + 3 * EG_N_YEARS + 1 + 2 * EG_N_YEARS * EG_N_ACTIONS)
+
+typedef struct {
+  double mean, m2, min, max;
+} eg_moments;
+
+typedef struct {
+  uint64_t n_episodes;
+  uint64_t best_episode;               /* global episode id of the highest score, the lowest id among equal scores (0 if empty) */
+  uint64_t worst_episode;              /* the same for the lowest score */
+  uint32_t has_yearly;                 /* the per-year moments and counts below are filled */
+  uint32_t reserved;
+  eg_moments final_metrics[EG_EVAL_N_FINAL];
+  eg_moments yearly[EG_N_YEARS][EG_EVAL_N_YEAR_FIELDS];   /* follows final_metrics without a gap */
+  /* counters (EG_EVAL_COUNTER_WORDS words from n_flagged to the end): merged by addition */
+  uint64_t n_flagged;                  /* episodes with eg_result.flags != 0 */
+  uint64_t flag_counts[EG_EVAL_N_FLAGS];
+  uint64_t score_hist[EG_EVAL_SCORE_BINS];
+  uint64_t score_out_of_range;         /* scores outside [0, 2] and NaN */
+  uint64_t net_zero_or_below[EG_N_YEARS];       /* episodes with net_co2_emissions <= 0 in the year (yearly only) */
+  uint64_t in_deficit[EG_N_YEARS];              /* episodes with power_balance < 0 in the year (yearly only) */
+  uint64_t first_net_zero_year[EG_N_YEARS + 1]; /* first year with net_co2_emissions <= 0; [EG_N_YEARS] = never (yearly only) */
+  uint64_t additional_actions[EG_N_YEARS][EG_N_ACTIONS];  /* additional actions by year and code, as stored in eg_traj */
+  uint64_t deficit_actions[EG_N_YEARS][EG_N_ACTIONS];     /* deficit-handler actions by year and code */
+} eg_eval_stats;
+
+/* n episodes with ids first_episode .. first_episode + n - 1 sampled from w (uploads w as the ctx's snapshot, like
+ * eg_rollout_batch), rolled out and reduced on the device in chunks of EG_EVAL_CHUNK episodes; one copy to the host at the
+ * end. with_yearly = 0 reduces results and action records only, which runs the lean instantiation of the episode kernel
+ * whenever the snapshot allows it; 1 adds the per-year part. n = 0 gives the empty record. */
+int eg_evaluate(eg_ctx* ctx, const eg_weights* w, const eg_run_cfg* cfg, uint64_t seed, uint64_t first_episode, uint64_t n,
+                uint32_t with_yearly, eg_eval_stats* out);
+/* Folds n episodes already on the device (global ids first_global_episode..) into the DEVICE record *d_acc, asynchronously on
+ * the ctx stream, in the chunks eg_evaluate uses. d_yearly may be NULL; every call on one record passes it or none does. */
+int eg_eval_accumulate_device(eg_ctx* ctx, const eg_result* d_results, const eg_traj* d_traj, const eg_yearly* d_yearly,
+                              uint32_t n, uint64_t first_global_episode, eg_eval_stats* d_acc);
+/* Host only, needs no device: dst <- dst followed by src (the shards of an evaluation in episode order). The same merge as
+ * the device's, so the bits agree. EG_ERR_INVALID when both are non-empty and only one has the per-year part. */
+int eg_eval_stats_merge(eg_eval_stats* dst, const eg_eval_stats* src);
+/* The record as JSON (DESIGN.md §4.6): moments as mean / std / min / max, score quantiles from the histogram, per-year
+ * moments and probabilities, action counts by name. Host only. */
+int eg_eval_stats_write_json(const eg_eval_stats* s, const char* path);
+
 /* ---- CSV export of the best run (SURVEY.md §8(f) N2; utils/csv_export.rs:114-432,456-530 and the call site
  * core/multi_simulation.rs:852-925). The best strategy stored in `w` is replayed on the GPU (eg_replay_batch) and written as
  *   <output_dir>/<%Y%m%d_%H%M%S>/simulation_summary.csv     final metrics, actions taken with estimated costs, yearly summary
