@@ -2,6 +2,7 @@
 // There is no CPU fallback: every compute entry point needs a CUDA device and fails with
 // EG_ERR_NO_DEVICE / EG_ERR_CUDA otherwise.
 #include <cuda_runtime.h>
+#include <algorithm>
 #include <cmath>
 #include <cstring>
 #include <memory>
@@ -15,6 +16,7 @@
 #include "site_tables.cuh"
 #include "stats.cuh"
 #include "suitability.cuh"
+#include "traj_rows.hpp"
 #include "update.cuh"
 #include "weights.hpp"
 
@@ -506,6 +508,7 @@ int eg_update_pack_best_device(eg_ctx* c, const eg_result* d_results, const eg_t
                                const unsigned long long* d_best_index, uint64_t first_global_episode, void* d_record) {
   if (!c || !d_results || !d_trajs || !d_best_score || !d_best_index || !d_record)
     return eg_fail(EG_ERR_INVALID, "eg_update_pack_best_device: NULL argument");
+  if ((uintptr_t)d_record % 8) return eg_fail(EG_ERR_INVALID, "eg_update_pack_best_device: d_record is not 8-byte aligned");
   EG_CUDA(use_device(c));
   EG_CUDA(eg_launch_pack_best(d_results, d_trajs, n, d_best_score, d_best_index, first_global_episode, d_record, c->stream));
   c->launches++;
@@ -708,15 +711,14 @@ int eg_export_best_run_csv(eg_ctx* c, const eg_weights* w, const eg_run_cfg* cfg
   // the best run as a record: best_actions[y] = deficit actions followed by the additional actions (Appendix C of SURVEY.md)
   eg_traj traj;
   std::memset(&traj, 0, sizeof(traj));
-  int row[EG_NY + 1];  // first slot of each year's row in the record
-  row[0] = 0;
+  EgTrajRow r{};
   for (int y = 0; y < EG_NY; y++) {
-    const size_t n = std::min<size_t>(w->best_actions[y].size(), (size_t)(EG_TRAJ_CAPACITY - row[y]));
-    const size_t nd = std::min<size_t>(w->best_deficit_actions[y].size(), n);
-    traj.n_deficit[y] = (uint16_t)nd;
-    traj.n_additional[y] = (uint16_t)(n - nd);
-    for (size_t i = 0; i < n; i++) traj.actions[row[y] + i] = w->best_actions[y][i];
-    row[y + 1] = row[y] + (int)n;
+    const std::vector<uint8_t>& run = w->best_actions[y];
+    const int nd = (int)std::min(w->best_deficit_actions[y].size(), run.size());
+    r = eg_traj_row_at(r.row + r.nd + r.na, nd, (int)run.size() - nd);  // the lists are cut where the record is full
+    traj.n_deficit[y] = (uint16_t)r.nd;
+    traj.n_additional[y] = (uint16_t)r.na;
+    std::copy(run.begin(), run.begin() + r.nd + r.na, traj.actions + r.row);
   }
   eg_result res;
   eg_yearly yearly;
@@ -724,7 +726,7 @@ int eg_export_best_run_csv(eg_ctx* c, const eg_weights* w, const eg_run_cfg* cfg
   rcfg.replay_best = 0;
   eg_sites sites;
   if ((rc = eg_replay_batch(c, &rcfg, &traj, 1, &res, &sites, &yearly))) return rc;
-  return eg_write_best_run_csv(output_dir, w, c->hmap, c->htab, traj, row, res, yearly, sites, written_dir);
+  return eg_write_best_run_csv(output_dir, w, c->hmap, c->htab, traj, res, yearly, sites, written_dir);
 }
 
 int eg_location_analysis(eg_ctx* c, int use_loaded_map, int32_t half_steps, double step, double* scores_out,

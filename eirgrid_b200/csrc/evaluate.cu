@@ -11,7 +11,7 @@
 #include "evaluate.cuh"
 #include <cstring>
 #include "common.hpp"
-#include "traj_items.cuh"
+#include "traj_rows.hpp"
 
 namespace {
 

@@ -9,6 +9,7 @@
 #include "eg_math.hpp"
 #include "host_tables.hpp"
 #include "json_min.hpp"
+#include "traj_rows.hpp"
 #include "weights.hpp"
 
 namespace {
@@ -60,7 +61,7 @@ double powi(double a, int b) { double r = 1.0; for (;;) { if (b & 1) r *= a; b /
 }  // namespace
 
 int eg_write_best_run_csv(const char* output_dir, const eg_weights* w, const EgHostMap& hmap, const EgHostTables& htab, const eg_traj& traj,
-                          const int* row, const eg_result& res, const eg_yearly& yearly, const eg_sites& sites, char* written_dir) {
+                          const eg_result& res, const eg_yearly& yearly, const eg_sites& sites, char* written_dir) {
   char ts[32];
   const std::time_t t = std::time(nullptr);
   std::tm tmv;
@@ -79,10 +80,12 @@ int eg_write_best_run_csv(const char* output_dir, const eg_weights* w, const EgH
     std::fprintf(f, "Total Cost (\xE2\x82\xAC),%s\n", fixed(res.total_cost, 2).c_str());
     std::fprintf(f, "Power Reliability (%%),%s\n\n", fixed(res.power_reliability * 100.0, 2).c_str());
     std::fprintf(f, "Actions Taken\nYear,Action Type,Generator Type,Generator ID,Operation %%,Offset Type,Estimated Cost (\xE2\x82\xAC)\n");
+    EgTrajRow yr{};
     for (int y = 0; y < EG_NY; y++) {
+      yr = eg_traj_next_row(traj, y, yr);
       // SimulationResult.actions holds the additional actions only (simulation.rs:193, iteration.rs:90)
-      for (int i = traj.n_deficit[y]; i < traj.n_deficit[y] + traj.n_additional[y]; i++) {
-        const int a = traj.actions[row[y] + i];
+      for (int i = yr.nd; i < yr.nd + yr.na; i++) {
+        const int a = traj.actions[yr.row + i];
         const int year = EG_BASE_YEAR + y;
         if (a < 45) {
           const int tp = a / 3, m = a % 3;
@@ -164,10 +167,12 @@ int eg_write_best_run_csv(const char* output_dir, const eg_weights* w, const EgH
     for (size_t g = 0; g < m.ex.size(); g++)  // "Existing_{type}_{n}" (generators_loader.rs:190): the third id field is the row number
       plants.push_back({std::string("Existing_") + kGenNames[m.etype[g]] + "_" + std::to_string(g), m.etype[g],
                         g < htab.ex_online_year.size() && htab.ex_online_year[g] ? htab.ex_online_year[g] : 1 << 30, (int)g, m.ex[g], m.ey[g]});
-    for (int y = 0; y < EG_NY; y++)
-      for (int i = 0; i < traj.n_deficit[y] + traj.n_additional[y]; i++) {
-        const int a = traj.actions[row[y] + i];
-        if (a >= 45 || sites.site[row[y] + i] == EG_SITE_NONE) continue;
+    EgTrajRow yr{};
+    for (int y = 0; y < EG_NY; y++) {
+      yr = eg_traj_next_row(traj, y, yr);
+      for (int i = 0; i < yr.nd + yr.na; i++) {
+        const int a = traj.actions[yr.row + i];
+        if (a >= 45 || sites.site[yr.row + i] == EG_SITE_NONE) continue;
         const int year = EG_BASE_YEAR + y;
         Plant p{std::string("Gen_") + kGenNames[a / 3] + "_" + std::to_string(year) + "_" + std::to_string(plants.size()), a / 3, year, year, 0, 0};
         uint32_t h = 0;
@@ -176,6 +181,7 @@ int eg_write_best_run_csv(const char* output_dir, const eg_weights* w, const EgH
         p.y = 5000.0 + (double)((h / 100) % 100) / 100.0 * (50000.0 - 10000.0);
         plants.push_back(p);
       }
+    }
     for (int y = 0; y < EG_NY; y++) {
       const int year = EG_BASE_YEAR + y;
       for (const Plant& p : plants) {
@@ -210,9 +216,11 @@ int eg_write_best_run_csv(const char* output_dir, const eg_weights* w, const EgH
     static const double kOffOpTrend[EG_N_OFFSET_TYPES] = {1.0, 1.01, 0.97, 1.02};
     struct Offset { std::string id; int type, year, mult; double x, y; };
     std::vector<Offset> offs;
-    for (int y = 0; y < EG_NY; y++)
-      for (int i = traj.n_deficit[y]; i < traj.n_deficit[y] + traj.n_additional[y]; i++) {
-        const int a = traj.actions[row[y] + i];
+    EgTrajRow yr{};
+    for (int y = 0; y < EG_NY; y++) {
+      yr = eg_traj_next_row(traj, y, yr);
+      for (int i = yr.nd; i < yr.nd + yr.na; i++) {
+        const int a = traj.actions[yr.row + i];
         if (a < 45 || a >= 57) continue;
         const int o = (a - 45) / 3, year = EG_BASE_YEAR + y;
         Offset r{std::string("Offset_") + kOffsetNames[o] + "_" + std::to_string(year) + "_" + std::to_string(offs.size()), o, year, (a - 45) % 3, 0, 0};
@@ -220,6 +228,7 @@ int eg_write_best_run_csv(const char* output_dir, const eg_weights* w, const EgH
         r.y = csv_uniform((uint32_t)offs.size(), 1) * 50000.0;
         offs.push_back(r);
       }
+    }
     for (int y = 0; y < EG_NY; y++) {
       const int year = EG_BASE_YEAR + y;
       for (const Offset& r : offs) {

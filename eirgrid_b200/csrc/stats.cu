@@ -11,9 +11,10 @@
 //             [183,198) occurrences of deficit key k in current_deficit_actions
 // Integer sums make the result independent of the reduction order and of the number of GPUs.
 #include "stats.cuh"
-#include "traj_items.cuh"
+#include "traj_rows.hpp"
 #include "update_rule.hpp"
 #include <algorithm>
+#include <cstddef>
 
 namespace {
 
@@ -115,40 +116,40 @@ __global__ void __launch_bounds__(256) eg_stats_argbest_kernel(const EgStatsPara
   if (score == *p.best_score) atomicMin(p.best_index, (unsigned long long)ep);
 }
 
-__global__ void __launch_bounds__(320) eg_stats_pack_best_kernel(const eg_result* results, const eg_traj* trajs, uint32_t n, const double* best_score,
-                                                                 const unsigned long long* best_index, unsigned long long first_global, uint32_t* record) {
-  // 16 + 64 + 1088 bytes = 292 words, one per thread
+// Word w of the winner record (EgBestRecord) of the shard's best episode. An index past the shard (none was found) is clamped
+// to its last episode; an empty shard reads element 0 of its buffers.
+__device__ __forceinline__ long long best_record_word(const eg_result* results, const eg_traj* trajs, uint32_t n, const double* best_score,
+                                                      const unsigned long long* best_index, unsigned long long first_global, int w) {
+  constexpr int kScore = offsetof(EgBestRecord, score) / 8, kEpisode = offsetof(EgBestRecord, episode) / 8;
+  constexpr int kResult = offsetof(EgBestRecord, result) / 8, kTraj = offsetof(EgBestRecord, traj) / 8;
+  static_assert(kScore == 0 && kEpisode == 1 && kResult == 2 && kTraj > kResult, "fields in declaration order, 8-byte aligned");
   const unsigned long long raw = *best_index;
   const uint32_t idx = raw < n ? (uint32_t)raw : (n ? n - 1 : 0);
+  if (w == kScore) return __double_as_longlong(*best_score);
+  if (w == kEpisode) return (long long)(first_global + idx);
+  if (w < kTraj) return ((const long long*)(results + idx))[w - kResult];
+  return ((const long long*)(trajs + idx))[w - kTraj];
+}
+
+constexpr int kRecordWords = (int)(sizeof(EgBestRecord) / 8);
+constexpr int kPackThreads = (kRecordWords + 31) / 32 * 32;  // one word per thread
+
+__global__ void __launch_bounds__(kPackThreads) eg_stats_pack_best_kernel(const eg_result* results, const eg_traj* trajs, uint32_t n, const double* best_score,
+                                                                          const unsigned long long* best_index, unsigned long long first_global, long long* record) {
   const int w = threadIdx.x;
-  constexpr int kRes = (int)sizeof(eg_result) / 4, kTraj = (int)sizeof(eg_traj) / 4;
-  if (w < 2) record[w] = ((const uint32_t*)best_score)[w];
-  else if (w < 4) { const unsigned long long g = first_global + idx; record[w] = (uint32_t)(g >> (32 * (w - 2))); }
-  else if (w < 4 + kRes) record[w] = ((const uint32_t*)(results + idx))[w - 4];
-  else if (w < 4 + kRes + kTraj) record[w] = ((const uint32_t*)(trajs + idx))[w - 4 - kRes];
+  if (w < kRecordWords) record[w] = best_record_word(results, trajs, n, best_score, best_index, first_global, w);
 }
 
 // block b of rank r: r's buffer -> slot r of peer b's gather buffer (half `epoch & 1`), then flag r on peer b, then wait for
 // flag b on r. The two halves alternate: a rank cannot start epoch e + 2 before every peer has started e + 1, i.e. has
 // finished reading e (stream order on the peer), so a half is never overwritten while it is read.
 __global__ void __launch_bounds__(256) eg_pack_exchange_kernel(const EgExchangeParams p) {
-  constexpr int kRec = (int)(EG_BEST_RECORD_BYTES / 8), kWords = EG_STATS_WORDS + kRec;
-  constexpr int kRes = (int)sizeof(eg_result) / 8;
+  constexpr int kWords = EG_STATS_WORDS + kRecordWords;
   const uint32_t peer = blockIdx.x;
-  const unsigned long long raw = *p.best_index;
-  const uint32_t idx = raw < p.n ? (uint32_t)raw : (p.n ? p.n - 1 : 0);
   long long* dst = (long long*)p.peer_buf[peer] + ((size_t)(p.epoch & 1u) * p.world + p.rank) * kWords;
-  const long long* res = (const long long*)(p.results + idx);
-  const long long* trj = (const long long*)(p.trajs + idx);
-  for (int i = threadIdx.x; i < kWords; i += blockDim.x) {
-    long long v;
-    if (i < EG_STATS_WORDS) v = p.stats[i];
-    else {
-      const int w = i - EG_STATS_WORDS;  // [score f64 | global id i64 | eg_result | eg_traj]
-      v = w == 0 ? __double_as_longlong(*p.best_score) : w == 1 ? (long long)(p.first_global + idx) : w < 2 + kRes ? res[w - 2] : trj[w - 2 - kRes];
-    }
-    dst[i] = v;
-  }
+  for (int i = threadIdx.x; i < kWords; i += blockDim.x)
+    dst[i] = i < EG_STATS_WORDS ? p.stats[i]
+                                : best_record_word(p.results, p.trajs, p.n, p.best_score, p.best_index, p.first_global, i - EG_STATS_WORDS);
   __threadfence_system();
   __syncthreads();
   if (threadIdx.x == 0) {
@@ -168,7 +169,6 @@ __global__ void __launch_bounds__(256) eg_pack_exchange_kernel(const EgExchangeP
 }  // namespace
 
 cudaError_t eg_launch_pack_exchange(const EgExchangeParams& p, cudaStream_t stream) {
-  static_assert(EG_BEST_RECORD_BYTES % 8 == 0 && sizeof(eg_result) % 8 == 0 && sizeof(eg_traj) % 8 == 0, "the record is copied in 64-bit words");
   if (p.world == 0 || p.world > EG_MAX_PEERS || p.rank >= p.world) return cudaErrorInvalidValue;
   eg_pack_exchange_kernel<<<p.world, 256, 0, stream>>>(p);
   return cudaGetLastError();
@@ -176,8 +176,7 @@ cudaError_t eg_launch_pack_exchange(const EgExchangeParams& p, cudaStream_t stre
 
 cudaError_t eg_launch_pack_best(const eg_result* results, const eg_traj* trajs, uint32_t n, const double* best_score,
                                 const unsigned long long* best_index, unsigned long long first_global, void* record, cudaStream_t stream) {
-  static_assert(sizeof(eg_result) % 4 == 0 && sizeof(eg_traj) % 4 == 0, "record is copied in 32-bit words");
-  eg_stats_pack_best_kernel<<<1, 320, 0, stream>>>(results, trajs, n, best_score, best_index, first_global, (uint32_t*)record);
+  eg_stats_pack_best_kernel<<<1, kPackThreads, 0, stream>>>(results, trajs, n, best_score, best_index, first_global, (long long*)record);
   return cudaGetLastError();
 }
 

@@ -16,7 +16,20 @@ struct EgStatsParams {
   double ln100;
 };
 
-// 1 launch: [score | global id | eg_result | eg_traj] of the shard's best episode as one flat record
+// The winner record of a shard: its best score and the episode that holds it. One flat record of EG_BEST_RECORD_BYTES
+// without padding, so that ranks can exchange it as raw bytes (int64 words).
+struct EgBestRecord {
+  double score;
+  int64_t episode;  // global id
+  eg_result result;
+  eg_traj traj;
+};
+static_assert(sizeof(EgBestRecord) == EG_BEST_RECORD_BYTES &&
+                  sizeof(EgBestRecord) == sizeof(double) + sizeof(int64_t) + sizeof(eg_result) + sizeof(eg_traj),
+              "the winner record is EG_BEST_RECORD_BYTES without padding");
+static_assert(sizeof(EgBestRecord) % 8 == 0 && alignof(EgBestRecord) == 8, "the winner record is packed and exchanged in 64-bit words");
+
+// 1 launch: the winner record (EgBestRecord) of the shard's best episode; `record` is 8-byte aligned
 cudaError_t eg_launch_pack_best(const eg_result* results, const eg_traj* trajs, uint32_t n, const double* best_score,
                                 const unsigned long long* best_index, unsigned long long first_global, void* record, cudaStream_t stream);
 

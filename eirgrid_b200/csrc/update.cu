@@ -21,6 +21,7 @@
 //     factors of the randomisation branch (one Philox draw per table entry and episode) are produced by a parallel kernel
 //     beforehand and stream in the same way.
 #include "update.cuh"
+#include "traj_rows.hpp"
 #include "update_rule.hpp"
 #include <cstddef>
 
@@ -203,52 +204,6 @@ __global__ void __launch_bounds__(128) upd_ctl_kernel(uint32_t n, EgUpdBuffers b
   if ((threadIdx.x & 31) == 0 && m) atomicAdd(&b.state->n_applied, (uint32_t)__popc(m));
 }
 
-// ---- the recorded lists of one year as the shared weights see them after transfer_recorded_actions_from --------------
-// run list = deficit actions then additional actions; replay iterations record every additional action twice and the
-// first four deficit actions twice in the deficit list (quirk Q10; weights.cpp Recorded::from_traj). Codes outside the
-// key set are skipped.
-template <typename F>
-__device__ __forceinline__ void for_each_run(const uint8_t* a, int nd, int na, bool replay, F f) {
-  for (int i = 0; i < nd; i++) {
-    const int c = a[i];
-    if (c < EG_N_ACTIONS) f(c);
-  }
-  for (int i = nd; i < nd + na; i++) {
-    const int c = a[i];
-    if (c < EG_N_ACTIONS) {
-      f(c);
-      if (replay) f(c);
-    }
-  }
-}
-template <typename F>
-__device__ __forceinline__ void for_each_deficit(const uint8_t* a, int nd, bool replay, F f) {
-  for (int i = 0; i < nd; i++) {
-    const int c = a[i];
-    if (c < EG_N_ACTIONS) {
-      f(c);
-      if (replay && i < 4) f(c);
-    }
-  }
-}
-
-// lane y: first slot and clamped lengths of year y's row in a record (rows are stored back to back)
-__device__ __forceinline__ void year_row(const eg_traj* t, int lane, int* row, int* nd, int* na) {
-  int d = 0, a = 0;
-  if (lane < EG_NY) { d = t->n_deficit[lane]; a = t->n_additional[lane]; }
-  int end = d + a;
-#pragma unroll
-  for (int o = 1; o < 32; o <<= 1) {
-    const int v = __shfl_up_sync(0xFFFFFFFFu, end, o);
-    if (lane >= o) end += v;
-  }
-  int r = end - (d + a);
-  if (r > EG_TRAJ_CAPACITY) r = EG_TRAJ_CAPACITY;
-  d = min(d, EG_TRAJ_CAPACITY - r);
-  a = min(a, EG_TRAJ_CAPACITY - r - d);
-  *row = r; *nd = d; *na = a;
-}
-
 // ---- 4. best-strategy lists of the improving episodes (one warp per episode, lane = year) ------------------------------
 __global__ void __launch_bounds__(256) upd_expand_kernel(const eg_traj* trajs, uint32_t n, uint32_t replay, EgUpdBuffers b) {
   const uint32_t e = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
@@ -256,13 +211,12 @@ __global__ void __launch_bounds__(256) upd_expand_kernel(const eg_traj* trajs, u
   if (e >= n || !b.pre[e].improved) return;
   const eg_traj* t = trajs + e;
   EgUpdSlot* s = b.slots + e + 1;
-  int row, nd, na;
-  year_row(t, lane, &row, &nd, &na);
-  const uint8_t* a = t->actions + row;
+  const EgTrajRow r = eg_warp_traj_row(t, lane);
+  const uint8_t* a = t->actions + r.row;
   int len_run = 0, len_def = 0;
   unsigned long long mall = 0ull, mdef = 0ull;
-  for_each_run(a, nd, na, replay != 0, [&](int c) { len_run++; mall |= 1ull << c; });
-  for_each_deficit(a, nd, replay != 0, [&](int c) { len_def++; mdef |= 1ull << c; });
+  eg_for_each_run(a, r.nd, r.na, replay != 0, [&](int c) { len_run++; mall |= 1ull << c; });
+  eg_for_each_deficit(a, r.nd, replay != 0, [&](int c) { len_def++; mdef |= 1ull << c; });
   int end = len_run + len_def;
 #pragma unroll
   for (int o = 1; o < 32; o <<= 1) {
@@ -278,8 +232,8 @@ __global__ void __launch_bounds__(256) upd_expand_kernel(const eg_traj* trajs, u
   s->mask_def[lane] = mdef;
   uint8_t* out = s->cat + off;
   int i = 0;
-  for_each_run(a, nd, na, replay != 0, [&](int c) { out[i++] = (uint8_t)c; });
-  for_each_deficit(a, nd, replay != 0, [&](int c) { out[i++] = (uint8_t)c; });
+  eg_for_each_run(a, r.nd, r.na, replay != 0, [&](int c) { out[i++] = (uint8_t)c; });
+  eg_for_each_deficit(a, r.nd, replay != 0, [&](int c) { out[i++] = (uint8_t)c; });
 }
 
 // Number of penalty / mild-penalty multiplications entry `key` of year `y` receives from one episode (learning.rs:228-262),
@@ -293,14 +247,14 @@ __device__ int count_regular(const uint8_t* a, int nd, int na, bool replay, cons
     if (c == key && (!in_best || (i < LB && B[i] != c))) cnt++;
     i++;
   };
-  for_each_run(a, nd, na, replay, visit);
-  for_each_deficit(a, nd, replay, visit);
+  eg_for_each_run(a, nd, na, replay, visit);
+  eg_for_each_deficit(a, nd, replay, visit);
   return cnt;
 }
 __device__ int count_deficit(const uint8_t* a, int nd, bool replay, const EgUpdSlot* s, int y, int dkey) {
   const unsigned long long mdef = s->mask_def[y];
   int cnt = 0;
-  for_each_deficit(a, nd, replay, [&](int c) {
+  eg_for_each_deficit(a, nd, replay, [&](int c) {
     if (!((mdef >> c) & 1ull) && egrule::deficit_key_of_action(c) == dkey) cnt++;
   });
   return cnt;
@@ -315,14 +269,13 @@ __global__ void __launch_bounds__(kPrepWarps * 32) upd_prep_kernel(const eg_traj
   if (e >= n) return;
   const uint32_t flags = b.ctl[e].flags;
   const eg_traj* t = trajs + e;
-  int row, nd, na;
-  year_row(t, lane, &row, &nd, &na);
+  const EgTrajRow yr = eg_warp_traj_row(t, lane);
   if (lane >= EG_NY) return;
   uint8_t* r = rows[w][lane];
   uint4* r4 = (uint4*)r;
 #pragma unroll
   for (int q = 0; q < EG_UPD_ROW / 16; q++) r4[q] = make_uint4(0u, 0u, 0u, 0u);
-  const uint8_t* a = t->actions + row;
+  const uint8_t* a = t->actions + yr.row;
   const EgUpdSlot* s = b.slots + (b.pre[e].improver + 1);
   const bool rp = replay != 0;
   auto bump = [&](int idx) {
@@ -339,12 +292,12 @@ __global__ void __launch_bounds__(kPrepWarps * 32) upd_prep_kernel(const eg_traj
       else if (i < LB && B[i] != c) bump(c);              // part of it, at another position: mild penalty
       i++;
     };
-    for_each_run(a, nd, na, rp, visit);
-    for_each_deficit(a, nd, rp, visit);
+    eg_for_each_run(a, yr.nd, yr.na, rp, visit);
+    eg_for_each_deficit(a, yr.nd, rp, visit);
   }
   if (flags & EG_UPD_D_APPLIED) {
     const unsigned long long mdef = s->mask_def[lane];
-    for_each_deficit(a, nd, rp, [&](int c) {
+    eg_for_each_deficit(a, yr.nd, rp, [&](int c) {
       if (!((mdef >> c) & 1ull)) {
         const int k = egrule::deficit_key_of_action(c);
         if (k >= 0) bump(EG_N_ACTIONS + k);
@@ -418,13 +371,10 @@ static_assert(offsetof(WalkSmem, cnt) % 16 == 0 && offsetof(WalkSmem, factors) %
 // rare paths of the walk, kept out of line so that the episode loop stays short
 template <bool DEFICIT>
 __device__ __noinline__ int walk_recount(const eg_traj* t, int y, int key, bool rp, const EgUpdSlot* cur) {
-  int row = 0, nd = 0, na = 0;
-  for (int yy = 0; yy <= y; yy++) {
-    row = min(row + nd + na, EG_TRAJ_CAPACITY);
-    nd = min((int)t->n_deficit[yy], EG_TRAJ_CAPACITY - row);
-    na = min((int)t->n_additional[yy], EG_TRAJ_CAPACITY - row - nd);
-  }
-  return DEFICIT ? count_deficit(t->actions + row, nd, rp, cur, y, key) : count_regular(t->actions + row, nd, na, rp, cur, y, key);
+  EgTrajRow r{};
+  for (int yy = 0; yy <= y; yy++) r = eg_traj_next_row(*t, yy, r);
+  const uint8_t* a = t->actions + r.row;
+  return DEFICIT ? count_deficit(a, r.nd, rp, cur, y, key) : count_regular(a, r.nd, r.na, rp, cur, y, key);
 }
 template <bool DEFICIT>
 __device__ __noinline__ int walk_occurrences(const EgUpdSlot* s, int y, int key) {

@@ -9,6 +9,8 @@
 #include "weights.hpp"
 #include "json_min.hpp"
 #include "common.hpp"
+#include "stats.cuh"
+#include "traj_rows.hpp"
 #include "update_rule.hpp"
 #include "update.cuh"
 #include <algorithm>
@@ -200,27 +202,14 @@ bool read_action_lists(const egjson::Value* v, std::vector<uint8_t>* lists) {
 struct Recorded {
   std::vector<uint8_t> run[EG_NY], deficit[EG_NY];
   void from_traj(const eg_traj& t, bool replay) {
-    int row = 0;  // the year rows follow each other in the record; counts that run past its capacity are cut
+    EgTrajRow r{};
     for (int y = 0; y < EG_NY; y++) {
+      r = eg_traj_next_row(t, y, r);
       run[y].clear();
       deficit[y].clear();
-      const int nd = std::min<int>(t.n_deficit[y], EG_TRAJ_CAPACITY - row);
-      const int na = std::min<int>(t.n_additional[y], EG_TRAJ_CAPACITY - row - nd);
-      const uint8_t* a = t.actions + row;
-      // replay iterations record every sampled action twice (sampling.rs:97-99,262-264 + simulation.rs:197,406-409; quirk Q10)
-      // (codes outside the key set never come from the device; a malformed record must not index the tables with them)
-      for (int i = 0; i < nd; i++) {
-        if (a[i] >= EG_N_ACTIONS) continue;
-        run[y].push_back(a[i]);
-        deficit[y].push_back(a[i]);
-        if (replay && i < 4) deficit[y].push_back(a[i]);
-      }
-      for (int i = nd; i < nd + na; i++) {
-        if (a[i] >= EG_N_ACTIONS) continue;
-        run[y].push_back(a[i]);
-        if (replay) run[y].push_back(a[i]);
-      }
-      row += nd + na;
+      const uint8_t* a = t.actions + r.row;
+      eg_for_each_run(a, r.nd, r.na, replay, [&](int c) { run[y].push_back((uint8_t)c); });
+      eg_for_each_deficit(a, r.nd, replay, [&](int c) { deficit[y].push_back((uint8_t)c); });
     }
   }
 };
@@ -858,26 +847,16 @@ int eg_weights_history_append(const eg_weights* w, uint64_t iteration, const cha
 int eg_update_combine_apply(eg_weights* w, const int64_t* stats_sum, const void* records, uint32_t n_records, uint64_t n_total,
                             uint64_t first_episode, eg_update_stats* stats_out) {
   if (!w || !stats_sum || (!records && n_records)) return eg_fail(EG_ERR_INVALID, "eg_update_combine_apply: NULL argument");
-  const unsigned char* rec = (const unsigned char*)records;
-  const unsigned char* win = nullptr;
-  double win_score = 0.0;
-  int64_t win_id = 0;
+  EgBestRecord win, cand;  // copied out: `records` is a byte buffer with no alignment promised
+  bool found = false;
   for (uint32_t r = 0; r < n_records; r++) {
-    const unsigned char* p = rec + (size_t)r * EG_BEST_RECORD_BYTES;
-    double score;
-    int64_t id;
-    std::memcpy(&score, p, 8);
-    std::memcpy(&id, p + 8, 8);
-    if (!win || score > win_score || (score == win_score && id < win_id)) { win = p; win_score = score; win_id = id; }
+    std::memcpy(&cand, (const unsigned char*)records + (size_t)r * sizeof(EgBestRecord), sizeof(EgBestRecord));
+    if (!found || cand.score > win.score || (cand.score == win.score && cand.episode < win.episode)) { win = cand; found = true; }
   }
-  if (!win) return eg_update_apply_stats(w, stats_sum, n_total, nullptr, nullptr, -1, stats_out);
-  if (n_total > 0 && (win_id < (int64_t)first_episode || (uint64_t)(win_id - (int64_t)first_episode) >= n_total))
+  if (!found) return eg_update_apply_stats(w, stats_sum, n_total, nullptr, nullptr, -1, stats_out);
+  if (n_total > 0 && (win.episode < (int64_t)first_episode || (uint64_t)(win.episode - (int64_t)first_episode) >= n_total))
     return eg_fail(EG_ERR_INVALID, "eg_update_combine_apply: the winner record's episode id lies outside the batch");
-  eg_result res;
-  eg_traj traj;
-  std::memcpy(&res, win + 16, sizeof(res));
-  std::memcpy(&traj, win + 16 + sizeof(res), sizeof(traj));
-  return eg_update_apply_stats(w, stats_sum, n_total, &res, &traj, win_id - (int64_t)first_episode, stats_out);
+  return eg_update_apply_stats(w, stats_sum, n_total, &win.result, &win.traj, win.episode - (int64_t)first_episode, stats_out);
 }
 
 }  // extern "C"

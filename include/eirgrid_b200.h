@@ -298,7 +298,7 @@ int eg_update_stats_device(eg_ctx* ctx, const eg_weights* w, const eg_result* d_
 int eg_update_stats_clear_device(eg_ctx* ctx, int64_t* d_stats);
 /* This rank's candidate for the batch winner as one flat record on the device, ready for the all-gather:
  * [best score f64 | global episode id i64 | eg_result | eg_traj] (EG_BEST_RECORD_BYTES). d_best_score / d_best_index are
- * the outputs of eg_update_stats_device; global id = first_global_episode + index. */
+ * the outputs of eg_update_stats_device; global id = first_global_episode + index. d_record is 8-byte aligned. */
 #define EG_BEST_RECORD_BYTES (16 + sizeof(eg_result) + sizeof(eg_traj))
 int eg_update_pack_best_device(eg_ctx* ctx, const eg_result* d_results, const eg_traj* d_trajs, uint32_t n,
                                const double* d_best_score, const unsigned long long* d_best_index,

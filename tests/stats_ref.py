@@ -43,7 +43,7 @@ def contrast_consts(table, cost_only=False):
 
 def recorded_rows(t):
     """(run, deficit) action lists of each year as the update reads a record: year rows follow each other, and counts that
-    run past the record's capacity are cut (Recorded::from_traj in weights.cpp)."""
+    run past the record's capacity are cut (eg_traj_next_row in csrc/traj_rows.hpp)."""
     rows, row = [], 0
     a = t["actions"]
     for y in range(_abi.N_YEARS):

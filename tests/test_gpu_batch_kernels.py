@@ -229,6 +229,12 @@ def test_pack_best_record(gpu_ctx, trained, scale_batch):
     for recs in ((empty, rec), (rec, empty)):
         st = T.combine_and_apply(w.clone(), s.stats, np.stack(recs), SCALE_N, FIRST_GLOBAL)
         assert st.batch_best_episode == k
+    # the record is written in 64-bit words: a buffer that is not 8-byte aligned is refused without a launch
+    launches = gpu_ctx.kernel_launches()
+    with pytest.raises(_lib.EirgridError) as e:
+        gpu_ctx.update_pack_best_device(s.n, s.d_res, s.d_traj, s.d_bs, s.d_bi, FIRST_GLOBAL, d_rec.data_ptr() + 4)
+    assert e.value.code == -1
+    assert gpu_ctx.kernel_launches() == launches
 
 
 SENTINEL = 0x5A5A5A5A5A5A5A5A
