@@ -23,7 +23,7 @@ EXPORTS = [
     "eg_location_analysis_year", "eg_microbench_fp64", "eg_export_best_run_csv", "eg_weights_history_append", "eg_train_batch_begin", "eg_train_batch_end", "eg_train_batch_results", "eg_update_combine_apply",
     "eg_update_device", "eg_train_batch_inorder", "eg_rule_math",
     "eg_location_analysis_sites", "eg_location_analysis_sites_device", "eg_location_analysis_write",
-    "eg_update_pack_exchange_device", "eg_evaluate", "eg_eval_accumulate_device", "eg_eval_stats_merge", "eg_eval_stats_write_json",
+    "eg_evaluate", "eg_eval_accumulate_device", "eg_eval_stats_merge", "eg_eval_stats_write_json",
 ]
 
 
@@ -80,7 +80,6 @@ def lib():
     L.eg_train_batch_inorder.argtypes = [vp, vp, C.POINTER(_abi.RunCfg), u64, u64, u32, u64, C.POINTER(_abi.UpdateStats)]
     L.eg_update_stats_device.argtypes = [vp, vp, vp, vp, u32, vp, vp, vp]
     L.eg_update_stats_clear_device.argtypes = [vp, vp]
-    L.eg_update_pack_exchange_device.argtypes = [vp, vp, vp, u32, vp, vp, vp, u64, vp, vp, u32, u32, u32, vp]
     L.eg_update_pack_best_device.argtypes = [vp, vp, vp, u32, vp, vp, u64, vp]
     L.eg_weights_history_append.argtypes = [vp, u64, C.c_char_p]
     L.eg_location_analysis_sites.argtypes = [vp, C.c_int, u32, C.c_double, u32, u32, u32, u32, vp]
@@ -332,16 +331,6 @@ class Context:
     def update_pack_best_device(self, n, d_results, d_traj, d_best_score, d_best_index, first_global_episode, d_record):
         check(self.L.eg_update_pack_best_device(self.h, _dev_ptr(d_results), _dev_ptr(d_traj), n, _dev_ptr(d_best_score),
                                                 _dev_ptr(d_best_index), first_global_episode, _dev_ptr(d_record)))
-
-    def update_pack_exchange_device(self, n, d_results, d_traj, d_stats, d_best_score, d_best_index, first_global_episode,
-                                    peer_buffers, peer_flags, rank, epoch, d_error):
-        """pack + all-gather over NVLink peer memory in one kernel (peer_buffers / peer_flags: lists of device addresses)"""
-        world = len(peer_buffers)
-        pb = (C.c_uint64 * world)(*[int(x) for x in peer_buffers])
-        pf = (C.c_uint64 * world)(*[int(x) for x in peer_flags])
-        check(self.L.eg_update_pack_exchange_device(self.h, _dev_ptr(d_results), _dev_ptr(d_traj), n, _dev_ptr(d_stats),
-                                                    _dev_ptr(d_best_score), _dev_ptr(d_best_index), int(first_global_episode),
-                                                    pb, pf, world, int(rank), int(epoch), _dev_ptr(d_error)))
 
     def export_best_run_csv(self, weights, output_dir, cfg=None):
         """CsvExporter::export_simulation_results for the best strategy in `weights`; returns the directory written."""

@@ -515,23 +515,6 @@ int eg_update_pack_best_device(eg_ctx* c, const eg_result* d_results, const eg_t
   return EG_OK;
 }
 
-int eg_update_pack_exchange_device(eg_ctx* c, const eg_result* d_results, const eg_traj* d_trajs, uint32_t n, const int64_t* d_stats,
-                                   const double* d_best_score, const unsigned long long* d_best_index, uint64_t first_global_episode,
-                                   const uint64_t* peer_buffers, const uint64_t* peer_flags, uint32_t world, uint32_t rank, uint32_t epoch,
-                                   uint32_t* d_error) {
-  if (!c || !d_results || !d_trajs || !d_stats || !d_best_score || !d_best_index || !peer_buffers || !peer_flags || !d_error)
-    return eg_fail(EG_ERR_INVALID, "eg_update_pack_exchange_device: NULL argument");
-  if (world == 0 || world > EG_MAX_PEERS || rank >= world) return eg_fail(EG_ERR_INVALID, "eg_update_pack_exchange_device: bad world / rank");
-  EG_CUDA(use_device(c));
-  EgExchangeParams p{};
-  p.results = d_results; p.trajs = d_trajs; p.n = n; p.best_score = d_best_score; p.best_index = d_best_index;
-  p.first_global = first_global_episode; p.stats = d_stats; p.world = world; p.rank = rank; p.epoch = epoch; p.error = d_error;
-  for (uint32_t r = 0; r < world; r++) { p.peer_buf[r] = peer_buffers[r]; p.peer_flag[r] = peer_flags[r]; }
-  EG_CUDA(eg_launch_pack_exchange(p, c->stream));
-  c->launches++;
-  return EG_OK;
-}
-
 int eg_train_batch_begin(eg_ctx* c, const eg_weights* w, const eg_run_cfg* cfg, uint64_t seed, uint64_t first_episode, uint32_t n) {
   int rc = check_cfg(c, cfg);
   if (rc) return rc;

@@ -3,7 +3,7 @@
 // The reference applies apply_contrast_learning / apply_deficit_contrast_learning (weights/learning.rs:131-373)
 // one episode at a time under a write lock (core/multi_simulation.rs:494-508). For a batch sampled from one frozen
 // snapshot and sharded over GPUs, the per-episode effect on the weight table is summarised here as a small integer
-// table (DESIGN.md §update) that ranks sum with one NCCL allreduce:
+// table (DESIGN.md §update) that ranks all-gather and sum:
 //   header[0] episodes, header[1] episodes whose deterioration passed the contrast threshold, header[2] flagged episodes
 //   per year: [0,61)    sum of ln(penalty_e)      over penalised occurrences of action k   (fixed point, 2^-24)
 //             [61,122)  sum of ln(mild_penalty_e) over mis-positioned occurrences of k      (fixed point)
@@ -116,63 +116,27 @@ __global__ void __launch_bounds__(256) eg_stats_argbest_kernel(const EgStatsPara
   if (score == *p.best_score) atomicMin(p.best_index, (unsigned long long)ep);
 }
 
-// Word w of the winner record (EgBestRecord) of the shard's best episode. An index past the shard (none was found) is clamped
-// to its last episode; an empty shard reads element 0 of its buffers.
-__device__ __forceinline__ long long best_record_word(const eg_result* results, const eg_traj* trajs, uint32_t n, const double* best_score,
-                                                      const unsigned long long* best_index, unsigned long long first_global, int w) {
-  constexpr int kScore = offsetof(EgBestRecord, score) / 8, kEpisode = offsetof(EgBestRecord, episode) / 8;
-  constexpr int kResult = offsetof(EgBestRecord, result) / 8, kTraj = offsetof(EgBestRecord, traj) / 8;
-  static_assert(kScore == 0 && kEpisode == 1 && kResult == 2 && kTraj > kResult, "fields in declaration order, 8-byte aligned");
-  const unsigned long long raw = *best_index;
-  const uint32_t idx = raw < n ? (uint32_t)raw : (n ? n - 1 : 0);
-  if (w == kScore) return __double_as_longlong(*best_score);
-  if (w == kEpisode) return (long long)(first_global + idx);
-  if (w < kTraj) return ((const long long*)(results + idx))[w - kResult];
-  return ((const long long*)(trajs + idx))[w - kTraj];
-}
-
 constexpr int kRecordWords = (int)(sizeof(EgBestRecord) / 8);
 constexpr int kPackThreads = (kRecordWords + 31) / 32 * 32;  // one word per thread
 
+// The winner record (EgBestRecord) of the shard's best episode, word w by thread w. An index past the shard (none was found)
+// is clamped to its last episode; an empty shard reads element 0 of its buffers.
 __global__ void __launch_bounds__(kPackThreads) eg_stats_pack_best_kernel(const eg_result* results, const eg_traj* trajs, uint32_t n, const double* best_score,
                                                                           const unsigned long long* best_index, unsigned long long first_global, long long* record) {
+  constexpr int kScore = offsetof(EgBestRecord, score) / 8, kEpisode = offsetof(EgBestRecord, episode) / 8;
+  constexpr int kResult = offsetof(EgBestRecord, result) / 8, kTraj = offsetof(EgBestRecord, traj) / 8;
+  static_assert(kScore == 0 && kEpisode == 1 && kResult == 2 && kTraj > kResult, "fields in declaration order, 8-byte aligned");
   const int w = threadIdx.x;
-  if (w < kRecordWords) record[w] = best_record_word(results, trajs, n, best_score, best_index, first_global, w);
-}
-
-// block b of rank r: r's buffer -> slot r of peer b's gather buffer (half `epoch & 1`), then flag r on peer b, then wait for
-// flag b on r. The two halves alternate: a rank cannot start epoch e + 2 before every peer has started e + 1, i.e. has
-// finished reading e (stream order on the peer), so a half is never overwritten while it is read.
-__global__ void __launch_bounds__(256) eg_pack_exchange_kernel(const EgExchangeParams p) {
-  constexpr int kWords = EG_STATS_WORDS + kRecordWords;
-  const uint32_t peer = blockIdx.x;
-  long long* dst = (long long*)p.peer_buf[peer] + ((size_t)(p.epoch & 1u) * p.world + p.rank) * kWords;
-  for (int i = threadIdx.x; i < kWords; i += blockDim.x)
-    dst[i] = i < EG_STATS_WORDS ? p.stats[i]
-                                : best_record_word(p.results, p.trajs, p.n, p.best_score, p.best_index, p.first_global, i - EG_STATS_WORDS);
-  __threadfence_system();
-  __syncthreads();
-  if (threadIdx.x == 0) {
-    uint32_t* remote = (uint32_t*)p.peer_flag[peer] + p.rank;
-    asm volatile("st.release.sys.global.u32 [%0], %1;" ::"l"(remote), "r"(p.epoch) : "memory");
-    const uint32_t* mine = (const uint32_t*)p.peer_flag[p.rank] + peer;
-    const long long t0 = clock64();
-    for (;;) {
-      uint32_t v;
-      asm volatile("ld.acquire.sys.global.u32 %0, [%1];" : "=r"(v) : "l"(mine) : "memory");
-      if ((int32_t)(v - p.epoch) >= 0) break;
-      if (clock64() - t0 > 4000000000ll) { *p.error = 1u; break; }  // ~2 s: a peer that never arrives must not hang the GPU
-    }
-  }
+  if (w >= kRecordWords) return;
+  const unsigned long long raw = *best_index;
+  const uint32_t idx = raw < n ? (uint32_t)raw : (n ? n - 1 : 0);
+  record[w] = w == kScore     ? __double_as_longlong(*best_score)
+              : w == kEpisode ? (long long)(first_global + idx)
+              : w < kTraj     ? ((const long long*)(results + idx))[w - kResult]
+                              : ((const long long*)(trajs + idx))[w - kTraj];
 }
 
 }  // namespace
-
-cudaError_t eg_launch_pack_exchange(const EgExchangeParams& p, cudaStream_t stream) {
-  if (p.world == 0 || p.world > EG_MAX_PEERS || p.rank >= p.world) return cudaErrorInvalidValue;
-  eg_pack_exchange_kernel<<<p.world, 256, 0, stream>>>(p);
-  return cudaGetLastError();
-}
 
 cudaError_t eg_launch_pack_best(const eg_result* results, const eg_traj* trajs, uint32_t n, const double* best_score,
                                 const unsigned long long* best_index, unsigned long long first_global, void* record, cudaStream_t stream) {

@@ -35,22 +35,3 @@ cudaError_t eg_launch_pack_best(const eg_result* results, const eg_traj* trajs, 
 
 // 3 launches: reset of the best slot, accumulation + max score, lowest index holding the max
 cudaError_t eg_launch_stats(const EgStatsParams& p, cudaStream_t stream);
-
-// Exchange step as ONE kernel over NVLink peer memory: every rank writes its [statistics | best-episode record] buffer
-// straight into slot `rank` of every peer's gather buffer (plain stores through the peer mappings of a symmetric allocation),
-// raises a flag on the peer and waits for the peers' flags on itself; when the kernel ends, the rank holds all ranks' buffers.
-#define EG_MAX_PEERS 16
-struct EgExchangeParams {
-  const eg_result* results;
-  const eg_traj* trajs;
-  uint32_t n;
-  const double* best_score;
-  const unsigned long long* best_index;
-  unsigned long long first_global;
-  const int64_t* stats;                          // this rank's statistics table [EG_STATS_WORDS]
-  unsigned long long peer_buf[EG_MAX_PEERS];     // every rank's gather buffer: int64[2][world][EG_STATS_WORDS + record words]
-  unsigned long long peer_flag[EG_MAX_PEERS];    // every rank's flags: uint32[world], flag r = last epoch rank r delivered
-  uint32_t world, rank, epoch;
-  uint32_t* error;                               // set to 1 when a peer's flag did not arrive in time
-};
-cudaError_t eg_launch_pack_exchange(const EgExchangeParams& p, cudaStream_t stream);

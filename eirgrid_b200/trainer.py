@@ -123,49 +123,9 @@ class BatchTrainer:
         self.h_all_pack = torch.zeros(self.world * self.pack_words, dtype=torch.int64).pin_memory()
         self.h2d_bytes_per_step = 0
         self.d2h_bytes_per_step = self.h_all_pack.numel() * 8
-        self._init_peer_exchange()
+        self.exchange_kind = "none" if self.world == 1 else "nccl all-gather"
         self.last_stats = None
         torch.cuda.synchronize(self.device)  # allocations above ran on the default stream
-
-    def _init_peer_exchange(self):
-        """Gather buffers and flags in symmetric memory (every rank's allocation mapped on every GPU over NVLink), so that the
-        exchange step is ONE kernel of this library writing straight into the peers (eg_update_pack_exchange_device) instead
-        of a pack kernel followed by an NCCL all-gather. EIRGRID_EXCHANGE=nccl, or a rendezvous that fails on any rank,
-        keeps the NCCL all-gather."""
-        torch = _torch()
-        self.peer = None
-        self.exchange_kind = "none" if self.world == 1 else "nccl all-gather"
-        if not (self.dist and self.world > 1):
-            return
-        ok, peer = 1, None
-        if os.environ.get("EIRGRID_EXCHANGE", "peer") != "peer":
-            ok = 0
-        else:
-            try:
-                import torch.distributed._symmetric_memory as symm
-                buf = symm.empty(2 * self.world * self.pack_words, dtype=torch.int64, device=self.device)
-                hdl = symm.rendezvous(buf, self.dist.group.WORLD)
-                flags = symm.empty(64, dtype=torch.int32, device=self.device)
-                fhdl = symm.rendezvous(flags, self.dist.group.WORLD)
-                buf.zero_()
-                flags.zero_()
-                peer = dict(buf=buf, hdl=hdl, flags=flags, fhdl=fhdl, buf_ptrs=[int(x) for x in hdl.buffer_ptrs],
-                            flag_ptrs=[int(x) for x in fhdl.buffer_ptrs])
-            except Exception as e:  # noqa: BLE001 - any failure of the private API means: use NCCL
-                import sys
-                print("eirgrid_b200: symmetric memory unavailable (%s: %s); exchange step uses the NCCL all-gather" % (type(e).__name__, e),
-                      file=sys.stderr)
-                ok = 0
-        agree = torch.tensor([ok], dtype=torch.int32, device=self.device)
-        self.dist.all_reduce(agree, op=self.dist.ReduceOp.MIN)  # every rank must take the same path
-        torch.cuda.synchronize(self.device)
-        if int(agree.item()) == 1:
-            self.peer = peer
-            self.epoch = 0
-            self.d_error = torch.zeros(1, dtype=torch.int32, device=self.device)
-            self.exchange_kind = "one kernel over NVLink peer memory (symmetric allocation)"
-            self.dist.barrier()  # the zeroed flags are visible everywhere before the first epoch
-            torch.cuda.synchronize(self.device)
 
     def set_batch(self, total):
         """Split a batch of `total` episodes over the ranks: rank r takes total // world episodes, the first total % world
@@ -194,15 +154,6 @@ class BatchTrainer:
     def exchange(self):
         """The path's only exchange step: one all-gather of every rank's [statistics | best-episode record] buffer,
         queued on the trainer's stream (a device copy when there is one rank)."""
-        if self.peer is not None:
-            # pack + gather in one kernel: this rank's buffer goes straight into every peer's gather buffer over NVLink
-            self.epoch += 1
-            self.ctx.update_pack_exchange_device(self.n, self.d_results, self.d_traj, self.d_stats, self.d_best_score, self.d_best_index,
-                                                 self.next_episode + self.offset, self.peer["buf_ptrs"], self.peer["flag_ptrs"], self.rank,
-                                                 self.epoch, self.d_error)
-            half = (self.epoch & 1) * self.world * self.pack_words
-            self.d_all_pack = self.peer["buf"][half:half + self.world * self.pack_words]
-            return
         self._pack_best()
         with _torch().cuda.stream(self.stream):
             if self.dist and self.world > 1:
@@ -215,9 +166,7 @@ class BatchTrainer:
         self.exchange()
 
     def check_exchange(self):
-        """Raises if a peer failed to deliver its buffer in time (the kernel gives up after ~2 s instead of hanging)."""
-        if self.peer is not None and int(self.d_error.item()) != 0:
-            raise _lib.EirgridError(-3, "exchange step: a peer rank did not deliver its statistics within 2 s")
+        """No-op: NCCL reports a failed all-gather itself. Kept for callers that check after every exchange step."""
 
     def warm_exchange(self):
         """Run the gather / copy part of step() once without applying anything (warm-up)."""
@@ -236,7 +185,6 @@ class BatchTrainer:
         with torch.cuda.stream(self.stream):
             self.h_all_pack.copy_(self.d_all_pack, non_blocking=True)
         self.stream.synchronize()
-        self.check_exchange()
         n_total = self.n_total
         st = sum_and_apply(self.weights, self.h_all_pack.numpy(), n_total, self.next_episode)
         self.next_episode += n_total

@@ -285,10 +285,11 @@ int eg_update_device(eg_ctx* ctx, eg_weights* w, const eg_result* d_results, con
 int eg_train_batch_inorder(eg_ctx* ctx, eg_weights* w, const eg_run_cfg* cfg, uint64_t seed, uint64_t first_episode, uint32_t n,
                            uint64_t rng_seed, eg_update_stats* stats_out);
 
-/* Batch-synchronous update for sharded episodes (DESIGN.md §update): statistics are accumulated on the
- * device by eg_update_stats_device into a table of EG_STATS_WORDS int64 words that the caller sums
- * across ranks (NCCL allreduce SUM), then eg_update_apply_stats applies the identical update on every
- * rank. `best_*` of the batch winner travel with the MAX-loc step done by the caller. */
+/* Batch-synchronous update for sharded episodes (DESIGN.md §update): eg_update_stats_device accumulates a rank's
+ * statistics on the device into a table of EG_STATS_WORDS int64 words and finds the rank's best episode, and
+ * eg_update_pack_best_device packs that episode as the rank's winner record. The ranks all-gather
+ * [statistics table | winner record]; every rank then calls eg_update_combine_apply, which sums the tables, picks the batch
+ * winner among the records and applies the identical update (eg_update_apply_stats). */
 #define EG_STATS_WORDS (8 + EG_N_YEARS * (3 * EG_N_ACTIONS + EG_N_DEFICIT_KEYS))
 int eg_update_stats_device(eg_ctx* ctx, const eg_weights* w, const eg_result* d_results, const eg_traj* d_trajs, uint32_t n,
                            int64_t* d_stats /* EG_STATS_WORDS, accumulated (not cleared) */,
@@ -303,18 +304,6 @@ int eg_update_stats_clear_device(eg_ctx* ctx, int64_t* d_stats);
 int eg_update_pack_best_device(eg_ctx* ctx, const eg_result* d_results, const eg_traj* d_trajs, uint32_t n,
                                const double* d_best_score, const unsigned long long* d_best_index,
                                uint64_t first_global_episode, void* d_record);
-/* The exchange step as one kernel over NVLink peer memory (one process per GPU): packs this rank's [statistics table | winner
- * record] (EG_STATS_WORDS int64 followed by EG_BEST_RECORD_BYTES) and stores it straight into slot `rank` of EVERY rank's gather
- * buffer through peer mappings, raises a flag on each peer and waits for the peers' flags; when the kernel ends this rank's gather
- * buffer holds all ranks' contributions of this `epoch` — no separate collective. peer_buffers[r] / peer_flags[r] (HOST arrays of
- * `world` device addresses) are rank r's gather buffer, int64[2][world][EG_STATS_WORDS + EG_BEST_RECORD_BYTES / 8] (the halves
- * alternate with the epoch's parity), and flag array, uint32[world] zeroed before the first epoch; both must be mapped on every
- * rank's GPU (a symmetric allocation, e.g. torch.distributed._symmetric_memory). `epoch` counts the calls from 1, identically
- * on every rank. *d_error is set to 1 if a peer did not deliver within ~2 s. */
-int eg_update_pack_exchange_device(eg_ctx* ctx, const eg_result* d_results, const eg_traj* d_trajs, uint32_t n, const int64_t* d_stats,
-                                   const double* d_best_score, const unsigned long long* d_best_index, uint64_t first_global_episode,
-                                   const uint64_t* peer_buffers, const uint64_t* peer_flags, uint32_t world, uint32_t rank,
-                                   uint32_t epoch, uint32_t* d_error);
 int eg_update_apply_stats(eg_weights* w, const int64_t* stats, uint64_t n_total,
                           const eg_result* batch_best_result, const eg_traj* batch_best_traj,
                           int64_t batch_best_index, eg_update_stats* stats_out);

@@ -22,19 +22,17 @@ for s in range(steps):
     ev[1].record(tr.stream)
     tr.launch_stats()
     ev[2].record(tr.stream)
-    tr._pack_best()
+    tr.exchange()
     with torch.cuda.stream(tr.stream):
-        tr.d_all_rec.copy_(tr.d_rec)
-        tr.h_stats.copy_(tr.d_stats, non_blocking=True)
-        tr.h_all_rec.copy_(tr.d_all_rec, non_blocking=True)
+        tr.h_all_pack.copy_(tr.d_all_pack, non_blocking=True)
     ev[3].record(tr.stream)
     tr.stream.synchronize()
     t2 = time.perf_counter()
-    st = T.combine_and_apply(tr.weights, tr.h_stats.numpy(), tr.h_all_rec.numpy(), n, tr.next_episode)
+    st = T.sum_and_apply(tr.weights, tr.h_all_pack.numpy(), n, tr.next_episode)
     tr.next_episode += n
     t3 = time.perf_counter()
     res, traj = tr.fetch_results()
-    print("step %d: upload %.2f ms | rollout %.2f ms | stats %.2f ms | pack+d2h %.2f ms | host apply %.2f ms | total %.2f ms | "
+    print("step %d: upload %.2f ms | rollout %.2f ms | stats %.2f ms | exchange+d2h %.2f ms | host apply %.2f ms | total %.2f ms | "
           "iwi %d best %.4f improved %d | mean gens %.1f actions/ep %.1f flags %d" % (
               s, (t1 - t0) * 1e3, ev[0].elapsed_time(ev[1]), ev[1].elapsed_time(ev[2]), ev[2].elapsed_time(ev[3]), (t3 - t2) * 1e3,
               (t3 - t0) * 1e3, st.iterations_without_improvement, st.best_score, st.n_improvements,

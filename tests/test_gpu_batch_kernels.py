@@ -3,8 +3,7 @@
 - eg_stats_kernel / eg_stats_argbest_kernel (csrc/stats.cu) against tests/stats_ref.py: 65,536 episodes (several trips of
   the grid-stride loop per warp), every score regime, the cost-only mode, best lists longer than the record (quirk Q10),
   records whose counts run past the capacity, ties for the best score, empty and odd-sized batches, accumulation.
-- eg_stats_pack_best_kernel and eg_pack_exchange_kernel byte for byte against trainer.pack_record / pack_buffer, with every
-  peer of the exchange on one GPU.
+- eg_stats_pack_best_kernel byte for byte against trainer.pack_record.
 - Which instantiation of eg_episode_kernel the launcher picks, read from a CUDA profiler trace.
 
 The statistics kernel reads only (results, records) from device memory and the uploaded policy, so most inputs are built by
@@ -235,60 +234,6 @@ def test_pack_best_record(gpu_ctx, trained, scale_batch):
         gpu_ctx.update_pack_best_device(s.n, s.d_res, s.d_traj, s.d_bs, s.d_bi, FIRST_GLOBAL, d_rec.data_ptr() + 4)
     assert e.value.code == -1
     assert gpu_ctx.kernel_launches() == launches
-
-
-SENTINEL = 0x5A5A5A5A5A5A5A5A
-
-
-@pytest.mark.parametrize("world", [1, 2, 8, 16])
-@pytest.mark.parametrize("last_rank", [False, True])
-def test_pack_exchange_with_every_peer_on_one_gpu(gpu_ctx, trained, scale_batch, world, last_rank):
-    """Rank `rank`'s [statistics | winner record] lands in slot (epoch & 1, rank) of every peer's gather buffer and nowhere
-    else, and its flag is raised on every peer. Every peer's buffer is an allocation on this GPU; the flags this rank waits
-    for are raised by the host before each launch, so the kernel's wait ends at its first read."""
-    torch = _torch()
-    dev = torch.device("cuda", 0)
-    rank = world - 1 if last_rank else 0
-    res, traj = scale_batch
-    s = _Stats(gpu_ctx, _with_iwi(trained, 900), res[:512], traj[:512])
-    bufs = [torch.full((2 * world * T.PACK_WORDS,), SENTINEL, dtype=torch.int64, device=dev) for _ in range(world)]
-    flags = [torch.zeros(world, dtype=torch.int32, device=dev) for _ in range(world)]
-    d_error = torch.zeros(1, dtype=torch.int32, device=dev)
-    expected = {}
-    for epoch in (1, 2):
-        first = FIRST_GLOBAL + 1000 * epoch  # a different record in each epoch
-        flags[rank].fill_(epoch)
-        torch.cuda.synchronize()
-        gpu_ctx.update_pack_exchange_device(512, s.d_res, s.d_traj, s.d_stats, s.d_bs, s.d_bi, first,
-                                            [b.data_ptr() for b in bufs], [f.data_ptr() for f in flags], rank, epoch, d_error)
-        gpu_ctx.sync()
-        k = s.best_index
-        expected[epoch & 1] = T.pack_buffer(s.stats, T.pack_record(s.best_score, first + k, res[k:k + 1], traj[k:k + 1]))
-        for b in range(world):
-            got = bufs[b].cpu().numpy().reshape(2, world, T.PACK_WORDS)
-            for half in (0, 1):
-                for r in range(world):
-                    if r == rank and half in expected:
-                        assert np.array_equal(got[half, r], expected[half]), (b, half, r, epoch)
-                    else:
-                        assert (got[half, r] == SENTINEL).all(), (b, half, r, epoch)
-            assert int(flags[b][rank].item()) == epoch
-        assert int(d_error.item()) == 0
-
-
-def test_pack_exchange_rejects_a_bad_world_without_a_launch(gpu_ctx):
-    torch = _torch()
-    dev = torch.device("cuda", 0)
-    one = torch.zeros(64, dtype=torch.int64, device=dev)
-    d_error = torch.zeros(1, dtype=torch.int32, device=dev)
-    launches = gpu_ctx.kernel_launches()
-    for world, rank in ((0, 0), (17, 0), (4, 4), (1, 1)):
-        with pytest.raises(_lib.EirgridError) as e:
-            gpu_ctx.update_pack_exchange_device(1, one, one, one, one, one, 0, [one.data_ptr()] * world, [one.data_ptr()] * world,
-                                                rank, 1, d_error)
-        assert e.value.code == -1
-    assert gpu_ctx.kernel_launches() == launches
-    assert int(d_error.item()) == 0
 
 
 # ---- which instantiation of eg_episode_kernel runs ----
