@@ -16,7 +16,11 @@ from test_host_sanitizers import ASSETS, _build, _run
 
 RADII = [3000.0, 5000.0, 6000.0, 7000.0, 8000.0, 12000.0]          # metal_location_search.rs:139-146, by radius class
 MAPS = [(51, 1000.0, 0), (21, 2500.0, 0), (47, 1086.0, 0), (64, 790.0, 0), (65, 780.0, 1), (101, 500.0, 1), (151, 331.0, 1),
-        (161, 312.0, 1), (181, 277.0, 1), (182, 275.0, 2), (191, 262.0, 2)]
+        (161, 312.0, 1), (181, 277.0, 1), (182, 275.0, 2), (191, 262.0, 2),
+        # the griddings of test_placement_edges.py: lists shorter than one walk step, the largest grid eg_map_set accepts, and the
+        # medium and general forms chosen by the size of the factor table on grids small enough for a narrower one
+        (2, 1000.0, 0), (3, 1000.0, 0), (5, 1000.0, 0), (41, 1000.0, 0), (255, 196.0, 2), (64, 300.0, 1), (40, 150.0, 2),
+        (41, 150.0, 2)]
 
 
 def _limits(step):
@@ -43,7 +47,7 @@ def dump(tmp_path_factory):
         m = re.match(r"map (\d+) (\S+) geom=(\d+) stride=(\d+) entries=(\d+)", line)
         if m:
             cur = dict(geom=int(m.group(3)), stride=int(m.group(4)), entries=int(m.group(5)), rclass=[], types=[])
-            maps[int(m.group(1))] = cur
+            maps[(int(m.group(1)), float(m.group(2)))] = cur
             continue
         m = re.match(r"\s+rclass (\d+) limit=(\d+) offset=(\d+) first=(\S+) last_inside=(\S+) at_limit=(\S+)", line)
         if m:
@@ -59,12 +63,12 @@ def dump(tmp_path_factory):
 
 
 def test_every_map_was_built(dump):
-    assert sorted(dump) == sorted(n for n, _, _ in MAPS)
+    assert sorted(dump) == sorted((n, step) for n, step, _ in MAPS)
 
 
 @pytest.mark.parametrize("n,step,geom", MAPS)
 def test_geometry_and_factor_table_layout(dump, n, step, geom):
-    d = dump[n]
+    d = dump[(n, step)]
     limits = _limits(step)
     assert [r["limit"] for r in d["rclass"]] == limits
     # block-shared copy: every class is followed by one entry (the 1.0), the offsets are running sums of limit + 1
@@ -89,7 +93,7 @@ def test_geometry_and_factor_table_layout(dump, n, step, geom):
 
 
 def test_per_type_words_agree_with_the_tables_they_replace(dump):
-    for n, d in dump.items():
+    for d in dump.values():
         assert len(d["types"]) == 15
         for t in d["types"]:
             # (plain, intermittent, storage, CO2): the net output in the slot of the accumulator class, +0.0 elsewhere
